@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the BPR-MF / NGCF train + full-catalog eval hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Headline (BASELINE.json configs[1]): NGCF 3-layer d=64 BPR training on the synthetic Yelp2018-shape graph
 (31,668 users x 38,048 items, 1,561,406 interactions), batch 2048, Adam lr 1e-4 — `value` = training triples/s
@@ -33,6 +33,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True       # the benchmark may run from a read-only tree: it leaves no bytecode caches there
 
 METRIC = "ngcf_bpr_train_triples_per_sec"
 UNIT = "triples/s"
@@ -135,6 +136,15 @@ def timed(fn, n, stream_sync=True):
     e1.record()
     torch.cuda.synchronize()
     return e0.elapsed_time(e1)
+
+
+def dump_outputs(out_dir, ntr, step_losses):
+    """What the timed NGCF step hands its caller after the last timed step: that step's batch-mean BPR loss and the
+    parameters it updated (state_dict names), one float32 .npy each (17.9 MB in all at the Yelp shape)."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": step_losses[-1:], **ntr.model.state_dict()}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().to(torch.float32).cpu().numpy())
 
 
 # ---------------------------------------------------------------------------------------------------------
@@ -302,7 +312,11 @@ def main():
     ap.add_argument("--c5-scale", type=float, default=1.0, help="shrink config 5 (users, items, interactions) by this factor")
     ap.add_argument("--only-c5", action="store_true", help="profiling aid: only the config-5 runs, no JSON contract")
     ap.add_argument("--only", default="", help="profiling aid: run only 'ngcf' | 'mf' | 'eval' steps, no JSON contract")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss and parameters of the last timed NGCF step (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.only_c5 or args.only in ("mf", "eval")):
+        ap.error("--dump-outputs writes the timed NGCF step's outputs: not with --impl reference, --only-c5 or --only mf|eval")
     args.warmup = max(args.warmup, 3) if not args.only else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -415,18 +429,11 @@ def main():
     sampler = ClockSampler(local)
     sampler.start()
     ms = timed(lambda i: ngcf_step(W + i), K)
-    # the contract's K steps above; then the same step for >= 240 more steps in chunks of 20 (SURVEY 8(d) asks >= 200 timed
-    # steps; the NVML clock sampler covers both regions, so a 15 ms region no longer means 6 samples)
-    long_chunks = []
-    if not args.only:
-        for c in range(12):
-            long_chunks.append(timed(lambda i: ngcf_step((c * 20 + i) % (K + W)), 20) / 20)
     clocks = sampler.stop()
     barrier()
     ms = max_over_ranks(ms)
-    long_run = ({"steps": 20 * len(long_chunks), "ms_per_step_median": float(np.median(long_chunks)),
-                 "ms_per_step_min": float(np.min(long_chunks)), "ms_per_step_max": float(np.max(long_chunks)),
-                 "note": "12 back-to-back chunks of 20 steps, CUDA events per chunk"} if long_chunks else None)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ntr, sl)
     ngcf_loss = ntr.loss_sum()
     value = world * K * B / (ms * 1e-3)
     if args.only == "ngcf":
@@ -787,7 +794,7 @@ def main():
                            "parallelism": "1 GPU" if world == 1 else f"{world} independent replicas (replicas only)",
                            "l2": "per-step working set (~0.4 GB of E/LE/G/T/CSR/Adam state) exceeds the 126 MB L2; no flush"},
                 "clocks": clocks, "e2e": e2e, "gpu_launches": launches_per_step * K, "roofline": roofline,
-                "cpu_baseline": cpu_baseline, "long_run": long_run, "extra": extra, "loss_sum": ngcf_loss,
+                "cpu_baseline": cpu_baseline, "extra": extra, "loss_sum": ngcf_loss,
                 "lib": os.path.relpath(_cabi.lib_path(), ROOT)}
         print(json.dumps(line))
     if world > 1:

@@ -1,5 +1,6 @@
 // Probe: cost of double-precision exp / log1p (the correctly rounded fp32 exp the trainers share with the oracle) next to
 // expf / log1pf and a plain DFMA chain on this GPU. One warp per "triple", like the BPR kernels: 2,048 warps x REPS calls.
+// Build: nvcc -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -o scripts/bin/fp64_probe scripts/fp64_probe.cu
 #include <cuda_runtime.h>
 #include <stdio.h>
 #define CK(x) do { cudaError_t e = (x); if (e != cudaSuccess) { printf("CUDA error %s line %d\n", cudaGetErrorString(e), __LINE__); return 1; } } while (0)
