@@ -552,6 +552,26 @@ int yr_topk_metrics(const int64_t* predicted, int64_t ldp, int64_t n, const int3
                     const int32_t* act_idx, const int32_t* act_nuniq, const double* inv_log2, int K,
                     double* user_metrics, double* metric_sums, yr_stream stream);
 
+/* ----------------------------------------------------------------------------------------------
+ * Top-K retrieval (retrieval.cu)
+ * ---------------------------------------------------------------------------------------------- */
+enum yr_dtype { YR_DTYPE_F32 = 0, YR_DTYPE_BF16 = 1 };
+
+/* For each of the B users user_ids[b]: score = U[uid] . V[i] over all nI items (U [nU x d], V [nI x d], both row-major
+ * of `dtype`, fp32 accumulation in one fma chain per score, k ascending: the scores of yr_eval_topk_metrics), and
+ * out_ids / out_scores [B x K] = the K best items by (score desc, item id asc). The B x nI scores are never stored.
+ * seen_ptr / seen_idx (both NULL = no seen lists): CSR of seen items, ascending per row, indexed by the user id
+ * (seen_by_row = 0, nU + 1 offsets) or by the batch row b (seen_by_row = 1, B + 1 offsets). A seen item scores
+ * masked_score instead: -INFINITY excludes it. Items scoring -inf or NaN are never returned; a row with fewer than K
+ * returnable items is padded with id -1 / score -inf. A user id outside [0, nU) sets *err = 1 (err may be NULL) and
+ * gets an all-padding row. 1 <= K <= 1024, d % 8 == 0, d <= 512, nI < 2^31 - 1.
+ * ws: yr_recommend_ws_bytes(B, nI, K) bytes (0 = none needed; same device as the call). */
+size_t yr_recommend_ws_bytes(int64_t B, int64_t nI, int K);
+int yr_recommend_topk(const void* U, int64_t nU, const void* V, int64_t nI, int d, int dtype, const int64_t* user_ids,
+                      int64_t B, const int32_t* seen_ptr, const int32_t* seen_idx, int seen_by_row, float masked_score,
+                      int K, int64_t* out_ids, float* out_scores, void* ws, size_t ws_bytes, int32_t* err,
+                      yr_stream stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -33,9 +33,11 @@ SYMBOLS = (
     "yr_sample_negatives", "yr_laplacian_ws_bytes", "yr_laplacian_build",
     "yr_synth_user_rows", "yr_laplacian_binary_values",
     "yr_split_ws_bytes", "yr_split_sizes", "yr_split_per_user",
+    "yr_recommend_ws_bytes", "yr_recommend_topk",
 )
 
 YR_OPT_SGD, YR_OPT_ADAM, YR_OPT_ADAMW = 0, 1, 2
+YR_DTYPE_F32, YR_DTYPE_BF16 = 0, 1
 # yr_dense_mode: where the NGCF d x d transforms run (per call / per trainer state)
 YR_DENSE_FP32, YR_DENSE_TC_FWD, YR_DENSE_TC = 0, 1, 2
 OPT_KINDS = {"sgd": YR_OPT_SGD, "adam": YR_OPT_ADAM, "adamw": YR_OPT_ADAMW}
@@ -197,6 +199,8 @@ def load() -> C.CDLL:
                                               p, p, p, p, p, sz, p, p]),
         "yr_eval_topk_metrics_tc_slice": (C.c_int, [p, i64, p, p, i64, i64, i32, p, i64, p, p, p, p, p, p, i32,
                                                     p, p, p, p, p, sz, p, i32, i32, p, p]),
+        "yr_recommend_ws_bytes": (sz, [i64, i64, i32]),
+        "yr_recommend_topk": (C.c_int, [p, i64, p, i64, i32, i32, p, i64, p, p, i32, f32, i32, p, p, p, sz, p, p]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)

@@ -1,0 +1,357 @@
+// Fused top-K retrieval (sm_100a): for a batch of users, score = u . v over the whole catalog, drop (or re-score) the
+// items each user has already seen, and keep the K best by (score desc, item id asc). The B x nI score matrix never
+// reaches global memory: scores live in registers, the running per-user top-K in shared memory.
+//
+// One block = TU users x one contiguous item range (a "split"). Items stream in tiles of 256, one item per thread;
+// a thread scores its item against all TU users with one fp32 fma chain per score, k ascending from 0 — the canonical
+// order of the evaluation kernels (eval.cu), so scores and therefore rankings are bit-identical to theirs. A candidate
+// (score, item) is packed into one u64 key that orders exactly like (score desc, id asc); keys beating the user's
+// current K-th best are appended to the user's candidate buffer, and a block-wide bitonic sort truncates a buffer to
+// its K best whenever one could overflow on the next tile. With more than one split, recommend_merge_kernel merges the
+// per-split lists.
+#include <float.h>
+#include <cuda_bf16.h>
+#include "common.cuh"
+
+namespace yr {
+
+constexpr int kRtThreads = 256;
+constexpr int kRtTile = 256;         // items per tile, one per thread
+constexpr int kRtEntries = 8192;     // candidate keys per block: TU users x (kRtEntries / TU)
+constexpr int kRtMaxK = 1024;
+constexpr int kRtMaxD = 512;
+constexpr int kRtMinSplit = 4096;    // items per split at least: long enough for the thresholds to settle
+constexpr int kRtMergeMax = 16384;   // keys one merge block sorts (128 KB of shared memory)
+
+// (score desc, id asc) == u64 key desc. Scores map to an order-preserving u32; ids are stored complemented.
+// Key 0 is never a candidate (it would be a negative NaN with id 2^32 - 1): it marks an empty slot.
+__device__ __forceinline__ uint64_t rt_key(float s, uint32_t item) {
+  uint32_t u = __float_as_uint(s);
+  u = (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+  return ((uint64_t)u << 32) | (uint64_t)(0xffffffffu - item);
+}
+
+__device__ __forceinline__ void rt_decode(uint64_t key, int64_t& id, float& s) {
+  if (key == 0) { id = -1; s = -INFINITY; return; }
+  uint32_t u = (uint32_t)(key >> 32);
+  u = (u & 0x80000000u) ? (u & 0x7fffffffu) : ~u;
+  s = __uint_as_float(u);
+  id = (int64_t)(0xffffffffu - (uint32_t)key);
+}
+
+__device__ __forceinline__ float rt_to_float(float x) { return x; }
+__device__ __forceinline__ float rt_to_float(__nv_bfloat16 x) { return __bfloat162float(x); }
+
+// v[0..7] = p[0..7] as floats (p 16-byte aligned)
+__device__ __forceinline__ void rt_load8(const float* p, float (&v)[8]) {
+  const float4 a = __ldg(reinterpret_cast<const float4*>(p));
+  const float4 b = __ldg(reinterpret_cast<const float4*>(p) + 1);
+  v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
+}
+__device__ __forceinline__ void rt_load8(const __nv_bfloat16* p, float (&v)[8]) {
+  const uint4 a = __ldg(reinterpret_cast<const uint4*>(p));
+  const uint32_t w[4] = {a.x, a.y, a.z, a.w};
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    v[2 * i] = __uint_as_float(w[i] << 16);
+    v[2 * i + 1] = __uint_as_float(w[i] & 0xffff0000u);
+  }
+}
+
+// Sort each of the `segs` segments of `n` keys (n a power of two) descending; the whole block takes part.
+__device__ void rt_bitonic_desc(uint64_t* keys, int segs, int n) {
+  const int half = n >> 1;
+  for (int size = 2; size <= n; size <<= 1)
+    for (int stride = size >> 1; stride > 0; stride >>= 1) {
+      for (int t = threadIdx.x; t < segs * half; t += blockDim.x) {
+        const int seg = t / half, r = t - seg * half;
+        const int lo = 2 * stride * (r / stride) + (r % stride);
+        uint64_t* base = keys + (size_t)seg * n;
+        const uint64_t a = base[lo], b = base[lo + stride];
+        const bool desc = (lo & size) == 0;
+        if ((a < b) == desc) { base[lo] = b; base[lo + stride] = a; }
+      }
+      __syncthreads();
+    }
+}
+
+// Truncate every candidate buffer to its K best; thr[u] becomes the K-th best key once a user has K candidates.
+template <int TU>
+__device__ void rt_compact(uint64_t* keys, int* cnt, uint64_t* thr, int K) {
+  constexpr int CAP = kRtEntries / TU;
+  for (int i = threadIdx.x; i < TU * CAP; i += blockDim.x)
+    if ((i % CAP) >= cnt[i / CAP]) keys[i] = 0;
+  __syncthreads();
+  rt_bitonic_desc(keys, TU, CAP);
+  if (threadIdx.x < TU) {
+    const int u = threadIdx.x;
+    const int c = min(cnt[u], K);
+    cnt[u] = c;
+    if (c == K && thr[u] != ~0ull) thr[u] = keys[(size_t)u * CAP + K - 1];
+  }
+  __syncthreads();
+}
+
+template <typename T, int TU>
+__global__ void __launch_bounds__(kRtThreads)
+recommend_topk_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ V, int64_t nI, int d,
+                      const int64_t* __restrict__ uids, int64_t B, const int32_t* __restrict__ seen_ptr,
+                      const int32_t* __restrict__ seen_idx, int seen_by_row, float masked_score, int K, int64_t per_split,
+                      uint64_t* __restrict__ partial, int64_t* __restrict__ out_ids, float* __restrict__ out_scores,
+                      int32_t* err) {
+  constexpr int CAP = kRtEntries / TU;
+  constexpr int kWords = kRtTile / 32;
+  extern __shared__ __align__(16) uint64_t rt_smem[];
+  uint64_t* keys = rt_smem;                                    // [TU][CAP]
+  uint64_t* thr = keys + kRtEntries;                           // [TU]; ~0 = inactive row (no candidate beats it)
+  float* Us = reinterpret_cast<float*>(thr + TU);              // [TU][d]
+  uint32_t* bits = reinterpret_cast<uint32_t*>(Us + (size_t)TU * d);   // [TU][kWords]: seen items of the tile
+  int* cnt = reinterpret_cast<int*>(bits + TU * kWords);       // [TU]
+  int* mcur = cnt + TU;                                        // [TU]: next unconsumed entry of the seen list
+  int* mend = mcur + TU;                                       // [TU]
+
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int64_t b0 = (int64_t)blockIdx.x * TU;
+  const int split = blockIdx.y;
+  const int64_t ib = (int64_t)split * per_split;
+  const int64_t ie = min(nI, ib + per_split);
+
+  for (int i = tid; i < TU * d; i += kRtThreads) {
+    const int u = i / d, k = i - u * d;
+    const int64_t b = b0 + u;
+    float x = 0.f;
+    if (b < B) {
+      const int64_t uid = uids[b];
+      if (uid >= 0 && uid < nU) x = rt_to_float(U[uid * d + k]);
+    }
+    Us[i] = x;
+  }
+  if (tid < TU) {
+    const int64_t b = b0 + tid;
+    bool active = false;
+    int c = 0, en = 0;
+    if (b < B) {
+      const int64_t uid = uids[b];
+      active = uid >= 0 && uid < nU;
+      if (!active && err) atomicExch(err, 1);
+      if (active && seen_ptr) {
+        const int64_t row = seen_by_row ? b : uid;
+        c = seen_ptr[row]; en = seen_ptr[row + 1];
+        int lo = c, hi = en;                       // first seen entry >= ib (lists ascending)
+        while (lo < hi) {
+          const int mid = (lo + hi) >> 1;
+          if (seen_idx[mid] < ib) lo = mid + 1; else hi = mid;
+        }
+        c = lo;
+      }
+    }
+    thr[tid] = active ? 0ull : ~0ull;
+    cnt[tid] = 0;
+    mcur[tid] = c; mend[tid] = en;
+  }
+  __syncthreads();
+
+  for (int64_t i0 = ib; i0 < ie; i0 += kRtTile) {
+    // ---- seen items of this tile -> bitmask (one warp per user, the sorted list is consumed in order) ----
+    for (int i = tid; i < TU * kWords; i += kRtThreads) bits[i] = 0;
+    __syncthreads();
+    if (seen_ptr) {
+      const int64_t tile_end = min(i0 + kRtTile, ie);
+      for (int u = warp; u < TU; u += kRtThreads / 32) {
+        int c = mcur[u];
+        const int en = mend[u];
+        while (c < en) {
+          const int p = c + lane;
+          const int64_t it = (p < en) ? (int64_t)seen_idx[p] : INT64_MAX;
+          const bool in = it < tile_end;
+          if (in && it >= i0) atomicOr(bits + u * kWords + (int)((it - i0) >> 5), 1u << ((it - i0) & 31));
+          const int n = __popc(__ballot_sync(kFull, in));
+          c += n;
+          if (n < 32) break;
+        }
+        if (lane == 0) mcur[u] = c;
+      }
+    }
+    // ---- scores of my item against every user of the tile: one fma chain each, k ascending ----
+    const int64_t item = i0 + tid;
+    const bool have = item < ie;
+    float acc[TU];
+#pragma unroll
+    for (int u = 0; u < TU; ++u) acc[u] = 0.f;
+    if (have) {
+      const T* vrow = V + item * d;
+      for (int k = 0; k < d; k += 8) {
+        float v[8];
+        rt_load8(vrow + k, v);
+#pragma unroll
+        for (int u = 0; u < TU; ++u) {
+          const float4 a0 = *reinterpret_cast<const float4*>(Us + u * d + k);
+          const float4 a1 = *reinterpret_cast<const float4*>(Us + u * d + k + 4);
+          float s = acc[u];
+          s = fmaf(a0.x, v[0], s); s = fmaf(a0.y, v[1], s); s = fmaf(a0.z, v[2], s); s = fmaf(a0.w, v[3], s);
+          s = fmaf(a1.x, v[4], s); s = fmaf(a1.y, v[5], s); s = fmaf(a1.z, v[6], s); s = fmaf(a1.w, v[7], s);
+          acc[u] = s;
+        }
+      }
+    }
+    __syncthreads();   // bitmask complete
+    if (have) {
+#pragma unroll
+      for (int u = 0; u < TU; ++u) {
+        float s = acc[u];
+        if (seen_ptr && ((bits[u * kWords + warp] >> lane) & 1u)) s = masked_score;
+        if (s == 0.f) s = 0.f;                       // -0 ranks like +0
+        if (!(s > -INFINITY)) continue;              // excluded (-inf) or NaN: never returned
+        const uint64_t key = rt_key(s, (uint32_t)item);
+        if (key > thr[u]) {
+          const int p = atomicAdd(cnt + u, 1);
+          keys[(size_t)u * CAP + p] = key;
+        }
+      }
+    }
+    __syncthreads();
+    bool full = false;
+#pragma unroll
+    for (int u = 0; u < TU; ++u) full |= cnt[u] > CAP - kRtTile;   // the next tile could overflow the buffer
+    if (full) rt_compact<TU>(keys, cnt, thr, K);
+  }
+  rt_compact<TU>(keys, cnt, thr, K);
+
+  for (int i = tid; i < TU * K; i += kRtThreads) {
+    const int u = i / K, j = i - u * K;
+    const int64_t b = b0 + u;
+    if (b >= B) continue;
+    const uint64_t key = keys[(size_t)u * CAP + j];     // zero beyond the user's count: padding
+    if (partial) {
+      partial[((int64_t)split * B + b) * K + j] = key;
+    } else {
+      int64_t id; float s;
+      rt_decode(key, id, s);
+      out_ids[b * K + j] = id;
+      out_scores[b * K + j] = s;
+    }
+  }
+}
+
+// Row b: the K best of the S per-split lists partial[s][b][0..K).
+__global__ void __launch_bounds__(kRtThreads)
+recommend_merge_kernel(const uint64_t* __restrict__ partial, int S, int64_t B, int K, int P, int64_t* __restrict__ out_ids,
+                       float* __restrict__ out_scores) {
+  extern __shared__ __align__(16) uint64_t rt_smem[];
+  const int64_t b = blockIdx.x;
+  for (int i = threadIdx.x; i < P; i += blockDim.x) {
+    uint64_t key = 0;
+    if (i < S * K) {
+      const int s = i / K, j = i - s * K;
+      key = partial[((int64_t)s * B + b) * K + j];
+    }
+    rt_smem[i] = key;
+  }
+  __syncthreads();
+  rt_bitonic_desc(rt_smem, 1, P);
+  for (int j = threadIdx.x; j < K; j += blockDim.x) {
+    int64_t id; float s;
+    rt_decode(rt_smem[j], id, s);
+    out_ids[b * K + j] = id;
+    out_scores[b * K + j] = s;
+  }
+}
+
+}  // namespace yr
+
+using namespace yr;
+
+namespace {
+
+int rt_users_per_block(int K) { return K <= kRtEntries / 16 - kRtTile ? 16 : K <= kRtEntries / 8 - kRtTile ? 8 : 4; }
+
+int rt_pow2(int x) {
+  int p = 1;
+  while (p < x) p <<= 1;
+  return p;
+}
+
+// Item splits: enough blocks to give every SM a few, each split at least kRtMinSplit items (a multiple of the tile), and the
+// merge of S lists of K keys within one block's shared memory.
+int rt_splits(int64_t B, int64_t nI, int K, int sm, int64_t* per_split) {
+  const int TU = rt_users_per_block(K);
+  const int64_t bx = (B + TU - 1) / TU;
+  int64_t S = (4 * (int64_t)sm + bx - 1) / bx;
+  const int64_t by_len = nI / kRtMinSplit;
+  if (S > by_len) S = by_len;
+  while (S > 1 && rt_pow2((int)(S * K)) > kRtMergeMax) --S;
+  if (S < 1) S = 1;
+  int64_t per = (nI + S - 1) / S;
+  per = (per + kRtTile - 1) / kRtTile * kRtTile;
+  *per_split = per;
+  return (int)((nI + per - 1) / per);
+}
+
+size_t rt_smem_bytes(int TU, int d) {
+  return (size_t)kRtEntries * 8 + (size_t)TU * 8 + (size_t)TU * d * 4 + (size_t)TU * (kRtTile / 32) * 4 + 3 * (size_t)TU * 4;
+}
+
+template <typename T, int TU>
+int rt_launch(const void* U, int64_t nU, const void* V, int64_t nI, int d, const int64_t* uids, int64_t B,
+              const int32_t* seen_ptr, const int32_t* seen_idx, int seen_by_row, float masked_score, int K, int S,
+              int64_t per_split, uint64_t* partial, int64_t* out_ids, float* out_scores, int32_t* err, cudaStream_t s) {
+  static AttrOnce attr;
+  const size_t smem = rt_smem_bytes(TU, d);
+  int rc = attr.set(recommend_topk_kernel<T, TU>, (int)rt_smem_bytes(TU, kRtMaxD));
+  if (rc) return rc;
+  dim3 grid((unsigned)((B + TU - 1) / TU), (unsigned)S);
+  recommend_topk_kernel<T, TU><<<grid, kRtThreads, smem, s>>>(
+      reinterpret_cast<const T*>(U), nU, reinterpret_cast<const T*>(V), nI, d, uids, B, seen_ptr, seen_idx, seen_by_row,
+      masked_score, K, per_split, partial, out_ids, out_scores, err);
+  YR_CHECK_LAUNCH();
+  return YR_OK;
+}
+
+}  // namespace
+
+extern "C" size_t yr_recommend_ws_bytes(int64_t B, int64_t nI, int K) {
+  if (B <= 0 || nI <= 0 || K <= 0 || K > kRtMaxK) return 0;
+  int64_t per = 0;
+  const int S = rt_splits(B, nI, K, yr_sm_count(), &per);
+  return S > 1 ? (size_t)S * (size_t)B * (size_t)K * sizeof(uint64_t) : 0;
+}
+
+extern "C" int yr_recommend_topk(const void* U, int64_t nU, const void* V, int64_t nI, int d, int dtype,
+                                 const int64_t* user_ids, int64_t B, const int32_t* seen_ptr, const int32_t* seen_idx,
+                                 int seen_by_row, float masked_score, int K, int64_t* out_ids, float* out_scores, void* ws,
+                                 size_t ws_bytes, int32_t* err, yr_stream stream) {
+  if (!U || !V || !out_ids || !out_scores || (B > 0 && !user_ids)) return YR_ERR_BAD_ARG;
+  if ((seen_ptr == nullptr) != (seen_idx == nullptr)) return YR_ERR_BAD_ARG;
+  if (B < 0 || nU <= 0 || K <= 0 || K > kRtMaxK) return YR_ERR_BAD_ARG;
+  if (nI <= 0 || nI >= 0x7fffffffLL || d <= 0 || d > kRtMaxD || (d & 7) != 0) return YR_ERR_BAD_DIM;
+  if (dtype != YR_DTYPE_F32 && dtype != YR_DTYPE_BF16) return YR_ERR_BAD_ARG;
+  if (B == 0) return YR_OK;
+  cudaStream_t s = (cudaStream_t)stream;
+  int64_t per = 0;
+  const int S = rt_splits(B, nI, K, yr_sm_count(), &per);
+  uint64_t* partial = nullptr;
+  if (S > 1) {
+    if (!ws || ws_bytes < yr_recommend_ws_bytes(B, nI, K)) return YR_ERR_WORKSPACE;
+    partial = reinterpret_cast<uint64_t*>(ws);
+  }
+  const int TU = rt_users_per_block(K);
+  int rc;
+#define YR_RT_LAUNCH(T, TU_)                                                                                              \
+  rt_launch<T, TU_>(U, nU, V, nI, d, user_ids, B, seen_ptr, seen_idx, seen_by_row, masked_score, K, S, per, partial,     \
+                    out_ids, out_scores, err, s)
+  if (dtype == YR_DTYPE_F32)
+    rc = TU == 16 ? YR_RT_LAUNCH(float, 16) : TU == 8 ? YR_RT_LAUNCH(float, 8) : YR_RT_LAUNCH(float, 4);
+  else
+    rc = TU == 16 ? YR_RT_LAUNCH(__nv_bfloat16, 16) : TU == 8 ? YR_RT_LAUNCH(__nv_bfloat16, 8)
+                                                          : YR_RT_LAUNCH(__nv_bfloat16, 4);
+#undef YR_RT_LAUNCH
+  if (rc || S == 1) return rc;
+  const int P = rt_pow2(S * K);
+  static AttrOnce attr;
+  rc = attr.set(recommend_merge_kernel, kRtMergeMax * (int)sizeof(uint64_t));
+  if (rc) return rc;
+  recommend_merge_kernel<<<(unsigned)B, kRtThreads, (size_t)P * sizeof(uint64_t), s>>>(partial, S, B, K, P, out_ids,
+                                                                                     out_scores);
+  YR_CHECK_LAUNCH();
+  return YR_OK;
+}

@@ -511,6 +511,8 @@ def eval_topk_metrics(Uemb: torch.Tensor, Vemb: torch.Tensor, ecsr: DeviceEvalCS
 
     mode 'tc'    : tensor-core filter + exact re-score (yr_eval_topk_metrics_tc) — bit-identical outputs;
     mode 'exact' : FP32-pipe kernel (yr_eval_topk_metrics);
+    mode 'retrieval': top-K retrieval kernel (yr_recommend_topk, masked items score -3.40282e+38 as in the other modes)
+                   + yr_topk_metrics — the same scores, lists and metrics;
     mode None    : env YR_EVAL_MODE, else 'tc' whenever the library supports (d, K), 'exact' otherwise.
     slices       : item slices for small row sets (tensor-core mode only; None = eval_item_slices()); identical outputs."""
     import os
@@ -520,6 +522,12 @@ def eval_topk_metrics(Uemb: torch.Tensor, Vemb: torch.Tensor, ecsr: DeviceEvalCS
     dev = Uemb.device
     nI, d = Vemb.shape
     mode = mode or os.environ.get("YR_EVAL_MODE") or "auto"
+    if mode == "retrieval":
+        eval_topk_metrics.last_slices = 1
+        topk, tsc = recommend_topk(Uemb, Vemb, ecsr.eval_uid, ecsr.K, ecsr.mask_ptr, ecsr.mask_idx, seen_by_row=True,
+                                   masked_score=EVAL_MASK_VALUE)
+        um, sums = topk_metrics(topk, ecsr)
+        return topk, tsc, um, sums, torch.zeros(1, device=dev, dtype=I32)
     use_tc = mode == "tc" or (mode == "auto" and lib.yr_eval_tc_supported(d, ecsr.K) != 0)
     eval_topk_metrics.last_slices = 1
     if use_tc and ecsr.n_eval > 0:
@@ -572,6 +580,9 @@ def eval_topk_metrics(Uemb: torch.Tensor, Vemb: torch.Tensor, ecsr: DeviceEvalCS
     return topk[:n], tsc[:n], um[:n], sums, err
 
 
+EVAL_MASK_VALUE = -3.40282e+38     # score of a masked (train) item in evaluation (trainers/mf_trainer.py:167)
+
+
 def metrics_from_sums(sums, n_eval: int):
     """(precision, recall, map, ndcg) with the reference's divisors (metric.py:24,47,70,104 — quirk Q6)."""
     s = [float(x) for x in sums]
@@ -600,3 +611,69 @@ def topk_metrics(predicted: torch.Tensor, ecsr: DeviceEvalCSR):
                               dptr(ecsr.act_idx, I32), dptr(ecsr.act_nuniq, I32), dptr(ecsr.inv_log2, F64), ecsr.K,
                               dptr(um), dptr(sums), stream_ptr(predicted.device)), "yr_topk_metrics")
     return um[:n], sums
+
+
+# ----------------------------------------------------------------------------------------------------
+# top-K retrieval
+# ----------------------------------------------------------------------------------------------------
+RECOMMEND_MAX_K = 1024
+RECOMMEND_MAX_D = 512
+_RT_DTYPES = {F32: _cabi.YR_DTYPE_F32, torch.bfloat16: _cabi.YR_DTYPE_BF16}
+
+
+def recommend_topk(U: torch.Tensor, V: torch.Tensor, user_ids: torch.Tensor, K: int, seen_ptr: Optional[torch.Tensor] = None,
+                   seen_idx: Optional[torch.Tensor] = None, seen_by_row: bool = False,
+                   masked_score: float = float("-inf")) -> Tuple[torch.Tensor, torch.Tensor]:
+    """yr_recommend_topk: (ids int64 [B x K], scores float32 [B x K]) of the K best items per user by (score desc, id asc),
+    score = U[uid] . V[item] in fp32 (fp32 or bf16 tables). Seen items (CSR int32, ascending per row, rows = user ids, or
+    batch rows with seen_by_row) score `masked_score`; -inf drops them. Short rows are padded with id -1 / score -inf."""
+    if not (torch.is_tensor(U) and torch.is_tensor(V) and torch.is_tensor(user_ids)):
+        raise TypeError("recommend_topk: U, V and user_ids must be tensors")
+    if not (U.is_cuda and V.is_cuda and user_ids.is_cuda):
+        raise YelprecError("recommend_topk: U, V and user_ids must be CUDA tensors (the reference path is "
+                           "retrieval.recommend_reference)")
+    dev = U.device
+    if V.device != dev or user_ids.device != dev:
+        raise ValueError(f"recommend_topk: tensors on different devices ({U.device}, {V.device}, {user_ids.device})")
+    if U.dtype not in _RT_DTYPES or V.dtype != U.dtype:
+        raise TypeError(f"recommend_topk: U and V must both be float32 or both bfloat16, got {U.dtype} and {V.dtype}")
+    if U.dim() != 2 or V.dim() != 2 or U.shape[1] != V.shape[1]:
+        raise ValueError(f"recommend_topk: U [nU x d] and V [nI x d] expected, got {tuple(U.shape)} and {tuple(V.shape)}")
+    d = int(U.shape[1])
+    if d % 8 != 0 or d > RECOMMEND_MAX_D:
+        raise ValueError(f"recommend_topk: embedding width {d} must be a multiple of 8 and at most {RECOMMEND_MAX_D}")
+    nU, nI = int(U.shape[0]), int(V.shape[0])
+    if nU == 0 or nI == 0 or nI >= 2 ** 31 - 1:
+        raise ValueError(f"recommend_topk: {nU} users x {nI} items is not a valid catalog")
+    if isinstance(K, bool) or int(K) != K or not 1 <= int(K) <= RECOMMEND_MAX_K:
+        raise ValueError(f"recommend_topk: k must be an integer in [1, {RECOMMEND_MAX_K}], got {K}")
+    K = int(K)
+    if user_ids.dtype not in (I64, I32) or user_ids.dim() != 1:
+        raise TypeError(f"recommend_topk: user_ids must be a 1-D int64 or int32 tensor, got {user_ids.dtype} {tuple(user_ids.shape)}")
+    if (seen_ptr is None) != (seen_idx is None):
+        raise ValueError("recommend_topk: seen_ptr and seen_idx go together")
+    uid = user_ids.to(I64).contiguous()
+    B = int(uid.numel())
+    if seen_ptr is not None:
+        rows = B if seen_by_row else nU
+        if seen_ptr.dtype != I32 or seen_idx.dtype != I32 or seen_ptr.numel() != rows + 1:
+            raise ValueError(f"recommend_topk: seen lists must be int32 CSR with {rows + 1} offsets")
+        if seen_ptr.device != dev or seen_idx.device != dev:
+            raise ValueError("recommend_topk: seen lists must live on the device of the embeddings")
+        seen_ptr = seen_ptr.contiguous()
+        seen_idx = seen_idx.contiguous() if seen_idx.numel() else torch.zeros(1, dtype=I32, device=dev)
+    lib = _cabi.load()
+    Uc, Vc = U.detach().contiguous(), V.detach().contiguous()
+    ids = torch.empty(B, K, device=dev, dtype=I64)
+    scores = torch.empty(B, K, device=dev, dtype=F32)
+    if B == 0:
+        return ids, scores
+    err = torch.zeros(1, device=dev, dtype=I32)
+    nbytes = lib.yr_recommend_ws_bytes(B, nI, K)
+    ws = torch.empty(max(nbytes, 1), device=dev, dtype=torch.uint8)
+    check(lib.yr_recommend_topk(Uc.data_ptr(), nU, Vc.data_ptr(), nI, d, _RT_DTYPES[U.dtype], dptr(uid, I64), B,
+                                dptr(seen_ptr), dptr(seen_idx), 1 if seen_by_row else 0, float(masked_score), K,
+                                dptr(ids), dptr(scores), dptr(ws), nbytes, dptr(err), stream_ptr(dev)), "yr_recommend_topk")
+    if int(err.item()) != 0:
+        raise IndexError(f"recommend_topk: user id out of range [0, {nU})")
+    return ids, scores

@@ -166,7 +166,7 @@ class MFTrainer(BaseTrainer):
         self.model.eval()
         ecsr = self._eval_csr(eval_data)
         U, V = self.model.user_embedding.weight.data, self.model.item_embedding.weight.data
-        topk, _, _, sums, err = ops.eval_topk_metrics(U, V, ecsr)
+        topk, _, _, sums, err = ops.eval_topk_metrics(U, V, ecsr, mode=getattr(self.cfg, "eval_mode", None))
         self.last_topk = topk
         sums_h = sums.cpu()
         ops._raise_if_err(err, "MFTrainer.evaluate")
@@ -176,6 +176,11 @@ class MFTrainer(BaseTrainer):
             logger.info(f"[Trainer] Test > precision@{k} : {result[0]:.4f} / Recall@{k}: {result[1]:.4f} / "
                         f"MAP@{k}: {result[2]:.4f} / NDCG@{k}: {result[3]:.4f}")
         return result
+
+    def recommender(self, seen=None):
+        """retrieval.Recommender over the current user / item tables (recommend(user_ids, k, exclude_seen=True))."""
+        from ..retrieval import Recommender
+        return Recommender(self.model.user_embedding.weight.data, self.model.item_embedding.weight.data, seen)
 
     def _generate_top_k_recommendation(self, pred: torch.Tensor, mask_items) -> np.ndarray:
         """One score row -> top-K item ids, best first (mf_trainer.py:163-178). Ties: (score desc, id asc)."""

@@ -259,7 +259,7 @@ class NGCFTrainer(BaseTrainer):
         layers, _, _ = self.propagate()
         cat = ops.ngcf_concat(layers)
         users, items = cat[: self.num_users], cat[self.num_users:]
-        topk, _, _, sums, err = ops.eval_topk_metrics(users, items, ecsr)
+        topk, _, _, sums, err = ops.eval_topk_metrics(users, items, ecsr, mode=getattr(self.cfg, "eval_mode", None))
         self.last_topk = topk
         sums_h = sums.cpu()
         ops._raise_if_err(err, "NGCFTrainer.evaluate")
@@ -269,6 +269,12 @@ class NGCFTrainer(BaseTrainer):
             logger.info(f"[Trainer] Test > precision@{k} : {result[0]:.4f} / Recall@{k}: {result[1]:.4f} / "
                         f"MAP@{k}: {result[2]:.4f} / NDCG@{k}: {result[3]:.4f}")
         return result
+
+    def recommender(self, seen=None):
+        """retrieval.Recommender over the propagated, layer-concatenated user / item embeddings that evaluate() ranks with."""
+        from ..retrieval import Recommender
+        cat = ops.ngcf_concat(self.propagate()[0])
+        return Recommender(cat[: self.num_users], cat[self.num_users:], seen)
 
     def _generate_top_k_recommendation(self, pred: torch.Tensor, mask_items) -> np.ndarray:
         if not pred.is_cuda:
