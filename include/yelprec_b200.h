@@ -572,6 +572,23 @@ int yr_recommend_topk(const void* U, int64_t nU, const void* V, int64_t nI, int 
                       int K, int64_t* out_ids, float* out_scores, void* ws, size_t ws_bytes, int32_t* err,
                       yr_stream stream);
 
+/* yr_recommend_topk restricted per row to one subset of the catalog. The G subsets are a CSR of item ids: subset g is
+ * subset_idx[subset_ptr[g] .. subset_ptr[g + 1]), ascending and duplicate-free; subsets may overlap. Row b ranks only the
+ * items of subset subset_ids[b], or the whole catalog when subset_ids[b] = -1, and gets exactly the ids and scores
+ * yr_recommend_topk returns when every other item is a seen item with masked_score = -INFINITY (same scores, order,
+ * seen-item exclusion via seen_ptr / seen_idx indexed by user id, padding with id -1 / score -inf). Rows are grouped by
+ * subset on the device; outputs are in request order. max_subset_len: the longest list a row streams (the longest
+ * subset, nI if a row is -1); it only sets the number of item splits, any value >= 0 gives the same results. A user id
+ * outside [0, nU) sets bit 0 of *err (*err |= 1), a subset id outside [-1, G) bit 1 (*err |= 2); either row is all
+ * padding. B < 2^31 - 1, G >= 0; the other limits as yr_recommend_topk.
+ * ws: yr_recommend_subset_ws_bytes(B, G, max_subset_len, K) bytes (row grouping and per-split lists; same device). */
+size_t yr_recommend_subset_ws_bytes(int64_t B, int G, int64_t max_subset_len, int K);
+int yr_recommend_subset_topk(const void* U, int64_t nU, const void* V, int64_t nI, int d, int dtype,
+                             const int64_t* user_ids, int64_t B, const int32_t* subset_ptr, const int32_t* subset_idx,
+                             int G, int64_t max_subset_len, const int64_t* subset_ids, const int32_t* seen_ptr,
+                             const int32_t* seen_idx, int K, int64_t* out_ids, float* out_scores, void* ws,
+                             size_t ws_bytes, int32_t* err, yr_stream stream);
+
 #ifdef __cplusplus
 }
 #endif

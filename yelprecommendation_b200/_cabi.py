@@ -33,7 +33,7 @@ SYMBOLS = (
     "yr_sample_negatives", "yr_laplacian_ws_bytes", "yr_laplacian_build",
     "yr_synth_user_rows", "yr_laplacian_binary_values",
     "yr_split_ws_bytes", "yr_split_sizes", "yr_split_per_user",
-    "yr_recommend_ws_bytes", "yr_recommend_topk",
+    "yr_recommend_ws_bytes", "yr_recommend_topk", "yr_recommend_subset_ws_bytes", "yr_recommend_subset_topk",
 )
 
 YR_OPT_SGD, YR_OPT_ADAM, YR_OPT_ADAMW = 0, 1, 2
@@ -201,6 +201,9 @@ def load() -> C.CDLL:
                                                     p, p, p, p, p, sz, p, i32, i32, p, p]),
         "yr_recommend_ws_bytes": (sz, [i64, i64, i32]),
         "yr_recommend_topk": (C.c_int, [p, i64, p, i64, i32, i32, p, i64, p, p, i32, f32, i32, p, p, p, sz, p, p]),
+        "yr_recommend_subset_ws_bytes": (sz, [i64, i32, i64, i32]),
+        "yr_recommend_subset_topk": (C.c_int, [p, i64, p, i64, i32, i32, p, i64, p, p, i32, i64, p, p, p, i32, p, p, p,
+                                               sz, p, p]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)

@@ -9,7 +9,11 @@
 // current K-th best are appended to the user's candidate buffer, and a block-wide bitonic sort truncates a buffer to
 // its K best whenever one could overflow on the next tile. With more than one split, recommend_merge_kernel merges the
 // per-split lists.
+//
+// recommend_subset_kernel restricts each row to one subset of the catalog (an ascending item-id list): the same scores,
+// masking and selection over the gathered ids of the row's subset, with rows grouped by subset on the device first.
 #include <float.h>
+#include <algorithm>
 #include <cuda_bf16.h>
 #include "common.cuh"
 
@@ -90,6 +94,39 @@ __device__ void rt_compact(uint64_t* keys, int* cnt, uint64_t* thr, int K) {
     if (c == K && thr[u] != ~0ull) thr[u] = keys[(size_t)u * CAP + K - 1];
   }
   __syncthreads();
+}
+
+// acc[u] = Us[u] . vrow for the TU staged users, one fma chain each, k ascending (acc = 0 when vrow is null).
+template <typename T, int TU>
+__device__ __forceinline__ void rt_score(const T* __restrict__ vrow, const float* Us, int d, float (&acc)[TU]) {
+#pragma unroll
+  for (int u = 0; u < TU; ++u) acc[u] = 0.f;
+  if (!vrow) return;
+  for (int k = 0; k < d; k += 8) {
+    float v[8];
+    rt_load8(vrow + k, v);
+#pragma unroll
+    for (int u = 0; u < TU; ++u) {
+      const float4 a0 = *reinterpret_cast<const float4*>(Us + u * d + k);
+      const float4 a1 = *reinterpret_cast<const float4*>(Us + u * d + k + 4);
+      float s = acc[u];
+      s = fmaf(a0.x, v[0], s); s = fmaf(a0.y, v[1], s); s = fmaf(a0.z, v[2], s); s = fmaf(a0.w, v[3], s);
+      s = fmaf(a1.x, v[4], s); s = fmaf(a1.y, v[5], s); s = fmaf(a1.z, v[6], s); s = fmaf(a1.w, v[7], s);
+      acc[u] = s;
+    }
+  }
+}
+
+// Append (s, item) to user u's candidate buffer if it beats the user's current K-th best.
+template <int TU>
+__device__ __forceinline__ void rt_offer(uint64_t* keys, int* cnt, const uint64_t* thr, int u, float s, uint32_t item) {
+  if (s == 0.f) s = 0.f;                       // -0 ranks like +0
+  if (!(s > -INFINITY)) return;                // excluded (-inf) or NaN: never returned
+  const uint64_t key = rt_key(s, item);
+  if (key > thr[u]) {
+    const int p = atomicAdd(cnt + u, 1);
+    keys[(size_t)u * (kRtEntries / TU) + p] = key;
+  }
 }
 
 template <typename T, int TU>
@@ -257,6 +294,238 @@ recommend_merge_kernel(const uint64_t* __restrict__ partial, int S, int64_t B, i
   }
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// Subset-restricted retrieval. Row b ranks only the items of subset subset_ids[b] (an ascending id list of the subset
+// CSR; -1 = the whole catalog). Rows are grouped by subset on the device so that the TU users of a block share one list;
+// the block streams that list in tiles of 256 ids, gathering the item rows, and otherwise runs the path above. Groups:
+// g < G the subsets, G the whole catalog, G + 1 rows with an invalid subset id (an empty list: all-padding rows).
+// ---------------------------------------------------------------------------------------------------------------------
+constexpr int kRsPlanThreads = 1024;
+
+__device__ __forceinline__ int rs_group(const int64_t* subset_ids, int64_t b, int G, int32_t* err) {
+  const int64_t s = subset_ids[b];
+  if (s == -1) return G;
+  if (s < -1 || s >= G) {
+    if (err) atomicOr(err, 2);
+    return G + 1;
+  }
+  return (int)s;
+}
+
+// One block. Counting sort of the B rows by group: order[rows_at[g] .. rows_at[g + 1]) = the rows of group g (in no
+// particular order: a row's result does not depend on the rows it shares a block with), and blocks_at[g] = the first
+// scoring block of group g (ceil(rows / TU) blocks per group; blocks_at[G + 2] = all of them). cursor: G + 2 ints.
+__global__ void __launch_bounds__(kRsPlanThreads)
+recommend_subset_plan_kernel(const int64_t* __restrict__ subset_ids, int B, int G, int TU, int32_t* __restrict__ cursor,
+                             int32_t* __restrict__ rows_at, int32_t* __restrict__ blocks_at, int32_t* __restrict__ order,
+                             int32_t* err) {
+  __shared__ long long wsum[kRsPlanThreads / 32];
+  __shared__ long long carry;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int ng = G + 2;
+  for (int g = tid; g < ng; g += kRsPlanThreads) cursor[g] = 0;
+  if (tid == 0) carry = 0;
+  __syncthreads();
+  // histogram; lanes of a warp with the same group add once
+  for (int b0 = 0; b0 < B; b0 += kRsPlanThreads) {
+    const int b = b0 + tid;
+    const int g = b < B ? rs_group(subset_ids, b, G, err) : -1;
+    const unsigned same = __match_any_sync(kFull, g);
+    if (g >= 0 && lane == __ffs(same) - 1) atomicAdd(cursor + g, __popc(same));
+  }
+  __syncthreads();
+  // exclusive scan of (blocks << 32 | rows) over the groups
+  for (int g0 = 0; g0 < ng; g0 += kRsPlanThreads) {
+    const int g = g0 + tid;
+    const int c = g < ng ? __ldcg(cursor + g) : 0;   // the histogram's atomics live in L2
+    const long long v = ((long long)((c + TU - 1) / TU) << 32) | (long long)c;
+    long long x = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const long long y = __shfl_up_sync(kFull, x, o);
+      if (lane >= o) x += y;
+    }
+    if (lane == 31) wsum[warp] = x;
+    __syncthreads();
+    if (warp == 0) {
+      long long w = wsum[lane];
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const long long y = __shfl_up_sync(kFull, w, o);
+        if (lane >= o) w += y;
+      }
+      wsum[lane] = w;
+    }
+    __syncthreads();
+    const long long ex = carry + (warp ? wsum[warp - 1] : 0) + x - v;
+    if (g < ng) {
+      rows_at[g] = (int32_t)(ex & 0xffffffffll);
+      blocks_at[g] = (int32_t)(ex >> 32);
+      cursor[g] = (int32_t)(ex & 0xffffffffll);
+    }
+    __syncthreads();
+    if (tid == 0) carry += wsum[kRsPlanThreads / 32 - 1];
+    __syncthreads();
+  }
+  if (tid == 0) {
+    rows_at[ng] = B;
+    blocks_at[ng] = (int32_t)(carry >> 32);
+  }
+  // scatter; groups re-read from subset_ids (err is already set)
+  for (int b0 = 0; b0 < B; b0 += kRsPlanThreads) {
+    const int b = b0 + tid;
+    const int g = b < B ? rs_group(subset_ids, b, G, nullptr) : -1;
+    const unsigned same = __match_any_sync(kFull, g);
+    const int leader = __ffs(same) - 1;
+    int base = 0;
+    if (g >= 0 && lane == leader) base = atomicAdd(cursor + g, __popc(same));
+    base = __shfl_sync(kFull, base, leader);
+    if (g >= 0) order[base + __popc(same & ((1u << lane) - 1))] = b;
+  }
+}
+
+// Grid (upper bound on the plan's block count, S). Block x takes TU rows of one group and split y of the group's list:
+// a slice of at least kRtMinSplit ids (a multiple of the tile) so that groups shorter than the longest use fewer splits;
+// a split past the end of its list writes padding keys.
+template <typename T, int TU>
+__global__ void __launch_bounds__(kRtThreads, 2)   // 2 blocks an SM: up to 128 registers, no spills
+recommend_subset_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ V, int64_t nI, int d,
+                        const int64_t* __restrict__ uids, int64_t B, const int32_t* __restrict__ sub_ptr,
+                        const int32_t* __restrict__ sub_idx, int G, const int32_t* __restrict__ rows_at,
+                        const int32_t* __restrict__ blocks_at, const int32_t* __restrict__ order,
+                        const int32_t* __restrict__ seen_ptr, const int32_t* __restrict__ seen_idx, int K, int S,
+                        uint64_t* __restrict__ partial, int64_t* __restrict__ out_ids, float* __restrict__ out_scores,
+                        int32_t* err) {
+  constexpr int CAP = kRtEntries / TU;
+  constexpr int kWords = kRtTile / 32;
+  extern __shared__ __align__(16) uint64_t rt_smem[];
+  uint64_t* keys = rt_smem;                                    // [TU][CAP]
+  uint64_t* thr = keys + kRtEntries;                           // [TU]; ~0 = inactive row (no candidate beats it)
+  float* Us = reinterpret_cast<float*>(thr + TU);              // [TU][d]
+  uint32_t* bits = reinterpret_cast<uint32_t*>(Us + (size_t)TU * d);   // [TU][kWords]: seen items of the tile, by position
+  int* cnt = reinterpret_cast<int*>(bits + TU * kWords);       // [TU]
+  int* mcur = cnt + TU;                                        // [TU]: next unconsumed entry of the seen list
+  int* mend = mcur + TU;                                       // [TU]
+  int* rowb = mend + TU;                                       // [TU]: batch row of each user, -1 = none
+  int* sid = rowb + TU;                                        // [kRtTile]: item ids of the tile, ascending
+
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int blk = blockIdx.x, split = blockIdx.y;
+  if (blk >= blocks_at[G + 2]) return;
+  int lo = 0, hi = G + 2;                                      // group: the last g with blocks_at[g] <= blk
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (blocks_at[mid] <= blk) lo = mid + 1; else hi = mid;
+  }
+  const int g = lo - 1;
+  const int r0 = rows_at[g] + (blk - blocks_at[g]) * TU;
+  const int nr = min(TU, rows_at[g + 1] - r0);
+  const int32_t* list = g < G ? sub_idx + sub_ptr[g] : nullptr;   // null: the identity (whole catalog)
+  const int64_t len = g < G ? sub_ptr[g + 1] - sub_ptr[g] : g == G ? nI : 0;
+  int64_t per = max((len + S - 1) / S, (int64_t)kRtMinSplit);
+  per = (per + kRtTile - 1) / kRtTile * kRtTile;
+  const int64_t pb = min(len, (int64_t)split * per);
+  const int64_t pe = min(len, pb + per);
+
+  if (tid < TU) {
+    const int b = tid < nr ? order[r0 + tid] : -1;
+    bool active = false;
+    int c = 0, en = 0;
+    if (b >= 0) {
+      const int64_t uid = uids[b];
+      active = uid >= 0 && uid < nU;
+      if (!active && err) atomicOr(err, 1);
+      if (active && seen_ptr && pb < pe) {
+        c = seen_ptr[uid]; en = seen_ptr[uid + 1];
+        const int64_t first = list ? list[pb] : pb;
+        int l = c, h = en;                         // first seen entry >= the split's first id (lists ascending)
+        while (l < h) {
+          const int mid = (l + h) >> 1;
+          if (seen_idx[mid] < first) l = mid + 1; else h = mid;
+        }
+        c = l;
+      }
+    }
+    rowb[tid] = b;
+    thr[tid] = active ? 0ull : ~0ull;
+    cnt[tid] = 0;
+    mcur[tid] = c; mend[tid] = en;
+  }
+  __syncthreads();
+  if (pb < pe) {
+    for (int i = tid; i < TU * d; i += kRtThreads) {
+      const int u = i / d, k = i - u * d;
+      float x = 0.f;
+      if (thr[u] == 0ull) x = rt_to_float(U[uids[rowb[u]] * d + k]);
+      Us[i] = x;
+    }
+    for (int64_t p0 = pb; p0 < pe; p0 += kRtTile) {
+      const int n = (int)min((int64_t)kRtTile, pe - p0);
+      for (int i = tid; i < TU * kWords; i += kRtThreads) bits[i] = 0;
+      if (tid < n) sid[tid] = list ? list[p0 + tid] : (int)(p0 + tid);
+      __syncthreads();
+      // ---- seen items of this tile -> bitmask by tile position (one warp per user, the sorted list consumed in order) ----
+      if (seen_ptr) {
+        const int last = sid[n - 1];
+        for (int u = warp; u < TU; u += kRtThreads / 32) {
+          int c = mcur[u];
+          const int en = mend[u];
+          while (c < en) {
+            const int p = c + lane;
+            const int it = (p < en) ? seen_idx[p] : INT32_MAX;
+            const bool in = it <= last;
+            if (in) {
+              int l = 0, h = n;                    // position of `it` among the tile's ids, if it is one
+              while (l < h) {
+                const int mid = (l + h) >> 1;
+                if (sid[mid] < it) l = mid + 1; else h = mid;
+              }
+              if (l < n && sid[l] == it) atomicOr(bits + u * kWords + (l >> 5), 1u << (l & 31));
+            }
+            const int m = __popc(__ballot_sync(kFull, in));
+            c += m;
+            if (m < 32) break;
+          }
+          if (lane == 0) mcur[u] = c;
+        }
+      }
+      // ---- scores of my item against every user of the block: one fma chain each, k ascending ----
+      const bool have = tid < n;
+      const int item = have ? sid[tid] : 0;
+      float acc[TU];
+      rt_score<T, TU>(have ? V + (int64_t)item * d : nullptr, Us, d, acc);
+      __syncthreads();   // bitmask complete, tile ids consumed
+      if (have) {
+#pragma unroll
+        for (int u = 0; u < TU; ++u) {
+          if (seen_ptr && ((bits[u * kWords + warp] >> lane) & 1u)) continue;
+          rt_offer<TU>(keys, cnt, thr, u, acc[u], (uint32_t)item);
+        }
+      }
+      __syncthreads();
+      bool full = p0 + kRtTile >= pe;              // the last tile: truncate to the K best
+#pragma unroll
+      for (int u = 0; u < TU; ++u) full |= cnt[u] > CAP - kRtTile;   // the next tile could overflow a buffer
+      if (full) rt_compact<TU>(keys, cnt, thr, K);
+    }
+  }
+
+  for (int i = tid; i < TU * K; i += kRtThreads) {
+    const int u = i / K, j = i - u * K;
+    const int b = rowb[u];
+    if (b < 0) continue;
+    const uint64_t key = pb < pe ? keys[(size_t)u * CAP + j] : 0;   // zero beyond the user's count: padding
+    if (partial) {
+      partial[((int64_t)split * B + b) * K + j] = key;
+    } else {
+      int64_t id; float s;
+      rt_decode(key, id, s);
+      out_ids[(int64_t)b * K + j] = id;
+      out_scores[(int64_t)b * K + j] = s;
+    }
+  }
+}
+
 }  // namespace yr
 
 using namespace yr;
@@ -307,6 +576,43 @@ int rt_launch(const void* U, int64_t nU, const void* V, int64_t nI, int d, const
   return YR_OK;
 }
 
+size_t rs_smem_bytes(int TU, int d) { return rt_smem_bytes(TU, d) + (size_t)TU * 4 + (size_t)kRtTile * 4; }
+
+template <typename T, int TU>
+int rs_launch(const void* U, int64_t nU, const void* V, int64_t nI, int d, const int64_t* uids, int64_t B,
+              const int32_t* sub_ptr, const int32_t* sub_idx, int G, const int32_t* rows_at, const int32_t* blocks_at,
+              const int32_t* order, const int32_t* seen_ptr, const int32_t* seen_idx, int K, int S, uint64_t* partial,
+              int64_t* out_ids, float* out_scores, int32_t* err, cudaStream_t s) {
+  static AttrOnce attr;
+  int rc = attr.set(recommend_subset_kernel<T, TU>, (int)rs_smem_bytes(TU, kRtMaxD));
+  if (rc) return rc;
+  // the plan makes sum over groups of ceil(rows / TU) blocks: at most ceil(B / TU) + one per non-empty group
+  dim3 grid((unsigned)((B + TU - 1) / TU + std::min<int64_t>((int64_t)G + 2, B)), (unsigned)S);
+  recommend_subset_kernel<T, TU><<<grid, kRtThreads, rs_smem_bytes(TU, d), s>>>(
+      reinterpret_cast<const T*>(U), nU, reinterpret_cast<const T*>(V), nI, d, uids, B, sub_ptr, sub_idx, G, rows_at,
+      blocks_at, order, seen_ptr, seen_idx, K, S, partial, out_ids, out_scores, err);
+  YR_CHECK_LAUNCH();
+  return YR_OK;
+}
+
+int rs_splits(int64_t B, int64_t max_len, int K) {
+  int64_t per = 0;
+  return rt_splits(B, std::max<int64_t>(max_len, 1), K, yr_sm_count(), &per);
+}
+
+size_t rs_partial_bytes(int S, int64_t B, int K) { return S > 1 ? (size_t)S * (size_t)B * (size_t)K * sizeof(uint64_t) : 0; }
+
+int merge_launch(const uint64_t* partial, int S, int64_t B, int K, int64_t* out_ids, float* out_scores, cudaStream_t s) {
+  const int P = rt_pow2(S * K);
+  static AttrOnce attr;
+  int rc = attr.set(recommend_merge_kernel, kRtMergeMax * (int)sizeof(uint64_t));
+  if (rc) return rc;
+  recommend_merge_kernel<<<(unsigned)B, kRtThreads, (size_t)P * sizeof(uint64_t), s>>>(partial, S, B, K, P, out_ids,
+                                                                                     out_scores);
+  YR_CHECK_LAUNCH();
+  return YR_OK;
+}
+
 }  // namespace
 
 extern "C" size_t yr_recommend_ws_bytes(int64_t B, int64_t nI, int K) {
@@ -346,12 +652,53 @@ extern "C" int yr_recommend_topk(const void* U, int64_t nU, const void* V, int64
                                                           : YR_RT_LAUNCH(__nv_bfloat16, 4);
 #undef YR_RT_LAUNCH
   if (rc || S == 1) return rc;
-  const int P = rt_pow2(S * K);
-  static AttrOnce attr;
-  rc = attr.set(recommend_merge_kernel, kRtMergeMax * (int)sizeof(uint64_t));
-  if (rc) return rc;
-  recommend_merge_kernel<<<(unsigned)B, kRtThreads, (size_t)P * sizeof(uint64_t), s>>>(partial, S, B, K, P, out_ids,
-                                                                                     out_scores);
+  return merge_launch(partial, S, B, K, out_ids, out_scores, s);
+}
+
+extern "C" size_t yr_recommend_subset_ws_bytes(int64_t B, int G, int64_t max_subset_len, int K) {
+  if (B <= 0 || G < 0 || K <= 0 || K > kRtMaxK) return 0;
+  const size_t plan = ((size_t)3 * G + 8 + (size_t)B) * sizeof(int32_t);
+  return rs_partial_bytes(rs_splits(B, max_subset_len, K), B, K) + plan;
+}
+
+extern "C" int yr_recommend_subset_topk(const void* U, int64_t nU, const void* V, int64_t nI, int d, int dtype,
+                                        const int64_t* user_ids, int64_t B, const int32_t* subset_ptr,
+                                        const int32_t* subset_idx, int G, int64_t max_subset_len,
+                                        const int64_t* subset_ids, const int32_t* seen_ptr, const int32_t* seen_idx, int K,
+                                        int64_t* out_ids, float* out_scores, void* ws, size_t ws_bytes, int32_t* err,
+                                        yr_stream stream) {
+  if (!U || !V || !out_ids || !out_scores || !subset_ptr || !subset_idx) return YR_ERR_BAD_ARG;
+  if (B > 0 && (!user_ids || !subset_ids)) return YR_ERR_BAD_ARG;
+  if ((seen_ptr == nullptr) != (seen_idx == nullptr)) return YR_ERR_BAD_ARG;
+  if (B < 0 || B >= 0x7fffffffLL || G < 0 || G >= 0x7ffffff0 || max_subset_len < 0 || nU <= 0 || K <= 0 ||
+      K > kRtMaxK)
+    return YR_ERR_BAD_ARG;
+  if (nI <= 0 || nI >= 0x7fffffffLL || d <= 0 || d > kRtMaxD || (d & 7) != 0) return YR_ERR_BAD_DIM;
+  if (dtype != YR_DTYPE_F32 && dtype != YR_DTYPE_BF16) return YR_ERR_BAD_ARG;
+  if (B == 0) return YR_OK;
+  if (!ws || ws_bytes < yr_recommend_subset_ws_bytes(B, G, max_subset_len, K)) return YR_ERR_WORKSPACE;
+  cudaStream_t s = (cudaStream_t)stream;
+  const int S = rs_splits(B, max_subset_len, K);
+  const size_t pbytes = rs_partial_bytes(S, B, K);
+  uint64_t* partial = S > 1 ? reinterpret_cast<uint64_t*>(ws) : nullptr;
+  int32_t* cursor = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(ws) + pbytes);   // [G + 2]
+  int32_t* rows_at = cursor + G + 2;                                                      // [G + 3]
+  int32_t* blocks_at = rows_at + G + 3;                                                   // [G + 3]
+  int32_t* order = blocks_at + G + 3;                                                     // [B]
+  const int TU = rt_users_per_block(K);
+  recommend_subset_plan_kernel<<<1, kRsPlanThreads, 0, s>>>(subset_ids, (int)B, G, TU, cursor, rows_at, blocks_at, order,
+                                                            err);
   YR_CHECK_LAUNCH();
-  return YR_OK;
+  int rc;
+#define YR_RS_LAUNCH(T, TU_)                                                                                              \
+  rs_launch<T, TU_>(U, nU, V, nI, d, user_ids, B, subset_ptr, subset_idx, G, rows_at, blocks_at, order, seen_ptr,        \
+                    seen_idx, K, S, partial, out_ids, out_scores, err, s)
+  if (dtype == YR_DTYPE_F32)
+    rc = TU == 16 ? YR_RS_LAUNCH(float, 16) : TU == 8 ? YR_RS_LAUNCH(float, 8) : YR_RS_LAUNCH(float, 4);
+  else
+    rc = TU == 16 ? YR_RS_LAUNCH(__nv_bfloat16, 16) : TU == 8 ? YR_RS_LAUNCH(__nv_bfloat16, 8)
+                                                          : YR_RS_LAUNCH(__nv_bfloat16, 4);
+#undef YR_RS_LAUNCH
+  if (rc || S == 1) return rc;
+  return merge_launch(partial, S, B, K, out_ids, out_scores, s);
 }

@@ -677,3 +677,86 @@ def recommend_topk(U: torch.Tensor, V: torch.Tensor, user_ids: torch.Tensor, K: 
     if int(err.item()) != 0:
         raise IndexError(f"recommend_topk: user id out of range [0, {nU})")
     return ids, scores
+
+
+def recommend_subset_topk(U: torch.Tensor, V: torch.Tensor, user_ids: torch.Tensor, K: int, subset_ptr: torch.Tensor,
+                          subset_idx: torch.Tensor, subset_ids: torch.Tensor, max_len: int,
+                          seen_ptr: Optional[torch.Tensor] = None,
+                          seen_idx: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """yr_recommend_subset_topk: recommend_topk with row b restricted to the items of subset subset_ids[b] (-1 = the whole
+    catalog). Subsets: CSR int32 (subset_ptr [G + 1], subset_idx ascending per subset). max_len: the longest list a row
+    streams (the longest subset, num_items if a row is -1); it sets only the number of item splits. Seen lists are indexed
+    by user id. (ids int64 [B x K], scores float32 [B x K]), identical to recommend_topk with the items outside each row's
+    subset excluded."""
+    if not (torch.is_tensor(subset_ptr) and torch.is_tensor(subset_idx) and torch.is_tensor(subset_ids)):
+        raise TypeError("recommend_subset_topk: subset_ptr, subset_idx and subset_ids must be tensors")
+    if not (torch.is_tensor(U) and torch.is_tensor(V) and torch.is_tensor(user_ids)):
+        raise TypeError("recommend_subset_topk: U, V and user_ids must be tensors")
+    if not (U.is_cuda and V.is_cuda and user_ids.is_cuda):
+        raise YelprecError("recommend_subset_topk: U, V and user_ids must be CUDA tensors (the reference path is "
+                           "retrieval.recommend_reference)")
+    dev = U.device
+    if V.device != dev or user_ids.device != dev:
+        raise ValueError(f"recommend_subset_topk: tensors on different devices ({U.device}, {V.device}, {user_ids.device})")
+    if U.dtype not in _RT_DTYPES or V.dtype != U.dtype:
+        raise TypeError(f"recommend_subset_topk: U and V must both be float32 or both bfloat16, got {U.dtype} and {V.dtype}")
+    if U.dim() != 2 or V.dim() != 2 or U.shape[1] != V.shape[1]:
+        raise ValueError(f"recommend_subset_topk: U [nU x d] and V [nI x d] expected, got {tuple(U.shape)} and "
+                         f"{tuple(V.shape)}")
+    d = int(U.shape[1])
+    if d % 8 != 0 or d > RECOMMEND_MAX_D:
+        raise ValueError(f"recommend_subset_topk: embedding width {d} must be a multiple of 8 and at most {RECOMMEND_MAX_D}")
+    nU, nI = int(U.shape[0]), int(V.shape[0])
+    if nU == 0 or nI == 0 or nI >= 2 ** 31 - 1:
+        raise ValueError(f"recommend_subset_topk: {nU} users x {nI} items is not a valid catalog")
+    if isinstance(K, bool) or int(K) != K or not 1 <= int(K) <= RECOMMEND_MAX_K:
+        raise ValueError(f"recommend_subset_topk: k must be an integer in [1, {RECOMMEND_MAX_K}], got {K}")
+    K = int(K)
+    if user_ids.dtype not in (I64, I32) or user_ids.dim() != 1:
+        raise TypeError(f"recommend_subset_topk: user_ids must be a 1-D int64 or int32 tensor, got {user_ids.dtype} "
+                        f"{tuple(user_ids.shape)}")
+    B = int(user_ids.numel())
+    if subset_ids.dtype not in (I64, I32) or subset_ids.dim() != 1:
+        raise TypeError(f"recommend_subset_topk: subset_ids must be a 1-D int64 or int32 tensor, got {subset_ids.dtype} "
+                        f"{tuple(subset_ids.shape)}")
+    if subset_ids.numel() != B:
+        raise ValueError(f"recommend_subset_topk: {subset_ids.numel()} subset ids for {B} users")
+    if subset_ptr.dtype != I32 or subset_idx.dtype != I32 or subset_ptr.dim() != 1 or subset_ptr.numel() < 1:
+        raise ValueError("recommend_subset_topk: subsets must be an int32 CSR (subset_ptr [G + 1], subset_idx)")
+    if subset_ptr.device != dev or subset_idx.device != dev or subset_ids.device != dev:
+        raise ValueError("recommend_subset_topk: subsets and subset ids must live on the device of the embeddings")
+    G = int(subset_ptr.numel()) - 1
+    if isinstance(max_len, bool) or int(max_len) != max_len or int(max_len) < 0:
+        raise ValueError(f"recommend_subset_topk: max_len must be a non-negative integer, got {max_len}")
+    if (seen_ptr is None) != (seen_idx is None):
+        raise ValueError("recommend_subset_topk: seen_ptr and seen_idx go together")
+    if seen_ptr is not None:
+        if seen_ptr.dtype != I32 or seen_idx.dtype != I32 or seen_ptr.numel() != nU + 1:
+            raise ValueError(f"recommend_subset_topk: seen lists must be int32 CSR with {nU + 1} offsets")
+        if seen_ptr.device != dev or seen_idx.device != dev:
+            raise ValueError("recommend_subset_topk: seen lists must live on the device of the embeddings")
+        seen_ptr = seen_ptr.contiguous()
+        seen_idx = seen_idx.contiguous() if seen_idx.numel() else torch.zeros(1, dtype=I32, device=dev)
+    uid = user_ids.to(I64).contiguous()
+    sid = subset_ids.to(I64).contiguous()
+    sptr = subset_ptr.contiguous()
+    sidx = subset_idx.contiguous() if subset_idx.numel() else torch.zeros(1, dtype=I32, device=dev)
+    lib = _cabi.load()
+    Uc, Vc = U.detach().contiguous(), V.detach().contiguous()
+    ids = torch.empty(B, K, device=dev, dtype=I64)
+    scores = torch.empty(B, K, device=dev, dtype=F32)
+    if B == 0:
+        return ids, scores
+    err = torch.zeros(1, device=dev, dtype=I32)
+    nbytes = lib.yr_recommend_subset_ws_bytes(B, G, int(max_len), K)
+    ws = torch.empty(max(nbytes, 1), device=dev, dtype=torch.uint8)
+    check(lib.yr_recommend_subset_topk(Uc.data_ptr(), nU, Vc.data_ptr(), nI, d, _RT_DTYPES[U.dtype], dptr(uid, I64), B,
+                                       dptr(sptr, I32), dptr(sidx, I32), G, int(max_len), dptr(sid, I64), dptr(seen_ptr),
+                                       dptr(seen_idx), K, dptr(ids), dptr(scores), dptr(ws), nbytes, dptr(err),
+                                       stream_ptr(dev)), "yr_recommend_subset_topk")
+    e = int(err.item())
+    if e & 1:
+        raise IndexError(f"recommend_subset_topk: user id out of range [0, {nU})")
+    if e & 2:
+        raise IndexError(f"recommend_subset_topk: subset id out of range [-1, {G})")
+    return ids, scores
