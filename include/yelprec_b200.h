@@ -426,6 +426,17 @@ int yr_cdae_hidden_ex(const yr_cdae_tensors* P, int64_t nU, int64_t nI, int h, i
                       const float* x, const float* keep, int64_t B, float* z_out, int64_t ldz, void* ws, size_t ws_bytes,
                       int32_t* err, yr_stream stream);
 
+/* The hidden activations of yr_cdae_hidden_ex (keep == NULL) from interaction lists instead of a dense multi-hot:
+ * z[b, 0:h] = act(bh + Vu[u] + sum over j in in_idx[in_ptr[u] .. in_ptr[u + 1]) of Wh[:, j]), u = user_ids[b]. The lists are
+ * a CSR indexed by user id (nU + 1 offsets, ascending unique item ids per row) and Wh is read in place; nothing of size
+ * B x nI is needed. Bit-identical to yr_cdae_hidden_ex on the dense multi-hot of the same lists. Columns h..ldz-1 of z
+ * are not written. A user id outside [0, nU) sets *err |= 1 and the row is computed for user 0; an item id outside
+ * [0, nI), or offsets that decrease or run past in_ptr[nU], set *err |= 2 and the row is computed from an empty list.
+ * Nothing is read out of bounds. h as yr_cdae_hidden_ex. */
+int yr_cdae_encode(const yr_cdae_tensors* P, int64_t nU, int64_t nI, int h, int hidden_act, const int64_t* user_ids,
+                   int64_t B, const int32_t* in_ptr, const int32_t* in_idx, float* z, int64_t ldz, int32_t* err,
+                   yr_stream stream);
+
 /* pred[b,i] = sigmoid( z[b,:] . Wo[i,:] + bo[i] )  — CDAE.forward's dense output (models/cdae.py:52). */
 int yr_cdae_output(const yr_cdae_tensors* P, int64_t nI, int h, const float* z, int64_t ldz, int64_t B,
                    float* pred, yr_stream stream);
@@ -564,13 +575,20 @@ enum yr_dtype { YR_DTYPE_F32 = 0, YR_DTYPE_BF16 = 1 };
  * (seen_by_row = 0, nU + 1 offsets) or by the batch row b (seen_by_row = 1, B + 1 offsets). A seen item scores
  * masked_score instead: -INFINITY excludes it. Items scoring -inf or NaN are never returned; a row with fewer than K
  * returnable items is padded with id -1 / score -inf. A user id outside [0, nU) sets *err = 1 (err may be NULL) and
- * gets an all-padding row. 1 <= K <= 1024, d % 8 == 0, d <= 512, nI < 2^31 - 1.
+ * gets an all-padding row. 1 <= K <= 1024, d % 8 == 0, d <= 1024, nI < 2^31 - 1.
  * ws: yr_recommend_ws_bytes(B, nI, K) bytes (0 = none needed; same device as the call). */
 size_t yr_recommend_ws_bytes(int64_t B, int64_t nI, int K);
 int yr_recommend_topk(const void* U, int64_t nU, const void* V, int64_t nI, int d, int dtype, const int64_t* user_ids,
                       int64_t B, const int32_t* seen_ptr, const int32_t* seen_idx, int seen_by_row, float masked_score,
                       int K, int64_t* out_ids, float* out_scores, void* ws, size_t ws_bytes, int32_t* err,
                       yr_stream stream);
+/* Same with a per-item bias: item_bias [nI] fp32 (for fp32 and bf16 tables; NULL = none) makes the score
+ * U[uid] . V[i] + item_bias[i], the bias added after the fma chain, before seen items are masked. That equals, bit for bit,
+ * the unbiased call on the tables [U | 1 | 0...] and [V | item_bias | 0...]. */
+int yr_recommend_topk_ex(const void* U, int64_t nU, const void* V, int64_t nI, int d, int dtype, const int64_t* user_ids,
+                         int64_t B, const int32_t* seen_ptr, const int32_t* seen_idx, int seen_by_row, float masked_score,
+                         int K, int64_t* out_ids, float* out_scores, void* ws, size_t ws_bytes, int32_t* err,
+                         yr_stream stream, const float* item_bias);
 
 /* yr_recommend_topk restricted per row to one subset of the catalog. The G subsets are a CSR of item ids: subset g is
  * subset_idx[subset_ptr[g] .. subset_ptr[g + 1]), ascending and duplicate-free; subsets may overlap. Row b ranks only the
@@ -588,6 +606,12 @@ int yr_recommend_subset_topk(const void* U, int64_t nU, const void* V, int64_t n
                              int G, int64_t max_subset_len, const int64_t* subset_ids, const int32_t* seen_ptr,
                              const int32_t* seen_idx, int K, int64_t* out_ids, float* out_scores, void* ws,
                              size_t ws_bytes, int32_t* err, yr_stream stream);
+/* Same with a per-item bias, as yr_recommend_topk_ex. */
+int yr_recommend_subset_topk_ex(const void* U, int64_t nU, const void* V, int64_t nI, int d, int dtype,
+                                const int64_t* user_ids, int64_t B, const int32_t* subset_ptr, const int32_t* subset_idx,
+                                int G, int64_t max_subset_len, const int64_t* subset_ids, const int32_t* seen_ptr,
+                                const int32_t* seen_idx, int K, int64_t* out_ids, float* out_scores, void* ws,
+                                size_t ws_bytes, int32_t* err, yr_stream stream, const float* item_bias);
 
 #ifdef __cplusplus
 }

@@ -34,6 +34,7 @@ SYMBOLS = (
     "yr_synth_user_rows", "yr_laplacian_binary_values",
     "yr_split_ws_bytes", "yr_split_sizes", "yr_split_per_user",
     "yr_recommend_ws_bytes", "yr_recommend_topk", "yr_recommend_subset_ws_bytes", "yr_recommend_subset_topk",
+    "yr_recommend_topk_ex", "yr_recommend_subset_topk_ex", "yr_cdae_encode",
 )
 
 YR_OPT_SGD, YR_OPT_ADAM, YR_OPT_ADAMW = 0, 1, 2
@@ -204,6 +205,10 @@ def load() -> C.CDLL:
         "yr_recommend_subset_ws_bytes": (sz, [i64, i32, i64, i32]),
         "yr_recommend_subset_topk": (C.c_int, [p, i64, p, i64, i32, i32, p, i64, p, p, i32, i64, p, p, p, i32, p, p, p,
                                                sz, p, p]),
+        "yr_recommend_topk_ex": (C.c_int, [p, i64, p, i64, i32, i32, p, i64, p, p, i32, f32, i32, p, p, p, sz, p, p, p]),
+        "yr_recommend_subset_topk_ex": (C.c_int, [p, i64, p, i64, i32, i32, p, i64, p, p, i32, i64, p, p, p, i32, p, p,
+                                                  p, sz, p, p, p]),
+        "yr_cdae_encode": (C.c_int, [C.POINTER(YrCdaeTensors), i64, i64, i32, i32, p, i64, p, p, p, i64, p, p]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)

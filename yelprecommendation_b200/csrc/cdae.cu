@@ -166,6 +166,37 @@ cdae_lists_kernel(const int32_t* __restrict__ in_ptr, const int32_t* __restrict_
 
 __device__ __forceinline__ float sigmoidf_(float x) { return 1.f / (1.f + expf(-x)); }
 
+// Hidden layer, phase 1: part[g][k] = sum over j = g, g + G, ... < nx of xv[j] * Wh[k, xi[j]], one fma chain each
+// (G partial sums per unit, KS units per pass of the CTA). xv: the input values, or CdaeOnes for a multi-hot list.
+template <int H, int G, int KS, typename XV>
+__device__ __forceinline__ void cdae_hidden_part(int tid, const float* Wh, int64_t nI, const int32_t* xi, XV xv, int nx,
+                                                 float (*part)[H]) {
+  const int g = tid / KS;
+  for (int k = tid % KS; k < H; k += KS) {
+    float acc = 0.f;
+    for (int j = g; j < nx; j += G) acc = fmaf(xv[j], __ldg(Wh + (int64_t)k * nI + xi[j]), acc);
+    part[g][k] = acc;
+  }
+}
+
+// Hidden layer, phase 2 for unit k: act(pre + the G partial sums), pre = bh[k] + Vu[u, k].
+template <int H, int G>
+__device__ __forceinline__ float cdae_hidden_unit(const float (*part)[H], int k, float pre, int act) {
+  if constexpr (G == 4) {
+    pre += (part[0][k] + part[1][k]) + (part[2][k] + part[3][k]);
+  } else {
+    float t = part[0][k];
+#pragma unroll
+    for (int g = 1; g < G; ++g) t += part[g][k];
+    pre += t;
+  }
+  return act ? pre : sigmoidf_(pre);
+}
+
+struct CdaeOnes {
+  __device__ __forceinline__ float operator[](int) const { return 1.f; }
+};
+
 // Block per batch row. H = 32 * VPL = hidden size (32 ... 1,024: the values of the reference's cdae_sweep_config.yaml).
 // Phase 1: hidden activation (act: 0 sigmoid, 1 identity — models/base_model.py:10-14) from the compacted inputs.
 // Phase 2 (targets given): logits at the loss positions, BCE terms, and — if GRAD — every gradient.
@@ -190,26 +221,10 @@ cdae_row_kernel(yr_cdae_tensors P, yr_cdae_tensors Gr, int64_t nU, int64_t nI, c
   const float* xv = w.xin_val + (int64_t)b * nI;
 
   // ---- hidden: z = act(bh + Vu[u] + sum_j xv_j * Wh[:, xi_j]) ; thread = (group g of G, unit k)
-  {
-    const int g = tid / KS;
-    for (int k = tid % KS; k < H; k += KS) {
-      float acc = 0.f;
-      for (int j = g; j < nx; j += G) acc = fmaf(xv[j], __ldg(P.Wh + (int64_t)k * nI + xi[j]), acc);
-      part[g][k] = acc;
-    }
-  }
+  cdae_hidden_part<H, G, KS>(tid, P.Wh, nI, xi, xv, nx, part);
   __syncthreads();
   for (int k = tid; k < H; k += kCdaeThreads) {
-    float pre = P.bh[k] + P.Vu[u * H + k];
-    if constexpr (G == 4) {
-      pre += (part[0][k] + part[1][k]) + (part[2][k] + part[3][k]);
-    } else {
-      float t = part[0][k];
-#pragma unroll
-      for (int g = 1; g < G; ++g) t += part[g][k];
-      pre += t;
-    }
-    const float z = act ? pre : sigmoidf_(pre);
+    const float z = cdae_hidden_unit<H, G>(part, k, P.bh[k] + P.Vu[u * H + k], act);
     z_s[k] = z;
     w.z[(int64_t)b * H + k] = z;
     if (z_out) z_out[(int64_t)b * ldz + k] = z;
@@ -291,6 +306,37 @@ cdae_row_kernel(yr_cdae_tensors P, yr_cdae_tensors Gr, int64_t nU, int64_t nI, c
       for (int j = g; j < nx; j += G) atomicAdd(Gr.Wh + (int64_t)k * nI + xi[j], dpre * xv[j]);
     }
   }
+}
+
+// Block per batch row: the hidden activations from the row's interaction list (a CSR indexed by user id), with the
+// arithmetic of cdae_row_kernel's phase 1 on the dense multi-hot of the same list.
+template <int VPL>
+__global__ void __launch_bounds__(kCdaeThreads)
+cdae_encode_kernel(yr_cdae_tensors P, int64_t nU, int64_t nI, const int64_t* __restrict__ uid,
+                   const int32_t* __restrict__ in_ptr, const int32_t* __restrict__ in_idx, float* __restrict__ z,
+                   int64_t ldz, int32_t* err, int act) {
+  constexpr int H = VPL * 32;
+  constexpr int G = H >= kCdaeThreads ? 1 : kCdaeThreads / H;
+  constexpr int KS = H >= kCdaeThreads ? kCdaeThreads : H;
+  __shared__ float part[G][H];
+  const int b = blockIdx.x, tid = threadIdx.x;
+  int64_t u = uid[b];
+  if (u < 0 || u >= nU) { if (tid == 0 && err) atomicOr(err, 1); u = 0; }
+  const int64_t i0 = in_ptr[u], i1 = in_ptr[u + 1];
+  bool bad = i0 < 0 || i1 < i0 || i1 > in_ptr[nU];
+  const int32_t* xi = in_idx + (bad ? 0 : i0);
+  int nx = bad ? 0 : (int)(i1 - i0);
+  int out = 0;                                                  // every id checked before any is used as a column
+  for (int j = tid; j < nx; j += kCdaeThreads) out |= (xi[j] < 0) | (xi[j] >= nI);
+  bad = __syncthreads_or(out) || bad;
+  if (bad) {
+    nx = 0;
+    if (tid == 0 && err) atomicOr(err, 2);
+  }
+  cdae_hidden_part<H, G, KS>(tid, P.Wh, nI, xi, CdaeOnes{}, nx, part);
+  __syncthreads();
+  for (int k = tid; k < H; k += kCdaeThreads)
+    z[(int64_t)b * ldz + k] = cdae_hidden_unit<H, G>(part, k, P.bh[k] + P.Vu[u * H + k], act);
 }
 
 template <bool GRAD>
@@ -383,6 +429,31 @@ extern "C" int yr_cdae_hidden_ex(const yr_cdae_tensors* P, int64_t nU, int64_t n
   YR_CHECK_LAUNCH();
   yr_cdae_tensors none = {};
   return launch_cdae_row<false>(h, B, s, *P, none, nU, nI, uid, w, false, z_out, ldz, nullptr, err, hidden_act);
+}
+
+extern "C" int yr_cdae_encode(const yr_cdae_tensors* P, int64_t nU, int64_t nI, int h, int hidden_act,
+                              const int64_t* user_ids, int64_t B, const int32_t* in_ptr, const int32_t* in_idx, float* z,
+                              int64_t ldz, int32_t* err, yr_stream stream) {
+  if (cdae_tensors_ok(P) || !user_ids || !in_ptr || !in_idx || !z || B < 0 || nU <= 0 || nI <= 0 || ldz < h)
+    return YR_ERR_BAD_ARG;
+  if (hidden_act != YR_ACT_SIGMOID && hidden_act != YR_ACT_IDENTITY) return YR_ERR_BAD_ARG;
+  if (!dim_vpl(h)) return YR_ERR_BAD_DIM;
+  if (B == 0) return YR_OK;
+  cudaStream_t s = (cudaStream_t)stream;
+#define YR_CDAE_ENCODE(V) \
+  cdae_encode_kernel<V><<<(unsigned)B, kCdaeThreads, 0, s>>>(*P, nU, nI, user_ids, in_ptr, in_idx, z, ldz, err, hidden_act)
+  switch (dim_vpl(h)) {
+    case 1: YR_CDAE_ENCODE(1); break;
+    case 2: YR_CDAE_ENCODE(2); break;
+    case 4: YR_CDAE_ENCODE(4); break;
+    case 8: YR_CDAE_ENCODE(8); break;
+    case 16: YR_CDAE_ENCODE(16); break;
+    case 32: YR_CDAE_ENCODE(32); break;
+    default: return YR_ERR_BAD_DIM;
+  }
+#undef YR_CDAE_ENCODE
+  YR_CHECK_LAUNCH();
+  return YR_OK;
 }
 
 extern "C" int yr_cdae_output(const yr_cdae_tensors* P, int64_t nI, int h, const float* z, int64_t ldz, int64_t B,

@@ -12,6 +12,9 @@
 //
 // recommend_subset_kernel restricts each row to one subset of the catalog (an ascending item-id list): the same scores,
 // masking and selection over the gathered ids of the row's subset, with rows grouped by subset on the device first.
+//
+// The _bias kernels add a per-item fp32 bias to each score after the fma chain (a CDAE output layer: z . W_o[i] + b_o[i]);
+// they share their bodies with the unbiased kernels, whose code the bias does not touch.
 #include <float.h>
 #include <algorithm>
 #include <cuda_bf16.h>
@@ -23,7 +26,8 @@ constexpr int kRtThreads = 256;
 constexpr int kRtTile = 256;         // items per tile, one per thread
 constexpr int kRtEntries = 8192;     // candidate keys per block: TU users x (kRtEntries / TU)
 constexpr int kRtMaxK = 1024;
-constexpr int kRtMaxD = 512;
+constexpr int kRtMaxD = 1024;
+constexpr int kRtMaxUD = 16 * 512;   // TU x d at most: wider tables take fewer users per block (see rt_users)
 constexpr int kRtMinSplit = 4096;    // items per split at least: long enough for the thresholds to settle
 constexpr int kRtMergeMax = 16384;   // keys one merge block sorts (128 KB of shared memory)
 
@@ -129,13 +133,14 @@ __device__ __forceinline__ void rt_offer(uint64_t* keys, int* cnt, const uint64_
   }
 }
 
-template <typename T, int TU>
-__global__ void __launch_bounds__(kRtThreads)
-recommend_topk_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ V, int64_t nI, int d,
-                      const int64_t* __restrict__ uids, int64_t B, const int32_t* __restrict__ seen_ptr,
-                      const int32_t* __restrict__ seen_idx, int seen_by_row, float masked_score, int K, int64_t per_split,
-                      uint64_t* __restrict__ partial, int64_t* __restrict__ out_ids, float* __restrict__ out_scores,
-                      int32_t* err) {
+// The body of recommend_topk_kernel (kBias = false) and recommend_topk_bias_kernel (kBias: score + item_bias[item]).
+template <typename T, int TU, bool kBias>
+__device__ __forceinline__ void
+recommend_topk_body(const T* __restrict__ U, int64_t nU, const T* __restrict__ V, int64_t nI, int d,
+                    const int64_t* __restrict__ uids, int64_t B, const int32_t* __restrict__ seen_ptr,
+                    const int32_t* __restrict__ seen_idx, int seen_by_row, float masked_score, int K, int64_t per_split,
+                    uint64_t* __restrict__ partial, int64_t* __restrict__ out_ids, float* __restrict__ out_scores,
+                    int32_t* err, const float* __restrict__ item_bias) {
   constexpr int CAP = kRtEntries / TU;
   constexpr int kWords = kRtTile / 32;
   extern __shared__ __align__(16) uint64_t rt_smem[];
@@ -233,9 +238,12 @@ recommend_topk_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__
     }
     __syncthreads();   // bitmask complete
     if (have) {
+      float bias = 0.f;
+      if constexpr (kBias) bias = __ldg(item_bias + item);
 #pragma unroll
       for (int u = 0; u < TU; ++u) {
         float s = acc[u];
+        if constexpr (kBias) s += bias;
         if (seen_ptr && ((bits[u * kWords + warp] >> lane) & 1u)) s = masked_score;
         if (s == 0.f) s = 0.f;                       // -0 ranks like +0
         if (!(s > -INFINITY)) continue;              // excluded (-inf) or NaN: never returned
@@ -268,6 +276,28 @@ recommend_topk_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__
       out_scores[b * K + j] = s;
     }
   }
+}
+
+template <typename T, int TU>
+__global__ void __launch_bounds__(kRtThreads)
+recommend_topk_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ V, int64_t nI, int d,
+                      const int64_t* __restrict__ uids, int64_t B, const int32_t* __restrict__ seen_ptr,
+                      const int32_t* __restrict__ seen_idx, int seen_by_row, float masked_score, int K, int64_t per_split,
+                      uint64_t* __restrict__ partial, int64_t* __restrict__ out_ids, float* __restrict__ out_scores,
+                      int32_t* err) {
+  recommend_topk_body<T, TU, false>(U, nU, V, nI, d, uids, B, seen_ptr, seen_idx, seen_by_row, masked_score, K, per_split,
+                                    partial, out_ids, out_scores, err, nullptr);
+}
+
+template <typename T, int TU>
+__global__ void __launch_bounds__(kRtThreads)
+recommend_topk_bias_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ V, int64_t nI, int d,
+                           const int64_t* __restrict__ uids, int64_t B, const int32_t* __restrict__ seen_ptr,
+                           const int32_t* __restrict__ seen_idx, int seen_by_row, float masked_score, int K,
+                           int64_t per_split, uint64_t* __restrict__ partial, int64_t* __restrict__ out_ids,
+                           float* __restrict__ out_scores, int32_t* err, const float* __restrict__ item_bias) {
+  recommend_topk_body<T, TU, true>(U, nU, V, nI, d, uids, B, seen_ptr, seen_idx, seen_by_row, masked_score, K, per_split,
+                                   partial, out_ids, out_scores, err, item_bias);
 }
 
 // Row b: the K best of the S per-split lists partial[s][b][0..K).
@@ -387,15 +417,16 @@ recommend_subset_plan_kernel(const int64_t* __restrict__ subset_ids, int B, int 
 // Grid (upper bound on the plan's block count, S). Block x takes TU rows of one group and split y of the group's list:
 // a slice of at least kRtMinSplit ids (a multiple of the tile) so that groups shorter than the longest use fewer splits;
 // a split past the end of its list writes padding keys.
-template <typename T, int TU>
-__global__ void __launch_bounds__(kRtThreads, 2)   // 2 blocks an SM: up to 128 registers, no spills
-recommend_subset_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ V, int64_t nI, int d,
-                        const int64_t* __restrict__ uids, int64_t B, const int32_t* __restrict__ sub_ptr,
-                        const int32_t* __restrict__ sub_idx, int G, const int32_t* __restrict__ rows_at,
-                        const int32_t* __restrict__ blocks_at, const int32_t* __restrict__ order,
-                        const int32_t* __restrict__ seen_ptr, const int32_t* __restrict__ seen_idx, int K, int S,
-                        uint64_t* __restrict__ partial, int64_t* __restrict__ out_ids, float* __restrict__ out_scores,
-                        int32_t* err) {
+// kBias: score + item_bias[item] (recommend_subset_bias_kernel).
+template <typename T, int TU, bool kBias>
+__device__ __forceinline__ void
+recommend_subset_body(const T* __restrict__ U, int64_t nU, const T* __restrict__ V, int64_t nI, int d,
+                      const int64_t* __restrict__ uids, int64_t B, const int32_t* __restrict__ sub_ptr,
+                      const int32_t* __restrict__ sub_idx, int G, const int32_t* __restrict__ rows_at,
+                      const int32_t* __restrict__ blocks_at, const int32_t* __restrict__ order,
+                      const int32_t* __restrict__ seen_ptr, const int32_t* __restrict__ seen_idx, int K, int S,
+                      uint64_t* __restrict__ partial, int64_t* __restrict__ out_ids, float* __restrict__ out_scores,
+                      int32_t* err, const float* __restrict__ item_bias) {
   constexpr int CAP = kRtEntries / TU;
   constexpr int kWords = kRtTile / 32;
   extern __shared__ __align__(16) uint64_t rt_smem[];
@@ -496,10 +527,12 @@ recommend_subset_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict
       rt_score<T, TU>(have ? V + (int64_t)item * d : nullptr, Us, d, acc);
       __syncthreads();   // bitmask complete, tile ids consumed
       if (have) {
+        float bias = 0.f;
+        if constexpr (kBias) bias = __ldg(item_bias + item);
 #pragma unroll
         for (int u = 0; u < TU; ++u) {
           if (seen_ptr && ((bits[u * kWords + warp] >> lane) & 1u)) continue;
-          rt_offer<TU>(keys, cnt, thr, u, acc[u], (uint32_t)item);
+          rt_offer<TU>(keys, cnt, thr, u, kBias ? acc[u] + bias : acc[u], (uint32_t)item);
         }
       }
       __syncthreads();
@@ -526,6 +559,32 @@ recommend_subset_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict
   }
 }
 
+template <typename T, int TU>
+__global__ void __launch_bounds__(kRtThreads, 2)   // 2 blocks an SM: up to 128 registers, no spills
+recommend_subset_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ V, int64_t nI, int d,
+                        const int64_t* __restrict__ uids, int64_t B, const int32_t* __restrict__ sub_ptr,
+                        const int32_t* __restrict__ sub_idx, int G, const int32_t* __restrict__ rows_at,
+                        const int32_t* __restrict__ blocks_at, const int32_t* __restrict__ order,
+                        const int32_t* __restrict__ seen_ptr, const int32_t* __restrict__ seen_idx, int K, int S,
+                        uint64_t* __restrict__ partial, int64_t* __restrict__ out_ids, float* __restrict__ out_scores,
+                        int32_t* err) {
+  recommend_subset_body<T, TU, false>(U, nU, V, nI, d, uids, B, sub_ptr, sub_idx, G, rows_at, blocks_at, order, seen_ptr,
+                                      seen_idx, K, S, partial, out_ids, out_scores, err, nullptr);
+}
+
+template <typename T, int TU>
+__global__ void __launch_bounds__(kRtThreads, 2)
+recommend_subset_bias_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ V, int64_t nI, int d,
+                             const int64_t* __restrict__ uids, int64_t B, const int32_t* __restrict__ sub_ptr,
+                             const int32_t* __restrict__ sub_idx, int G, const int32_t* __restrict__ rows_at,
+                             const int32_t* __restrict__ blocks_at, const int32_t* __restrict__ order,
+                             const int32_t* __restrict__ seen_ptr, const int32_t* __restrict__ seen_idx, int K, int S,
+                             uint64_t* __restrict__ partial, int64_t* __restrict__ out_ids,
+                             float* __restrict__ out_scores, int32_t* err, const float* __restrict__ item_bias) {
+  recommend_subset_body<T, TU, true>(U, nU, V, nI, d, uids, B, sub_ptr, sub_idx, G, rows_at, blocks_at, order, seen_ptr,
+                                     seen_idx, K, S, partial, out_ids, out_scores, err, item_bias);
+}
+
 }  // namespace yr
 
 using namespace yr;
@@ -534,6 +593,14 @@ namespace {
 
 int rt_users_per_block(int K) { return K <= kRtEntries / 16 - kRtTile ? 16 : K <= kRtEntries / 8 - kRtTile ? 8 : 4; }
 
+// Users per block of a launch: for d > 512 at most 8, so that the staged user rows (TU x d floats) never take more shared
+// memory than 16 users at d = 512. Fewer users per block never means more item splits (rt_splits), so the workspace
+// queries, which take rt_users_per_block(K), stay upper bounds.
+int rt_users(int K, int d) { return d > kRtMaxUD / 16 ? std::min(rt_users_per_block(K), 8) : rt_users_per_block(K); }
+
+// The widest d a launch with TU users per block can have.
+int rt_max_d(int TU) { return std::min(kRtMaxD, kRtMaxUD / TU); }
+
 int rt_pow2(int x) {
   int p = 1;
   while (p < x) p <<= 1;
@@ -541,9 +608,8 @@ int rt_pow2(int x) {
 }
 
 // Item splits: enough blocks to give every SM a few, each split at least kRtMinSplit items (a multiple of the tile), and the
-// merge of S lists of K keys within one block's shared memory.
-int rt_splits(int64_t B, int64_t nI, int K, int sm, int64_t* per_split) {
-  const int TU = rt_users_per_block(K);
+// merge of S lists of K keys within one block's shared memory. TU: the users per block of the launch.
+int rt_splits(int64_t B, int64_t nI, int K, int TU, int sm, int64_t* per_split) {
   const int64_t bx = (B + TU - 1) / TU;
   int64_t S = (4 * (int64_t)sm + bx - 1) / bx;
   const int64_t by_len = nI / kRtMinSplit;
@@ -560,47 +626,73 @@ size_t rt_smem_bytes(int TU, int d) {
   return (size_t)kRtEntries * 8 + (size_t)TU * 8 + (size_t)TU * d * 4 + (size_t)TU * (kRtTile / 32) * 4 + 3 * (size_t)TU * 4;
 }
 
-template <typename T, int TU>
+template <typename T, int TU, bool kBias>
 int rt_launch(const void* U, int64_t nU, const void* V, int64_t nI, int d, const int64_t* uids, int64_t B,
               const int32_t* seen_ptr, const int32_t* seen_idx, int seen_by_row, float masked_score, int K, int S,
-              int64_t per_split, uint64_t* partial, int64_t* out_ids, float* out_scores, int32_t* err, cudaStream_t s) {
+              int64_t per_split, uint64_t* partial, int64_t* out_ids, float* out_scores, int32_t* err,
+              const float* item_bias, cudaStream_t s) {
   static AttrOnce attr;
   const size_t smem = rt_smem_bytes(TU, d);
-  int rc = attr.set(recommend_topk_kernel<T, TU>, (int)rt_smem_bytes(TU, kRtMaxD));
-  if (rc) return rc;
+  const int max_smem = (int)rt_smem_bytes(TU, rt_max_d(TU));
   dim3 grid((unsigned)((B + TU - 1) / TU), (unsigned)S);
-  recommend_topk_kernel<T, TU><<<grid, kRtThreads, smem, s>>>(
-      reinterpret_cast<const T*>(U), nU, reinterpret_cast<const T*>(V), nI, d, uids, B, seen_ptr, seen_idx, seen_by_row,
-      masked_score, K, per_split, partial, out_ids, out_scores, err);
+  const T* Ut = reinterpret_cast<const T*>(U);
+  const T* Vt = reinterpret_cast<const T*>(V);
+  if constexpr (kBias) {
+    int rc = attr.set(recommend_topk_bias_kernel<T, TU>, max_smem);
+    if (rc) return rc;
+    recommend_topk_bias_kernel<T, TU><<<grid, kRtThreads, smem, s>>>(Ut, nU, Vt, nI, d, uids, B, seen_ptr, seen_idx,
+                                                                     seen_by_row, masked_score, K, per_split, partial,
+                                                                     out_ids, out_scores, err, item_bias);
+  } else {
+    int rc = attr.set(recommend_topk_kernel<T, TU>, max_smem);
+    if (rc) return rc;
+    recommend_topk_kernel<T, TU><<<grid, kRtThreads, smem, s>>>(Ut, nU, Vt, nI, d, uids, B, seen_ptr, seen_idx,
+                                                                seen_by_row, masked_score, K, per_split, partial, out_ids,
+                                                                out_scores, err);
+  }
   YR_CHECK_LAUNCH();
   return YR_OK;
 }
 
 size_t rs_smem_bytes(int TU, int d) { return rt_smem_bytes(TU, d) + (size_t)TU * 4 + (size_t)kRtTile * 4; }
 
-template <typename T, int TU>
+template <typename T, int TU, bool kBias>
 int rs_launch(const void* U, int64_t nU, const void* V, int64_t nI, int d, const int64_t* uids, int64_t B,
               const int32_t* sub_ptr, const int32_t* sub_idx, int G, const int32_t* rows_at, const int32_t* blocks_at,
               const int32_t* order, const int32_t* seen_ptr, const int32_t* seen_idx, int K, int S, uint64_t* partial,
-              int64_t* out_ids, float* out_scores, int32_t* err, cudaStream_t s) {
+              int64_t* out_ids, float* out_scores, int32_t* err, const float* item_bias, cudaStream_t s) {
   static AttrOnce attr;
-  int rc = attr.set(recommend_subset_kernel<T, TU>, (int)rs_smem_bytes(TU, kRtMaxD));
-  if (rc) return rc;
+  const int max_smem = (int)rs_smem_bytes(TU, rt_max_d(TU));
   // the plan makes sum over groups of ceil(rows / TU) blocks: at most ceil(B / TU) + one per non-empty group
   dim3 grid((unsigned)((B + TU - 1) / TU + std::min<int64_t>((int64_t)G + 2, B)), (unsigned)S);
-  recommend_subset_kernel<T, TU><<<grid, kRtThreads, rs_smem_bytes(TU, d), s>>>(
-      reinterpret_cast<const T*>(U), nU, reinterpret_cast<const T*>(V), nI, d, uids, B, sub_ptr, sub_idx, G, rows_at,
-      blocks_at, order, seen_ptr, seen_idx, K, S, partial, out_ids, out_scores, err);
+  const size_t smem = rs_smem_bytes(TU, d);
+  const T* Ut = reinterpret_cast<const T*>(U);
+  const T* Vt = reinterpret_cast<const T*>(V);
+  if constexpr (kBias) {
+    int rc = attr.set(recommend_subset_bias_kernel<T, TU>, max_smem);
+    if (rc) return rc;
+    recommend_subset_bias_kernel<T, TU><<<grid, kRtThreads, smem, s>>>(Ut, nU, Vt, nI, d, uids, B, sub_ptr, sub_idx, G,
+                                                                       rows_at, blocks_at, order, seen_ptr, seen_idx, K,
+                                                                       S, partial, out_ids, out_scores, err, item_bias);
+  } else {
+    int rc = attr.set(recommend_subset_kernel<T, TU>, max_smem);
+    if (rc) return rc;
+    recommend_subset_kernel<T, TU><<<grid, kRtThreads, smem, s>>>(Ut, nU, Vt, nI, d, uids, B, sub_ptr, sub_idx, G,
+                                                                  rows_at, blocks_at, order, seen_ptr, seen_idx, K, S,
+                                                                  partial, out_ids, out_scores, err);
+  }
   YR_CHECK_LAUNCH();
   return YR_OK;
 }
 
-int rs_splits(int64_t B, int64_t max_len, int K) {
+int rs_splits(int64_t B, int64_t max_len, int K, int TU) {
   int64_t per = 0;
-  return rt_splits(B, std::max<int64_t>(max_len, 1), K, yr_sm_count(), &per);
+  return rt_splits(B, std::max<int64_t>(max_len, 1), K, TU, yr_sm_count(), &per);
 }
 
 size_t rs_partial_bytes(int S, int64_t B, int K) { return S > 1 ? (size_t)S * (size_t)B * (size_t)K * sizeof(uint64_t) : 0; }
+
+size_t rs_plan_bytes(int64_t B, int G) { return ((size_t)3 * G + 8 + (size_t)B) * sizeof(int32_t); }
 
 int merge_launch(const uint64_t* partial, int S, int64_t B, int K, int64_t* out_ids, float* out_scores, cudaStream_t s) {
   const int P = rt_pow2(S * K);
@@ -618,14 +710,22 @@ int merge_launch(const uint64_t* partial, int S, int64_t B, int K, int64_t* out_
 extern "C" size_t yr_recommend_ws_bytes(int64_t B, int64_t nI, int K) {
   if (B <= 0 || nI <= 0 || K <= 0 || K > kRtMaxK) return 0;
   int64_t per = 0;
-  const int S = rt_splits(B, nI, K, yr_sm_count(), &per);
-  return S > 1 ? (size_t)S * (size_t)B * (size_t)K * sizeof(uint64_t) : 0;
+  const int S = rt_splits(B, nI, K, rt_users_per_block(K), yr_sm_count(), &per);
+  return rs_partial_bytes(S, B, K);
 }
 
 extern "C" int yr_recommend_topk(const void* U, int64_t nU, const void* V, int64_t nI, int d, int dtype,
                                  const int64_t* user_ids, int64_t B, const int32_t* seen_ptr, const int32_t* seen_idx,
                                  int seen_by_row, float masked_score, int K, int64_t* out_ids, float* out_scores, void* ws,
                                  size_t ws_bytes, int32_t* err, yr_stream stream) {
+  return yr_recommend_topk_ex(U, nU, V, nI, d, dtype, user_ids, B, seen_ptr, seen_idx, seen_by_row, masked_score, K,
+                              out_ids, out_scores, ws, ws_bytes, err, stream, nullptr);
+}
+
+extern "C" int yr_recommend_topk_ex(const void* U, int64_t nU, const void* V, int64_t nI, int d, int dtype,
+                                    const int64_t* user_ids, int64_t B, const int32_t* seen_ptr, const int32_t* seen_idx,
+                                    int seen_by_row, float masked_score, int K, int64_t* out_ids, float* out_scores,
+                                    void* ws, size_t ws_bytes, int32_t* err, yr_stream stream, const float* item_bias) {
   if (!U || !V || !out_ids || !out_scores || (B > 0 && !user_ids)) return YR_ERR_BAD_ARG;
   if ((seen_ptr == nullptr) != (seen_idx == nullptr)) return YR_ERR_BAD_ARG;
   if (B < 0 || nU <= 0 || K <= 0 || K > kRtMaxK) return YR_ERR_BAD_ARG;
@@ -633,23 +733,25 @@ extern "C" int yr_recommend_topk(const void* U, int64_t nU, const void* V, int64
   if (dtype != YR_DTYPE_F32 && dtype != YR_DTYPE_BF16) return YR_ERR_BAD_ARG;
   if (B == 0) return YR_OK;
   cudaStream_t s = (cudaStream_t)stream;
+  const int TU = rt_users(K, d);
   int64_t per = 0;
-  const int S = rt_splits(B, nI, K, yr_sm_count(), &per);
+  const int S = rt_splits(B, nI, K, TU, yr_sm_count(), &per);
   uint64_t* partial = nullptr;
   if (S > 1) {
-    if (!ws || ws_bytes < yr_recommend_ws_bytes(B, nI, K)) return YR_ERR_WORKSPACE;
+    if (!ws || ws_bytes < rs_partial_bytes(S, B, K)) return YR_ERR_WORKSPACE;
     partial = reinterpret_cast<uint64_t*>(ws);
   }
-  const int TU = rt_users_per_block(K);
   int rc;
-#define YR_RT_LAUNCH(T, TU_)                                                                                              \
-  rt_launch<T, TU_>(U, nU, V, nI, d, user_ids, B, seen_ptr, seen_idx, seen_by_row, masked_score, K, S, per, partial,     \
-                    out_ids, out_scores, err, s)
+#define YR_RT_LAUNCH(T, TU_, BIAS)                                                                                        \
+  rt_launch<T, TU_, BIAS>(U, nU, V, nI, d, user_ids, B, seen_ptr, seen_idx, seen_by_row, masked_score, K, S, per,        \
+                          partial, out_ids, out_scores, err, item_bias, s)
+#define YR_RT_TU(T, BIAS)                                                                                                 \
+  (TU == 16 ? YR_RT_LAUNCH(T, 16, BIAS) : TU == 8 ? YR_RT_LAUNCH(T, 8, BIAS) : YR_RT_LAUNCH(T, 4, BIAS))
   if (dtype == YR_DTYPE_F32)
-    rc = TU == 16 ? YR_RT_LAUNCH(float, 16) : TU == 8 ? YR_RT_LAUNCH(float, 8) : YR_RT_LAUNCH(float, 4);
+    rc = item_bias ? YR_RT_TU(float, true) : YR_RT_TU(float, false);
   else
-    rc = TU == 16 ? YR_RT_LAUNCH(__nv_bfloat16, 16) : TU == 8 ? YR_RT_LAUNCH(__nv_bfloat16, 8)
-                                                          : YR_RT_LAUNCH(__nv_bfloat16, 4);
+    rc = item_bias ? YR_RT_TU(__nv_bfloat16, true) : YR_RT_TU(__nv_bfloat16, false);
+#undef YR_RT_TU
 #undef YR_RT_LAUNCH
   if (rc || S == 1) return rc;
   return merge_launch(partial, S, B, K, out_ids, out_scores, s);
@@ -657,8 +759,7 @@ extern "C" int yr_recommend_topk(const void* U, int64_t nU, const void* V, int64
 
 extern "C" size_t yr_recommend_subset_ws_bytes(int64_t B, int G, int64_t max_subset_len, int K) {
   if (B <= 0 || G < 0 || K <= 0 || K > kRtMaxK) return 0;
-  const size_t plan = ((size_t)3 * G + 8 + (size_t)B) * sizeof(int32_t);
-  return rs_partial_bytes(rs_splits(B, max_subset_len, K), B, K) + plan;
+  return rs_partial_bytes(rs_splits(B, max_subset_len, K, rt_users_per_block(K)), B, K) + rs_plan_bytes(B, G);
 }
 
 extern "C" int yr_recommend_subset_topk(const void* U, int64_t nU, const void* V, int64_t nI, int d, int dtype,
@@ -667,6 +768,17 @@ extern "C" int yr_recommend_subset_topk(const void* U, int64_t nU, const void* V
                                         const int64_t* subset_ids, const int32_t* seen_ptr, const int32_t* seen_idx, int K,
                                         int64_t* out_ids, float* out_scores, void* ws, size_t ws_bytes, int32_t* err,
                                         yr_stream stream) {
+  return yr_recommend_subset_topk_ex(U, nU, V, nI, d, dtype, user_ids, B, subset_ptr, subset_idx, G, max_subset_len,
+                                     subset_ids, seen_ptr, seen_idx, K, out_ids, out_scores, ws, ws_bytes, err, stream,
+                                     nullptr);
+}
+
+extern "C" int yr_recommend_subset_topk_ex(const void* U, int64_t nU, const void* V, int64_t nI, int d, int dtype,
+                                           const int64_t* user_ids, int64_t B, const int32_t* subset_ptr,
+                                           const int32_t* subset_idx, int G, int64_t max_subset_len,
+                                           const int64_t* subset_ids, const int32_t* seen_ptr, const int32_t* seen_idx,
+                                           int K, int64_t* out_ids, float* out_scores, void* ws, size_t ws_bytes,
+                                           int32_t* err, yr_stream stream, const float* item_bias) {
   if (!U || !V || !out_ids || !out_scores || !subset_ptr || !subset_idx) return YR_ERR_BAD_ARG;
   if (B > 0 && (!user_ids || !subset_ids)) return YR_ERR_BAD_ARG;
   if ((seen_ptr == nullptr) != (seen_idx == nullptr)) return YR_ERR_BAD_ARG;
@@ -676,28 +788,30 @@ extern "C" int yr_recommend_subset_topk(const void* U, int64_t nU, const void* V
   if (nI <= 0 || nI >= 0x7fffffffLL || d <= 0 || d > kRtMaxD || (d & 7) != 0) return YR_ERR_BAD_DIM;
   if (dtype != YR_DTYPE_F32 && dtype != YR_DTYPE_BF16) return YR_ERR_BAD_ARG;
   if (B == 0) return YR_OK;
-  if (!ws || ws_bytes < yr_recommend_subset_ws_bytes(B, G, max_subset_len, K)) return YR_ERR_WORKSPACE;
-  cudaStream_t s = (cudaStream_t)stream;
-  const int S = rs_splits(B, max_subset_len, K);
+  const int TU = rt_users(K, d);
+  const int S = rs_splits(B, max_subset_len, K, TU);
   const size_t pbytes = rs_partial_bytes(S, B, K);
+  if (!ws || ws_bytes < pbytes + rs_plan_bytes(B, G)) return YR_ERR_WORKSPACE;
+  cudaStream_t s = (cudaStream_t)stream;
   uint64_t* partial = S > 1 ? reinterpret_cast<uint64_t*>(ws) : nullptr;
   int32_t* cursor = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(ws) + pbytes);   // [G + 2]
   int32_t* rows_at = cursor + G + 2;                                                      // [G + 3]
   int32_t* blocks_at = rows_at + G + 3;                                                   // [G + 3]
   int32_t* order = blocks_at + G + 3;                                                     // [B]
-  const int TU = rt_users_per_block(K);
   recommend_subset_plan_kernel<<<1, kRsPlanThreads, 0, s>>>(subset_ids, (int)B, G, TU, cursor, rows_at, blocks_at, order,
                                                             err);
   YR_CHECK_LAUNCH();
   int rc;
-#define YR_RS_LAUNCH(T, TU_)                                                                                              \
-  rs_launch<T, TU_>(U, nU, V, nI, d, user_ids, B, subset_ptr, subset_idx, G, rows_at, blocks_at, order, seen_ptr,        \
-                    seen_idx, K, S, partial, out_ids, out_scores, err, s)
+#define YR_RS_LAUNCH(T, TU_, BIAS)                                                                                        \
+  rs_launch<T, TU_, BIAS>(U, nU, V, nI, d, user_ids, B, subset_ptr, subset_idx, G, rows_at, blocks_at, order, seen_ptr,  \
+                          seen_idx, K, S, partial, out_ids, out_scores, err, item_bias, s)
+#define YR_RS_TU(T, BIAS)                                                                                                 \
+  (TU == 16 ? YR_RS_LAUNCH(T, 16, BIAS) : TU == 8 ? YR_RS_LAUNCH(T, 8, BIAS) : YR_RS_LAUNCH(T, 4, BIAS))
   if (dtype == YR_DTYPE_F32)
-    rc = TU == 16 ? YR_RS_LAUNCH(float, 16) : TU == 8 ? YR_RS_LAUNCH(float, 8) : YR_RS_LAUNCH(float, 4);
+    rc = item_bias ? YR_RS_TU(float, true) : YR_RS_TU(float, false);
   else
-    rc = TU == 16 ? YR_RS_LAUNCH(__nv_bfloat16, 16) : TU == 8 ? YR_RS_LAUNCH(__nv_bfloat16, 8)
-                                                          : YR_RS_LAUNCH(__nv_bfloat16, 4);
+    rc = item_bias ? YR_RS_TU(__nv_bfloat16, true) : YR_RS_TU(__nv_bfloat16, false);
+#undef YR_RS_TU
 #undef YR_RS_LAUNCH
   if (rc || S == 1) return rc;
   return merge_launch(partial, S, B, K, out_ids, out_scores, s);

@@ -95,6 +95,35 @@ class CDAE(BaseModel):
             raise IndexError("CDAE.forward: index out of range in self")
         return z
 
+    def hidden_from_lists(self, user_id, ptr, idx) -> torch.Tensor:
+        """[B x h] hidden activations of the evaluation-mode model (no dropout) from interaction lists instead of a dense
+        multi-hot: ptr int32 [num_users + 1] / idx int32 is a CSR indexed by user id with ascending unique item ids per row
+        (retrieval.SeenItems). Equal, bit for bit, to hidden(user_id, x)[:, :h] with x the multi-hot of the same lists;
+        nothing of size B x num_items is allocated."""
+        lib = _cabi.load()
+        dev = self.hidden_layer.weight.device
+        user_id = user_id.to(device=dev, dtype=I64).reshape(-1).contiguous()
+        if ptr.dtype != I32 or idx.dtype != I32 or ptr.numel() != self.num_users + 1:
+            raise ValueError(f"CDAE.hidden_from_lists: lists must be an int32 CSR with {self.num_users + 1} offsets")
+        if ptr.device != dev or idx.device != dev:
+            raise ValueError(f"CDAE.hidden_from_lists: lists must live on the model's device ({dev})")
+        ptr = ptr.contiguous()
+        idx = idx.contiguous() if idx.numel() else torch.zeros(1, device=dev, dtype=I32)
+        B = user_id.numel()
+        z = torch.empty(B, self.hidden_size, device=dev, dtype=F32)
+        err = torch.zeros(1, device=dev, dtype=I32)
+        st = self.tensors()
+        _cabi.check(lib.yr_cdae_encode(C.byref(st), self.num_users, self.num_items, self.hidden_size, self.hidden_act,
+                                       _cabi.dptr(user_id), B, _cabi.dptr(ptr), _cabi.dptr(idx), _cabi.dptr(z),
+                                       self.hidden_size, _cabi.dptr(err), _cabi.stream_ptr(dev)), "yr_cdae_encode")
+        e = int(err.item())
+        if e & 1:
+            raise IndexError(f"CDAE.hidden_from_lists: user id out of range [0, {self.num_users})")
+        if e & 2:
+            raise IndexError(f"CDAE.hidden_from_lists: item id out of range [0, {self.num_items}) "
+                             "(or malformed list offsets)")
+        return z
+
     def forward(self, user_id, x, keep=None):
         lib = _cabi.load()
         x = x.to(device=self.hidden_layer.weight.device, dtype=F32).contiguous()

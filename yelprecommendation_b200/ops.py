@@ -617,16 +617,29 @@ def topk_metrics(predicted: torch.Tensor, ecsr: DeviceEvalCSR):
 # top-K retrieval
 # ----------------------------------------------------------------------------------------------------
 RECOMMEND_MAX_K = 1024
-RECOMMEND_MAX_D = 512
+RECOMMEND_MAX_D = 1024
 _RT_DTYPES = {F32: _cabi.YR_DTYPE_F32, torch.bfloat16: _cabi.YR_DTYPE_BF16}
+
+
+def _item_bias(item_bias: Optional[torch.Tensor], nI: int, dev, what: str) -> Optional[torch.Tensor]:
+    """item_bias as a contiguous fp32 [nI] tensor on `dev` (None passes through)."""
+    if item_bias is None:
+        return None
+    if not torch.is_tensor(item_bias) or item_bias.dtype != F32 or item_bias.dim() != 1 or item_bias.numel() != nI:
+        raise ValueError(f"{what}: item_bias must be a float32 tensor of shape [{nI}]")
+    if item_bias.device != dev:
+        raise ValueError(f"{what}: item_bias must live on the device of the embeddings ({dev}), got {item_bias.device}")
+    return item_bias.detach().contiguous()
 
 
 def recommend_topk(U: torch.Tensor, V: torch.Tensor, user_ids: torch.Tensor, K: int, seen_ptr: Optional[torch.Tensor] = None,
                    seen_idx: Optional[torch.Tensor] = None, seen_by_row: bool = False,
-                   masked_score: float = float("-inf")) -> Tuple[torch.Tensor, torch.Tensor]:
-    """yr_recommend_topk: (ids int64 [B x K], scores float32 [B x K]) of the K best items per user by (score desc, id asc),
-    score = U[uid] . V[item] in fp32 (fp32 or bf16 tables). Seen items (CSR int32, ascending per row, rows = user ids, or
-    batch rows with seen_by_row) score `masked_score`; -inf drops them. Short rows are padded with id -1 / score -inf."""
+                   masked_score: float = float("-inf"),
+                   item_bias: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """yr_recommend_topk_ex: (ids int64 [B x K], scores float32 [B x K]) of the K best items per user by (score desc, id
+    asc), score = U[uid] . V[item] (+ item_bias[item]) in fp32 (fp32 or bf16 tables, fp32 bias). Seen items (CSR int32,
+    ascending per row, rows = user ids, or batch rows with seen_by_row) score `masked_score`; -inf drops them. Short rows
+    are padded with id -1 / score -inf."""
     if not (torch.is_tensor(U) and torch.is_tensor(V) and torch.is_tensor(user_ids)):
         raise TypeError("recommend_topk: U, V and user_ids must be tensors")
     if not (U.is_cuda and V.is_cuda and user_ids.is_cuda):
@@ -652,6 +665,7 @@ def recommend_topk(U: torch.Tensor, V: torch.Tensor, user_ids: torch.Tensor, K: 
         raise TypeError(f"recommend_topk: user_ids must be a 1-D int64 or int32 tensor, got {user_ids.dtype} {tuple(user_ids.shape)}")
     if (seen_ptr is None) != (seen_idx is None):
         raise ValueError("recommend_topk: seen_ptr and seen_idx go together")
+    bias = _item_bias(item_bias, nI, dev, "recommend_topk")
     uid = user_ids.to(I64).contiguous()
     B = int(uid.numel())
     if seen_ptr is not None:
@@ -671,9 +685,10 @@ def recommend_topk(U: torch.Tensor, V: torch.Tensor, user_ids: torch.Tensor, K: 
     err = torch.zeros(1, device=dev, dtype=I32)
     nbytes = lib.yr_recommend_ws_bytes(B, nI, K)
     ws = torch.empty(max(nbytes, 1), device=dev, dtype=torch.uint8)
-    check(lib.yr_recommend_topk(Uc.data_ptr(), nU, Vc.data_ptr(), nI, d, _RT_DTYPES[U.dtype], dptr(uid, I64), B,
-                                dptr(seen_ptr), dptr(seen_idx), 1 if seen_by_row else 0, float(masked_score), K,
-                                dptr(ids), dptr(scores), dptr(ws), nbytes, dptr(err), stream_ptr(dev)), "yr_recommend_topk")
+    check(lib.yr_recommend_topk_ex(Uc.data_ptr(), nU, Vc.data_ptr(), nI, d, _RT_DTYPES[U.dtype], dptr(uid, I64), B,
+                                   dptr(seen_ptr), dptr(seen_idx), 1 if seen_by_row else 0, float(masked_score), K,
+                                   dptr(ids), dptr(scores), dptr(ws), nbytes, dptr(err), stream_ptr(dev), dptr(bias)),
+          "yr_recommend_topk_ex")
     if int(err.item()) != 0:
         raise IndexError(f"recommend_topk: user id out of range [0, {nU})")
     return ids, scores
@@ -682,8 +697,9 @@ def recommend_topk(U: torch.Tensor, V: torch.Tensor, user_ids: torch.Tensor, K: 
 def recommend_subset_topk(U: torch.Tensor, V: torch.Tensor, user_ids: torch.Tensor, K: int, subset_ptr: torch.Tensor,
                           subset_idx: torch.Tensor, subset_ids: torch.Tensor, max_len: int,
                           seen_ptr: Optional[torch.Tensor] = None,
-                          seen_idx: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
-    """yr_recommend_subset_topk: recommend_topk with row b restricted to the items of subset subset_ids[b] (-1 = the whole
+                          seen_idx: Optional[torch.Tensor] = None,
+                          item_bias: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """yr_recommend_subset_topk_ex: recommend_topk with row b restricted to the items of subset subset_ids[b] (-1 = the whole
     catalog). Subsets: CSR int32 (subset_ptr [G + 1], subset_idx ascending per subset). max_len: the longest list a row
     streams (the longest subset, num_items if a row is -1); it sets only the number of item splits. Seen lists are indexed
     by user id. (ids int64 [B x K], scores float32 [B x K]), identical to recommend_topk with the items outside each row's
@@ -730,6 +746,7 @@ def recommend_subset_topk(U: torch.Tensor, V: torch.Tensor, user_ids: torch.Tens
         raise ValueError(f"recommend_subset_topk: max_len must be a non-negative integer, got {max_len}")
     if (seen_ptr is None) != (seen_idx is None):
         raise ValueError("recommend_subset_topk: seen_ptr and seen_idx go together")
+    bias = _item_bias(item_bias, nI, dev, "recommend_subset_topk")
     if seen_ptr is not None:
         if seen_ptr.dtype != I32 or seen_idx.dtype != I32 or seen_ptr.numel() != nU + 1:
             raise ValueError(f"recommend_subset_topk: seen lists must be int32 CSR with {nU + 1} offsets")
@@ -750,10 +767,10 @@ def recommend_subset_topk(U: torch.Tensor, V: torch.Tensor, user_ids: torch.Tens
     err = torch.zeros(1, device=dev, dtype=I32)
     nbytes = lib.yr_recommend_subset_ws_bytes(B, G, int(max_len), K)
     ws = torch.empty(max(nbytes, 1), device=dev, dtype=torch.uint8)
-    check(lib.yr_recommend_subset_topk(Uc.data_ptr(), nU, Vc.data_ptr(), nI, d, _RT_DTYPES[U.dtype], dptr(uid, I64), B,
-                                       dptr(sptr, I32), dptr(sidx, I32), G, int(max_len), dptr(sid, I64), dptr(seen_ptr),
-                                       dptr(seen_idx), K, dptr(ids), dptr(scores), dptr(ws), nbytes, dptr(err),
-                                       stream_ptr(dev)), "yr_recommend_subset_topk")
+    check(lib.yr_recommend_subset_topk_ex(Uc.data_ptr(), nU, Vc.data_ptr(), nI, d, _RT_DTYPES[U.dtype], dptr(uid, I64),
+                                          B, dptr(sptr, I32), dptr(sidx, I32), G, int(max_len), dptr(sid, I64),
+                                          dptr(seen_ptr), dptr(seen_idx), K, dptr(ids), dptr(scores), dptr(ws), nbytes,
+                                          dptr(err), stream_ptr(dev), dptr(bias)), "yr_recommend_subset_topk_ex")
     e = int(err.item())
     if e & 1:
         raise IndexError(f"recommend_subset_topk: user id out of range [0, {nU})")

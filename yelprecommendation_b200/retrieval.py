@@ -17,6 +17,12 @@ on chip, so the B x num_items score matrix is never materialised. On CPU tables 
 PyTorch restatement (dense scores, masked, stably sorted) that also serves as the kernel's oracle. With `subset`, the
 kernel is yr_recommend_subset_topk: rows are grouped by subset on the device and each streams only its subset's items;
 ids and scores equal what the unrestricted kernel returns with every item outside the subset excluded.
+
+    rec = CDAERecommender(cdae_model, seen)                    # or cdae_trainer.recommender(seen)
+    ids, logits = rec.recommend(user_ids, k=20)                # same contract; the scores are CDAE output logits
+
+A CDAE user is encoded from their interaction list (yr_cdae_encode), and the output bias enters the retrieval kernels as a
+per-item bias added after the dot product.
 """
 from __future__ import annotations
 
@@ -158,10 +164,10 @@ def _subset_rows(subset, B: int, subsets: Optional[ItemSubsets]):
 
 def recommend_reference(user_emb: torch.Tensor, item_emb: torch.Tensor, user_ids, k: int,
                         seen: Optional[SeenItems] = None, subsets: Optional[ItemSubsets] = None,
-                        subset=None) -> Tuple[torch.Tensor, torch.Tensor]:
-    """Plain PyTorch on the tables' device: dense [B x num_items] scores, seen items and items outside the row's subset
-    (subsets[subset[b]]; -1 = whole catalog) set to -inf, a stable descending sort (torch.topk does not fix the order of
-    ties), and slots holding -inf turned into padding (id -1)."""
+                        subset=None, item_bias: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Plain PyTorch on the tables' device: dense [B x num_items] scores (+ item_bias [num_items], fp32), seen items and
+    items outside the row's subset (subsets[subset[b]]; -1 = whole catalog) set to -inf, a stable descending sort
+    (torch.topk does not fix the order of ties), and slots holding -inf turned into padding (id -1)."""
     k = _check_k(k)
     dev = user_emb.device
     uid = torch.as_tensor(user_ids).to(device=dev, dtype=I64).reshape(-1)
@@ -170,6 +176,8 @@ def recommend_reference(user_emb: torch.Tensor, item_emb: torch.Tensor, user_ids
         raise IndexError(f"recommend: user id out of range [0, {nU})")
     B = uid.numel()
     scores = user_emb[uid].to(F32) @ item_emb.to(F32).T
+    if item_bias is not None:
+        scores = scores + item_bias.to(device=dev, dtype=F32)[None, :]
     scores = torch.where(torch.isnan(scores), torch.full_like(scores, float("-inf")), scores)
     if seen is not None:
         row, item = _list_entries(seen, uid, dev)
@@ -226,16 +234,105 @@ class Recommender:
         uid = user_ids if torch.is_tensor(user_ids) else torch.as_tensor(np.asarray(user_ids, dtype=np.int64))
         uid = uid.to(dev).reshape(-1)
         ptr, idx = seen.on(dev) if seen is not None else (None, None)
-        if subset is None:
-            return ops.recommend_topk(self.user_emb, self.item_emb, uid, k, ptr, idx)
-        sid = _subset_rows(subset, uid.numel(), self.subsets)
-        nI = self.item_emb.shape[0]
-        if sid.is_cuda:
+        return _recommend_kernel(self.user_emb, self.item_emb, uid, k, ptr, idx, self.subsets, subset)
+
+
+def _recommend_kernel(U, V, uid, k, seen_ptr, seen_idx, subsets: Optional[ItemSubsets], subset, item_bias=None):
+    """ops.recommend_topk, or with `subset` ops.recommend_subset_topk: seen lists indexed by uid, which is on U's device.
+    Host-side subset ids let the number of item splits follow the requested subsets; on a CUDA tensor it follows the whole
+    catalog (no device read)."""
+    if subset is None:
+        return ops.recommend_topk(U, V, uid, k, seen_ptr, seen_idx, item_bias=item_bias)
+    sid = _subset_rows(subset, uid.numel(), subsets)
+    nI = V.shape[0]
+    if sid.is_cuda:
+        max_len = nI
+    else:
+        h = sid.numpy()
+        max_len = int(subsets.lengths[h[h >= 0]].max(initial=0))
+        if (h == -1).any():
             max_len = nI
-        else:
-            h = sid.numpy()
-            max_len = int(self.subsets.lengths[h[h >= 0]].max(initial=0))
-            if (h == -1).any():
-                max_len = nI
-        sptr, sidx = self.subsets.on(dev)
-        return ops.recommend_subset_topk(self.user_emb, self.item_emb, uid, k, sptr, sidx, sid.to(dev), max_len, ptr, idx)
+    sptr, sidx = subsets.on(U.device)
+    return ops.recommend_subset_topk(U, V, uid, k, sptr, sidx, sid.to(U.device), max_len, seen_ptr, seen_idx,
+                                     item_bias=item_bias)
+
+
+def _cdae_check(model, seen: Optional[SeenItems], subsets: Optional[ItemSubsets], what: str) -> None:
+    if seen is None:
+        raise ValueError(f"{what}: CDAE needs the seen items even with exclude_seen=False: they are the model's input")
+    if seen.num_users != model.num_users or seen.num_items != model.num_items:
+        raise ValueError(f"{what}: seen items cover {seen.num_users} users x {seen.num_items} items, the model "
+                         f"{model.num_users} x {model.num_items}")
+    if subsets is not None and subsets.num_items != model.num_items:
+        raise ValueError(f"{what}: subsets cover {subsets.num_items} items, the model {model.num_items}")
+
+
+def cdae_recommend_reference(model, user_ids, k: int, seen: SeenItems, exclude_seen: bool = True,
+                             subsets: Optional[ItemSubsets] = None, subset=None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Plain PyTorch restatement of CDAERecommender.recommend on the model's device: the dense multi-hot x of the users'
+    seen items, z = act(x @ W_h^T + b_h + V_u[u]), then recommend_reference over the logits z . W_o[i] + b_o[i]."""
+    _cdae_check(model, seen, subsets, "cdae_recommend_reference")
+    dev = model.hidden_layer.weight.device
+    uid = torch.as_tensor(user_ids).to(device=dev, dtype=I64).reshape(-1)
+    if uid.numel() and (int(uid.min()) < 0 or int(uid.max()) >= model.num_users):
+        raise IndexError(f"recommend: user id out of range [0, {model.num_users})")
+    B = uid.numel()
+    x = torch.zeros(B, model.num_items, device=dev, dtype=F32)
+    row, item = _list_entries(seen, uid, dev)
+    x[row, item] = 1.0
+    Wh, bh = model.hidden_layer.weight.data, model.hidden_layer.bias.data
+    pre = x @ Wh.T + bh + model.user_nodes.weight.data[uid]
+    z = pre if model.hidden_act == 1 else torch.sigmoid(pre)
+    rows = SeenItems(*_batch_lists(seen, uid), B, model.num_items) if exclude_seen else None
+    return recommend_reference(z, model.output_layer.weight.data, torch.arange(B, device=dev), k, rows, subsets, subset,
+                               item_bias=model.output_layer.bias.data)
+
+
+def _batch_lists(seen: SeenItems, uid: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+    """(ptr int32 [B + 1], idx int32): seen[uid[b]] for every batch row b, a CSR indexed by the batch row (uid's device)."""
+    dev = uid.device
+    ptr = seen.on(dev)[0].to(I64)
+    bptr = torch.zeros(uid.numel() + 1, device=dev, dtype=I64)
+    bptr[1:] = torch.cumsum(ptr[uid + 1] - ptr[uid], 0)
+    return bptr.to(I32), _list_entries(seen, uid, dev)[1].to(I32)
+
+
+class CDAERecommender:
+    """Top-K retrieval for a CDAE model (models/cdae.py) on the device, through its live parameters: training between
+    calls is reflected. The user side is encoded from the user's interaction list (seen, which is the model's input and is
+    therefore required even with exclude_seen=False, as CDAETrainer.evaluate feeds and masks the same input), without a
+    B x num_items input or output: z = act(W_h[:, seen[u]].sum(1) + b_h + V_u[u]) (yr_cdae_encode), then the fused
+    retrieval kernel ranks the logits z . W_o[i] + b_o[i] (b_o as the per-item bias).
+
+    recommend(user_ids, k, exclude_seen=True, subset=None) has Recommender.recommend's contract: (item ids int64 [B x k],
+    scores float32 [B x k]), best first, ties to the lower id, short rows padded with -1 / -inf, the same subset semantics.
+    The scores are logits, the values CDAETrainer.evaluate ranks by; sigmoid(score) is the model's predicted probability.
+    """
+
+    def __init__(self, model, seen: SeenItems, subsets: Optional[ItemSubsets] = None):
+        _cdae_check(model, seen, subsets, "CDAERecommender")
+        if model.hidden_layer.weight.device.type != "cuda":
+            raise ops.YelprecError("CDAERecommender: the model must be on a CUDA device (the reference path is "
+                                   "retrieval.cdae_recommend_reference)")
+        self.model, self.seen, self.subsets = model, seen, subsets
+
+    def recommend(self, user_ids, k: int, exclude_seen: bool = True, subset=None) -> Tuple[torch.Tensor, torch.Tensor]:
+        """(item ids int64 [B x k], logits float32 [B x k]) on the model's device, best first; see the class docstring."""
+        m = self.model
+        dev = m.hidden_layer.weight.device
+        if subset is not None and self.subsets is None:
+            raise ValueError("recommend: subset needs the item subsets (CDAERecommender(..., subsets=ItemSubsets...))")
+        k = _check_k(k)
+        uid = user_ids if torch.is_tensor(user_ids) else torch.as_tensor(np.asarray(user_ids, dtype=np.int64))
+        uid = uid.to(device=dev, dtype=I64).reshape(-1)
+        B = uid.numel()
+        if subset is not None:
+            _subset_rows(subset, B, self.subsets)
+        if B == 0:
+            return torch.empty(0, k, device=dev, dtype=I64), torch.empty(0, k, device=dev, dtype=F32)
+        ptr, idx = self.seen.on(dev)
+        z = m.hidden_from_lists(uid, ptr, idx)
+        rows = torch.arange(B, device=dev, dtype=I64)
+        bptr, bidx = _batch_lists(self.seen, uid) if exclude_seen else (None, None)
+        return _recommend_kernel(z, m.output_layer.weight.data, rows, k, bptr, bidx, self.subsets, subset,
+                                 item_bias=m.output_layer.bias.data)
