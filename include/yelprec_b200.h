@@ -613,6 +613,28 @@ int yr_recommend_subset_topk_ex(const void* U, int64_t nU, const void* V, int64_
                                 const int32_t* seen_idx, int K, int64_t* out_ids, float* out_scores, void* ws,
                                 size_t ws_bytes, int32_t* err, yr_stream stream, const float* item_bias);
 
+/* yr_recommend_topk_ex restricted per row to the items within a radius of a point on the sphere. Item i is inside row b
+ * iff ((c_x * p_x) + (c_y * p_y)) + (c_z * p_z) >= threshold[b] in float64, each product and sum rounded on its own,
+ * where c = centre_xyz[3b .. 3b + 3) is the centre's unit vector, p = item_xyz[3i .. 3i + 3) the item's, and
+ * threshold[b] = cos(radius / Earth radius) (-INFINITY: every item). Row b gets exactly the ids and scores
+ * yr_recommend_topk_ex returns when every item outside is a seen item with masked_score = -INFINITY (seen lists indexed
+ * by user id; item_bias may be NULL). The item grid: cells of cell_deg degrees, num_lat = ceil(180 / cell_deg) lat bands
+ * and num_lon = ceil(360 / cell_deg) lon bands; an item at (lat, lon) degrees is in band floor((lat + 90) / cell_deg)
+ * and floor((lon + 180) / cell_deg), each clamped to the grid, cell key = lat band * num_lon + lon band. cell_items
+ * [nI] holds the item ids sorted by (key, id), cell_keys [num_cells] the ascending keys of the non-empty cells and
+ * cell_ptr [num_cells + 1] their offsets into cell_items. The grid only bounds which items are read: results do not
+ * depend on it as long as item_xyz and the cells come from the same (lat, lon). A user id outside [0, nU) sets
+ * *err |= 1, a non-finite centre or a NaN / +inf threshold *err |= 2; either row is all padding. The number of item
+ * splits follows nI (no device read). Other limits as yr_recommend_subset_topk.
+ * ws: yr_recommend_geo_ws_bytes(B, nI, K) bytes (window and row grouping per request, per-split lists; same device). */
+size_t yr_recommend_geo_ws_bytes(int64_t B, int64_t nI, int K);
+int yr_recommend_geo_topk(const void* U, int64_t nU, const void* V, int64_t nI, int d, int dtype, const int64_t* user_ids,
+                          int64_t B, const int64_t* cell_keys, const int32_t* cell_ptr, int64_t num_cells,
+                          const int32_t* cell_items, const double* item_xyz, double cell_deg, int64_t num_lat,
+                          int64_t num_lon, const double* centre_xyz, const double* threshold, const int32_t* seen_ptr,
+                          const int32_t* seen_idx, int K, int64_t* out_ids, float* out_scores, void* ws, size_t ws_bytes,
+                          int32_t* err, yr_stream stream, const float* item_bias);
+
 #ifdef __cplusplus
 }
 #endif

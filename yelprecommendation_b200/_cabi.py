@@ -35,6 +35,7 @@ SYMBOLS = (
     "yr_split_ws_bytes", "yr_split_sizes", "yr_split_per_user",
     "yr_recommend_ws_bytes", "yr_recommend_topk", "yr_recommend_subset_ws_bytes", "yr_recommend_subset_topk",
     "yr_recommend_topk_ex", "yr_recommend_subset_topk_ex", "yr_cdae_encode",
+    "yr_recommend_geo_ws_bytes", "yr_recommend_geo_topk",
 )
 
 YR_OPT_SGD, YR_OPT_ADAM, YR_OPT_ADAMW = 0, 1, 2
@@ -209,6 +210,9 @@ def load() -> C.CDLL:
         "yr_recommend_subset_topk_ex": (C.c_int, [p, i64, p, i64, i32, i32, p, i64, p, p, i32, i64, p, p, p, i32, p, p,
                                                   p, sz, p, p, p]),
         "yr_cdae_encode": (C.c_int, [C.POINTER(YrCdaeTensors), i64, i64, i32, i32, p, i64, p, p, p, i64, p, p]),
+        "yr_recommend_geo_ws_bytes": (sz, [i64, i64, i32]),
+        "yr_recommend_geo_topk": (C.c_int, [p, i64, p, i64, i32, i32, p, i64, p, p, i64, p, p, C.c_double, i64, i64, p,
+                                            p, p, p, i32, p, p, p, sz, p, p, p]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)

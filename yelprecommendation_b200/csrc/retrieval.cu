@@ -585,6 +585,303 @@ recommend_subset_bias_kernel(const T* __restrict__ U, int64_t nU, const T* __res
                                      seen_idx, K, S, partial, out_ids, out_scores, err, item_bias);
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// Radius-restricted retrieval. Row b ranks only the items i with ((c_x * p_x) + (c_y * p_y)) + (c_z * p_z) >= t_b in
+// float64, every product and sum rounded on its own (__dmul_rn / __dadd_rn: no fma contraction): c = the row's centre
+// (a unit vector), p = P[i] the item's unit vector, t_b = cos(radius / Earth radius), -inf for the whole Earth.
+//
+// Items are indexed by a grid of lat x lon cells w degrees on a side (lat band = floor((lat + 90) / w), lon band =
+// floor((lon + 180) / w), both clamped to the grid; key = lat band * nlon + lon band): cell_items holds the item ids
+// sorted by (key, id), cell_keys the ascending keys of the non-empty cells and cell_ptr their offsets into cell_items.
+// The items of one lat band and a lon-band range are therefore one contiguous run of cell_items, and so are the items of
+// a range of whole bands.
+//
+// recommend_geo_window_kernel gives every row a window of cells that covers its cap with one cell of margin: the lat
+// bands of [lat - a - w, lat + a + w] (a = the cap's angular radius) and, per band, the lon bands of [lon - D - w,
+// lon + D + w] (D = asin(sin a / cos lat), the cap's widest longitude offset), split in two at the antimeridian; every
+// longitude when the cap comes within a cell of a pole, when D + w reaches 180 degrees or when the window spans more than
+// kGeoMaxBands bands. The exact predicate decides membership; the window only has to be a superset. Rows are grouped by a
+// hash of their window (recommend_subset_plan_kernel over the hash buckets), and recommend_geo_kernel streams each
+// distinct window of its rows once for all of them.
+// ---------------------------------------------------------------------------------------------------------------------
+constexpr int kGeoMaxBands = 128;                  // wider windows take every longitude: one run of cell_items
+constexpr int kGeoMaxSegs = 2 * kGeoMaxBands;      // runs of one window: two lon ranges per band (== kRtThreads)
+constexpr int kGeoWin = 6;                         // window: lat bands [a, b], lon bands [lo0, hi0] and [lo1, hi1]
+static_assert(kGeoMaxSegs <= kRtThreads, "one thread per run");
+
+__device__ __forceinline__ int geo_band(double x, double w, int n) {   // floor(x / w) clamped to [0, n)
+  const double f = floor(x / w);
+  return f < 0.0 ? 0 : f >= (double)n ? n - 1 : (int)f;
+}
+
+// One thread per row: the window and its hash bucket (-1 for a non-finite centre or threshold: error bit 2, and an
+// all-padding row). A zero centre or t <= -|c| takes the whole grid.
+__global__ void __launch_bounds__(kRtThreads)
+recommend_geo_window_kernel(const double* __restrict__ c, const double* __restrict__ t, int64_t B, double w, int nlat,
+                            int nlon, int H, int32_t* __restrict__ win, int64_t* __restrict__ bucket, int32_t* err) {
+  const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  constexpr double kDeg = 57.295779513082320876798;   // degrees per radian
+  const double cx = c[3 * b], cy = c[3 * b + 1], cz = c[3 * b + 2], tb = t[b];
+  int v[kGeoWin] = {0, nlat - 1, -1, 0, 0, -1};      // every cell; lo0 = -1: every longitude
+  if (!isfinite(cx) || !isfinite(cy) || !isfinite(cz) || isnan(tb) || tb == INFINITY) {
+    if (err) atomicOr(err, 2);
+#pragma unroll
+    for (int i = 0; i < kGeoWin; ++i) win[kGeoWin * b + i] = 0;
+    bucket[b] = -1;
+    return;
+  }
+  const double n = sqrt(cx * cx + cy * cy + cz * cz);
+  if (n > 0.0 && tb / n > -1.0) {
+    const double ct = fmin(tb / n, 1.0), z = fmax(-1.0, fmin(1.0, cz / n));
+    const double a = acos(ct) * kDeg;
+    const double lat = asin(z) * kDeg;
+    const double lat_lo = lat - a - w, lat_hi = lat + a + w;
+    v[0] = geo_band(lat_lo + 90.0, w, nlat);
+    v[1] = geo_band(lat_hi + 90.0, w, nlat);
+    if (lat_lo > -90.0 && lat_hi < 90.0 && v[1] - v[0] < kGeoMaxBands) {
+      const double s = sqrt(fmax(0.0, 1.0 - ct * ct)) / sqrt(fmax(0.0, 1.0 - z * z));   // sin a / cos lat
+      const double dl = s < 1.0 ? asin(s) * kDeg + w : 180.0;
+      if (dl < 180.0) {
+        const double lon = atan2(cy, cx) * kDeg;
+        const double L = lon - dl, R = lon + dl;
+        if (L >= -180.0 && R <= 180.0) {
+          v[2] = geo_band(L + 180.0, w, nlon); v[3] = geo_band(R + 180.0, w, nlon);
+        } else {                                     // across the antimeridian: [L', 180] and [-180, R']
+          const double L2 = L < -180.0 ? L + 360.0 : L, R2 = R > 180.0 ? R - 360.0 : R;
+          v[2] = geo_band(L2 + 180.0, w, nlon); v[3] = nlon - 1;
+          v[4] = 0; v[5] = geo_band(R2 + 180.0, w, nlon);
+          if (v[5] >= v[2]) { v[2] = -1; v[3] = 0; v[4] = 0; v[5] = -1; }   // the two ranges meet: every longitude
+        }
+      }
+    }
+  }
+  uint32_t h = 2166136261u;                          // FNV-1a over the window, then a final mix
+#pragma unroll
+  for (int i = 0; i < kGeoWin; ++i) {
+    win[kGeoWin * b + i] = v[i];
+    h = (h ^ (uint32_t)v[i]) * 16777619u;
+  }
+  h ^= h >> 16; h *= 0x7feb352du; h ^= h >> 15;
+  bucket[b] = (int64_t)(h & (uint32_t)(H - 1));
+}
+
+// First position in cell_items of the cells with key >= k.
+__device__ __forceinline__ int geo_cell_lb(const int64_t* __restrict__ cell_keys, const int32_t* __restrict__ cell_ptr,
+                                           int64_t nC, int64_t k) {
+  int64_t lo = 0, hi = nC;
+  while (lo < hi) {
+    const int64_t mid = (lo + hi) >> 1;
+    if (cell_keys[mid] < k) lo = mid + 1; else hi = mid;
+  }
+  return cell_ptr[lo];
+}
+
+// Whether `item` is in the ascending list idx[lo, hi).
+__device__ __forceinline__ bool geo_listed(const int32_t* __restrict__ idx, int lo, int hi, int item) {
+  const int end = hi;
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (idx[mid] < item) lo = mid + 1; else hi = mid;
+  }
+  return lo < end && idx[lo] == item;
+}
+
+// Grid (upper bound on the plan's block count, S), as recommend_subset_kernel: block x takes up to TU rows of one hash
+// bucket (group H: rows with a non-finite centre or threshold, all padding), split y of each window. Rows of a bucket
+// normally share one window; on a hash collision the block streams each distinct window of its rows in turn, and a row
+// takes offers only during its own window. Window items come in cell order, not id order, so instead of the ascending
+// seen cursor of the subset kernel a candidate that beats the row's current K-th best is looked up in the row's seen
+// list (a binary search) before it enters the buffer: few items get that far once the thresholds settle.
+// kBias: score + item_bias[item].
+template <typename T, int TU, bool kBias>
+__global__ void __launch_bounds__(kRtThreads, 2)   // 2 blocks an SM: up to 128 registers, no spills
+recommend_geo_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ V, int d, const int64_t* __restrict__ uids,
+                     int64_t B, const int64_t* __restrict__ cell_keys, const int32_t* __restrict__ cell_ptr, int64_t nC,
+                     const int32_t* __restrict__ cell_items, const double* __restrict__ P, int nlon,
+                     const double* __restrict__ c, const double* __restrict__ t, const int32_t* __restrict__ win, int H,
+                     const int32_t* __restrict__ rows_at, const int32_t* __restrict__ blocks_at,
+                     const int32_t* __restrict__ order, const int32_t* __restrict__ seen_ptr,
+                     const int32_t* __restrict__ seen_idx, int K, int S, uint64_t* __restrict__ partial,
+                     int64_t* __restrict__ out_ids, float* __restrict__ out_scores, int32_t* err,
+                     const float* __restrict__ item_bias) {
+  constexpr int CAP = kRtEntries / TU;
+  extern __shared__ __align__(16) uint64_t rt_smem[];
+  uint64_t* keys = rt_smem;                                    // [TU][CAP]
+  uint64_t* thr = keys + kRtEntries;                           // [TU]; ~0 = inactive row (no candidate beats it)
+  double* cq = reinterpret_cast<double*>(thr + TU);            // [TU][4]: c_x, c_y, c_z, t of each row
+  float* Us = reinterpret_cast<float*>(cq + 4 * TU);           // [TU][d]
+  int* cnt = reinterpret_cast<int*>(Us + (size_t)TU * d);      // [TU]
+  int* sb = cnt + TU;                                          // [TU]: the row's seen list, seen_idx[sb, se)
+  int* se = sb + TU;                                           // [TU]
+  int* rowb = se + TU;                                         // [TU]: batch row of each user, -1 = none
+  int* pass = rowb + TU;                                       // [TU]: 0 to stream, 1 in the current window, 2 done
+  int* wv = pass + TU;                                         // [8]: the current window
+  int* seg = wv + 8;                                           // [kGeoMaxSegs]: first cell_items position of each run
+  int* pref = seg + kGeoMaxSegs;                               // [kGeoMaxSegs + 1]: window position of each run
+  int* misc = pref + kGeoMaxSegs + 1;                          // [16]: leader row, warp sums of the scan
+
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int blk = blockIdx.x, split = blockIdx.y;
+  if (blk >= blocks_at[H + 2]) return;
+  int lo = 0, hi = H + 2;                                      // group: the last g with blocks_at[g] <= blk
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (blocks_at[mid] <= blk) lo = mid + 1; else hi = mid;
+  }
+  const int g = lo - 1;
+  const int r0 = rows_at[g] + (blk - blocks_at[g]) * TU;
+  const int nr = min(TU, rows_at[g + 1] - r0);
+
+  if (tid < TU) {
+    const int b = tid < nr ? order[r0 + tid] : -1;
+    bool active = false;
+    int s0 = 0, s1 = 0;
+    if (b >= 0) {
+      const int64_t uid = uids[b];
+      active = uid >= 0 && uid < nU;
+      if (!active && err) atomicOr(err, 1);
+      if (active && seen_ptr) { s0 = seen_ptr[uid]; s1 = seen_ptr[uid + 1]; }
+      active = active && g < H;
+      if (active) {
+        cq[4 * tid] = c[3 * b]; cq[4 * tid + 1] = c[3 * b + 1]; cq[4 * tid + 2] = c[3 * b + 2]; cq[4 * tid + 3] = t[b];
+      }
+    }
+    rowb[tid] = b;
+    thr[tid] = active ? 0ull : ~0ull;
+    cnt[tid] = 0;
+    sb[tid] = s0; se[tid] = s1;
+    pass[tid] = active ? 0 : 2;
+  }
+  __syncthreads();
+  for (int i = tid; i < TU * d; i += kRtThreads) {
+    const int u = i / d, k = i - u * d;
+    float x = 0.f;
+    if (thr[u] == 0ull) x = rt_to_float(U[uids[rowb[u]] * d + k]);
+    Us[i] = x;
+  }
+
+  for (;;) {
+    if (tid == 0) {
+      int l = -1;
+      for (int u = 0; u < TU && l < 0; ++u)
+        if (pass[u] == 0) l = u;
+      misc[0] = l;
+    }
+    __syncthreads();
+    const int lead = misc[0];
+    if (lead < 0) break;
+    if (tid < kGeoWin) wv[tid] = win[(int64_t)kGeoWin * rowb[lead] + tid];
+    __syncthreads();
+    if (tid < TU && pass[tid] == 0) {
+      bool same = true;
+#pragma unroll
+      for (int i = 0; i < kGeoWin; ++i) same = same && win[(int64_t)kGeoWin * rowb[tid] + i] == wv[i];
+      if (same) pass[tid] = 1;
+    }
+    // ---- the window's runs of cell_items and their positions in the window (an exclusive scan of the lengths) ----
+    const bool all_lon = wv[2] < 0;
+    const int nseg = all_lon ? 1 : 2 * (wv[1] - wv[0] + 1);
+    int len = 0;
+    if (tid < nseg) {
+      int64_t k0, k1;
+      if (all_lon) {
+        k0 = (int64_t)wv[0] * nlon; k1 = (int64_t)(wv[1] + 1) * nlon;
+      } else {
+        const int64_t band = (int64_t)(wv[0] + (tid >> 1)) * nlon;
+        const int l = (tid & 1) ? wv[4] : wv[2], h = (tid & 1) ? wv[5] : wv[3];
+        k0 = band + l; k1 = l <= h ? band + h + 1 : k0;
+      }
+      const int p0 = geo_cell_lb(cell_keys, cell_ptr, nC, k0);
+      seg[tid] = p0;
+      len = k1 > k0 ? geo_cell_lb(cell_keys, cell_ptr, nC, k1) - p0 : 0;
+    }
+    int x = len;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int y = __shfl_up_sync(kFull, x, o);
+      if (lane >= o) x += y;
+    }
+    if (lane == 31) misc[8 + warp] = x;
+    __syncthreads();
+    int base = 0;
+    for (int i = 0; i < warp; ++i) base += misc[8 + i];
+    if (tid < nseg) pref[tid] = base + x - len;
+    if (tid == kRtThreads - 1) pref[nseg] = base + x;
+    __syncthreads();
+    const int64_t L = pref[nseg];
+    const bool whole = L == cell_ptr[nC];          // every item: stream them in id order, no cell_items lookup
+    int64_t per = max((L + S - 1) / S, (int64_t)kRtMinSplit);
+    per = (per + kRtTile - 1) / kRtTile * kRtTile;
+    const int64_t pb = min(L, (int64_t)split * per);
+    const int64_t pe = min(L, pb + per);
+
+    for (int64_t p0 = pb; p0 < pe; p0 += kRtTile) {
+      const int64_t p = p0 + tid;
+      int item = 0;
+      unsigned in = 0;                             // bit u: the item is inside row u's radius (rows of this window)
+      if (p < pe) {
+        int l = 0, h = nseg;                       // the run holding p: the last j with pref[j] <= p
+        while (!whole && h - l > 1) {
+          const int mid = (l + h) >> 1;
+          if (pref[mid] <= p) l = mid; else h = mid;
+        }
+        item = whole ? (int)p : cell_items[seg[l] + (int)(p - pref[l])];
+        const double px = P[3 * (int64_t)item], py = P[3 * (int64_t)item + 1], pz = P[3 * (int64_t)item + 2];
+#pragma unroll
+        for (int u = 0; u < TU; ++u) {
+          if (pass[u] != 1) continue;
+          if (cq[4 * u + 3] == -INFINITY) { in |= 1u << u; continue; }   // every finite dot product is >= -inf
+          const double dot = __dadd_rn(__dadd_rn(__dmul_rn(cq[4 * u], px), __dmul_rn(cq[4 * u + 1], py)),
+                                       __dmul_rn(cq[4 * u + 2], pz));
+          if (dot >= cq[4 * u + 3]) in |= 1u << u;
+        }
+      }
+      float acc[TU];
+      rt_score<T, TU>(in ? V + (int64_t)item * d : nullptr, Us, d, acc);
+      if (in) {
+        float bias = 0.f;
+        if constexpr (kBias) bias = __ldg(item_bias + item);
+#pragma unroll
+        for (int u = 0; u < TU; ++u) {
+          if (!((in >> u) & 1u)) continue;
+          float s = kBias ? acc[u] + bias : acc[u];
+          if (s == 0.f) s = 0.f;                   // -0 ranks like +0
+          if (!(s > -INFINITY)) continue;          // -inf or NaN: never returned
+          const uint64_t key = rt_key(s, (uint32_t)item);
+          if (key <= thr[u]) continue;
+          if (seen_ptr && geo_listed(seen_idx, sb[u], se[u], item)) continue;
+          const int q = atomicAdd(cnt + u, 1);
+          keys[(size_t)u * CAP + q] = key;
+        }
+      }
+      __syncthreads();
+      bool full = p0 + kRtTile >= pe;              // the last tile: truncate to the K best
+#pragma unroll
+      for (int u = 0; u < TU; ++u) full |= cnt[u] > CAP - kRtTile;   // the next tile could overflow a buffer
+      if (full) rt_compact<TU>(keys, cnt, thr, K);
+    }
+    if (tid < TU && pass[tid] == 1) pass[tid] = 2;
+    __syncthreads();
+  }
+
+  // every buffer that took an offer was truncated after its window's last tile: its first cnt keys are its K best
+  for (int i = tid; i < TU * K; i += kRtThreads) {
+    const int u = i / K, j = i - u * K;
+    const int b = rowb[u];
+    if (b < 0) continue;
+    const uint64_t key = j < cnt[u] ? keys[(size_t)u * CAP + j] : 0;   // zero beyond the user's count: padding
+    if (partial) {
+      partial[((int64_t)split * B + b) * K + j] = key;
+    } else {
+      int64_t id; float s;
+      rt_decode(key, id, s);
+      out_ids[(int64_t)b * K + j] = id;
+      out_scores[(int64_t)b * K + j] = s;
+    }
+  }
+}
+
 }  // namespace yr
 
 using namespace yr;
@@ -693,6 +990,41 @@ int rs_splits(int64_t B, int64_t max_len, int K, int TU) {
 size_t rs_partial_bytes(int S, int64_t B, int K) { return S > 1 ? (size_t)S * (size_t)B * (size_t)K * sizeof(uint64_t) : 0; }
 
 size_t rs_plan_bytes(int64_t B, int G) { return ((size_t)3 * G + 8 + (size_t)B) * sizeof(int32_t); }
+
+size_t geo_smem_bytes(int TU, int d) {
+  return (size_t)kRtEntries * 8 + (size_t)TU * 8 + (size_t)TU * 4 * 8 + (size_t)TU * d * 4 + 5 * (size_t)TU * 4 +
+         (size_t)(8 + 2 * kGeoMaxSegs + 1 + 16) * 4;
+}
+
+// Hash buckets of the row grouping: about two per row (few collisions), at most 2^16 (the plan scans them all).
+int geo_buckets(int64_t B) {
+  int64_t H = 64;
+  while (H < 2 * B && H < (1 << 16)) H <<= 1;
+  return (int)H;
+}
+
+// Workspace: per-split lists | bucket int64 [B] | plan | windows int32 [B][kGeoWin].
+size_t geo_ws_bytes(int S, int64_t B, int K) {
+  return rs_partial_bytes(S, B, K) + (size_t)B * 8 + rs_plan_bytes(B, geo_buckets(B)) + (size_t)B * kGeoWin * 4;
+}
+
+template <typename T, int TU, bool kBias>
+int geo_launch(const void* U, int64_t nU, const void* V, int d, const int64_t* uids, int64_t B, const int64_t* cell_keys,
+               const int32_t* cell_ptr, int64_t nC, const int32_t* cell_items, const double* P, int nlon, const double* c,
+               const double* t, const int32_t* win, int H, const int32_t* rows_at, const int32_t* blocks_at,
+               const int32_t* order, const int32_t* seen_ptr, const int32_t* seen_idx, int K, int S, uint64_t* partial,
+               int64_t* out_ids, float* out_scores, int32_t* err, const float* item_bias, cudaStream_t s) {
+  static AttrOnce attr;
+  int rc = attr.set(recommend_geo_kernel<T, TU, kBias>, (int)geo_smem_bytes(TU, rt_max_d(TU)));
+  if (rc) return rc;
+  dim3 grid((unsigned)((B + TU - 1) / TU + std::min<int64_t>((int64_t)H + 2, B)), (unsigned)S);
+  recommend_geo_kernel<T, TU, kBias><<<grid, kRtThreads, geo_smem_bytes(TU, d), s>>>(
+      reinterpret_cast<const T*>(U), nU, reinterpret_cast<const T*>(V), d, uids, B, cell_keys, cell_ptr, nC, cell_items,
+      P, nlon, c, t, win, H, rows_at, blocks_at, order, seen_ptr, seen_idx, K, S, partial, out_ids, out_scores, err,
+      item_bias);
+  YR_CHECK_LAUNCH();
+  return YR_OK;
+}
 
 int merge_launch(const uint64_t* partial, int S, int64_t B, int K, int64_t* out_ids, float* out_scores, cudaStream_t s) {
   const int P = rt_pow2(S * K);
@@ -813,6 +1145,64 @@ extern "C" int yr_recommend_subset_topk_ex(const void* U, int64_t nU, const void
     rc = item_bias ? YR_RS_TU(__nv_bfloat16, true) : YR_RS_TU(__nv_bfloat16, false);
 #undef YR_RS_TU
 #undef YR_RS_LAUNCH
+  if (rc || S == 1) return rc;
+  return merge_launch(partial, S, B, K, out_ids, out_scores, s);
+}
+
+extern "C" size_t yr_recommend_geo_ws_bytes(int64_t B, int64_t nI, int K) {
+  if (B <= 0 || B >= 0x7fffffffLL || nI <= 0 || K <= 0 || K > kRtMaxK) return 0;
+  return geo_ws_bytes(rs_splits(B, nI, K, rt_users_per_block(K)), B, K);
+}
+
+extern "C" int yr_recommend_geo_topk(const void* U, int64_t nU, const void* V, int64_t nI, int d, int dtype,
+                                     const int64_t* user_ids, int64_t B, const int64_t* cell_keys,
+                                     const int32_t* cell_ptr, int64_t num_cells, const int32_t* cell_items,
+                                     const double* item_xyz, double cell_deg, int64_t num_lat, int64_t num_lon,
+                                     const double* centre_xyz, const double* threshold, const int32_t* seen_ptr,
+                                     const int32_t* seen_idx, int K, int64_t* out_ids, float* out_scores, void* ws,
+                                     size_t ws_bytes, int32_t* err, yr_stream stream, const float* item_bias) {
+  if (!U || !V || !out_ids || !out_scores || !cell_keys || !cell_ptr || !cell_items || !item_xyz) return YR_ERR_BAD_ARG;
+  if (B > 0 && (!user_ids || !centre_xyz || !threshold)) return YR_ERR_BAD_ARG;
+  if ((seen_ptr == nullptr) != (seen_idx == nullptr)) return YR_ERR_BAD_ARG;
+  if (B < 0 || B >= 0x7fffffffLL || nU <= 0 || K <= 0 || K > kRtMaxK) return YR_ERR_BAD_ARG;
+  if (!(cell_deg > 0.0) || !(cell_deg <= 360.0) || num_lat < 1 || num_lon < 1 || num_lat > 0x7fffffffLL ||
+      num_lon > 0x7fffffffLL || num_cells < 0 || num_cells > nI)
+    return YR_ERR_BAD_ARG;
+  if (nI <= 0 || nI >= 0x7fffffffLL || d <= 0 || d > kRtMaxD || (d & 7) != 0) return YR_ERR_BAD_DIM;
+  if (dtype != YR_DTYPE_F32 && dtype != YR_DTYPE_BF16) return YR_ERR_BAD_ARG;
+  if (B == 0) return YR_OK;
+  const int TU = rt_users(K, d);
+  const int S = rs_splits(B, nI, K, TU);
+  const int H = geo_buckets(B);
+  if (!ws || ws_bytes < geo_ws_bytes(S, B, K)) return YR_ERR_WORKSPACE;
+  cudaStream_t s = (cudaStream_t)stream;
+  const size_t pbytes = rs_partial_bytes(S, B, K);
+  uint64_t* partial = S > 1 ? reinterpret_cast<uint64_t*>(ws) : nullptr;
+  int64_t* bucket = reinterpret_cast<int64_t*>(reinterpret_cast<char*>(ws) + pbytes);   // [B]
+  int32_t* cursor = reinterpret_cast<int32_t*>(bucket + B);                              // [H + 2]
+  int32_t* rows_at = cursor + H + 2;                                                      // [H + 3]
+  int32_t* blocks_at = rows_at + H + 3;                                                   // [H + 3]
+  int32_t* order = blocks_at + H + 3;                                                     // [B]
+  int32_t* win = order + B;                                                               // [B][kGeoWin]
+  recommend_geo_window_kernel<<<(unsigned)((B + kRtThreads - 1) / kRtThreads), kRtThreads, 0, s>>>(
+      centre_xyz, threshold, B, cell_deg, (int)num_lat, (int)num_lon, H, win, bucket, err);
+  YR_CHECK_LAUNCH();
+  recommend_subset_plan_kernel<<<1, kRsPlanThreads, 0, s>>>(bucket, (int)B, H, TU, cursor, rows_at, blocks_at, order,
+                                                            err);
+  YR_CHECK_LAUNCH();
+  int rc;
+#define YR_GEO_LAUNCH(T, TU_, BIAS)                                                                                       \
+  geo_launch<T, TU_, BIAS>(U, nU, V, d, user_ids, B, cell_keys, cell_ptr, num_cells, cell_items, item_xyz, (int)num_lon, \
+                           centre_xyz, threshold, win, H, rows_at, blocks_at, order, seen_ptr, seen_idx, K, S, partial,  \
+                           out_ids, out_scores, err, item_bias, s)
+#define YR_GEO_TU(T, BIAS)                                                                                                \
+  (TU == 16 ? YR_GEO_LAUNCH(T, 16, BIAS) : TU == 8 ? YR_GEO_LAUNCH(T, 8, BIAS) : YR_GEO_LAUNCH(T, 4, BIAS))
+  if (dtype == YR_DTYPE_F32)
+    rc = item_bias ? YR_GEO_TU(float, true) : YR_GEO_TU(float, false);
+  else
+    rc = item_bias ? YR_GEO_TU(__nv_bfloat16, true) : YR_GEO_TU(__nv_bfloat16, false);
+#undef YR_GEO_TU
+#undef YR_GEO_LAUNCH
   if (rc || S == 1) return rc;
   return merge_launch(partial, S, B, K, out_ids, out_scores, s);
 }

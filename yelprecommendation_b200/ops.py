@@ -777,3 +777,105 @@ def recommend_subset_topk(U: torch.Tensor, V: torch.Tensor, user_ids: torch.Tens
     if e & 2:
         raise IndexError(f"recommend_subset_topk: subset id out of range [-1, {G})")
     return ids, scores
+
+
+def geo_grid_shape(cell_deg: float) -> Tuple[int, int]:
+    """(lat bands, lon bands) of the item grid with cells of cell_deg degrees: ceil(180 / w), ceil(360 / w)."""
+    import math
+    return int(math.ceil(180.0 / cell_deg)), int(math.ceil(360.0 / cell_deg))
+
+
+def recommend_geo_topk(U: torch.Tensor, V: torch.Tensor, user_ids: torch.Tensor, K: int, cell_keys: torch.Tensor,
+                       cell_ptr: torch.Tensor, cell_items: torch.Tensor, item_xyz: torch.Tensor, cell_deg: float,
+                       centre_xyz: torch.Tensor, threshold: torch.Tensor, seen_ptr: Optional[torch.Tensor] = None,
+                       seen_idx: Optional[torch.Tensor] = None,
+                       item_bias: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """yr_recommend_geo_topk: recommend_topk with row b restricted to the items i inside its radius,
+    ((c_x * p_x) + (c_y * p_y)) + (c_z * p_z) >= threshold[b] in float64 with c = centre_xyz[b] and p = item_xyz[i] (unit
+    vectors, float64 [B x 3] and [nI x 3]); threshold = cos(radius / Earth radius), -inf for every item. The item grid
+    (cell_keys int64, cell_ptr int32, cell_items int32 and cells of cell_deg degrees) is retrieval.ItemLocations'; it
+    bounds which items are read, never the result. Seen lists are indexed by user id. (ids int64 [B x K], scores float32
+    [B x K]), identical to recommend_topk with the items outside each row's radius excluded. A user id out of range
+    raises IndexError, a non-finite centre or a NaN / +inf threshold ValueError (both after the launch, from the error
+    word: one scalar read per call)."""
+    if not all(torch.is_tensor(x) for x in (cell_keys, cell_ptr, cell_items, item_xyz, centre_xyz, threshold)):
+        raise TypeError("recommend_geo_topk: the item grid, item_xyz, centre_xyz and threshold must be tensors")
+    if not (torch.is_tensor(U) and torch.is_tensor(V) and torch.is_tensor(user_ids)):
+        raise TypeError("recommend_geo_topk: U, V and user_ids must be tensors")
+    if not (U.is_cuda and V.is_cuda and user_ids.is_cuda):
+        raise YelprecError("recommend_geo_topk: U, V and user_ids must be CUDA tensors (the reference path is "
+                           "retrieval.recommend_reference)")
+    dev = U.device
+    if V.device != dev or user_ids.device != dev:
+        raise ValueError(f"recommend_geo_topk: tensors on different devices ({U.device}, {V.device}, {user_ids.device})")
+    if U.dtype not in _RT_DTYPES or V.dtype != U.dtype:
+        raise TypeError(f"recommend_geo_topk: U and V must both be float32 or both bfloat16, got {U.dtype} and {V.dtype}")
+    if U.dim() != 2 or V.dim() != 2 or U.shape[1] != V.shape[1]:
+        raise ValueError(f"recommend_geo_topk: U [nU x d] and V [nI x d] expected, got {tuple(U.shape)} and "
+                         f"{tuple(V.shape)}")
+    d = int(U.shape[1])
+    if d % 8 != 0 or d > RECOMMEND_MAX_D:
+        raise ValueError(f"recommend_geo_topk: embedding width {d} must be a multiple of 8 and at most {RECOMMEND_MAX_D}")
+    nU, nI = int(U.shape[0]), int(V.shape[0])
+    if nU == 0 or nI == 0 or nI >= 2 ** 31 - 1:
+        raise ValueError(f"recommend_geo_topk: {nU} users x {nI} items is not a valid catalog")
+    if isinstance(K, bool) or int(K) != K or not 1 <= int(K) <= RECOMMEND_MAX_K:
+        raise ValueError(f"recommend_geo_topk: k must be an integer in [1, {RECOMMEND_MAX_K}], got {K}")
+    K = int(K)
+    if user_ids.dtype not in (I64, I32) or user_ids.dim() != 1:
+        raise TypeError(f"recommend_geo_topk: user_ids must be a 1-D int64 or int32 tensor, got {user_ids.dtype} "
+                        f"{tuple(user_ids.shape)}")
+    B = int(user_ids.numel())
+    if centre_xyz.dtype != F64 or threshold.dtype != F64:
+        raise TypeError(f"recommend_geo_topk: centre_xyz and threshold must be float64, got {centre_xyz.dtype} and "
+                        f"{threshold.dtype}")
+    if tuple(centre_xyz.shape) != (B, 3) or tuple(threshold.shape) != (B,):
+        raise ValueError(f"recommend_geo_topk: centre_xyz [{B} x 3] and threshold [{B}] expected, got "
+                         f"{tuple(centre_xyz.shape)} and {tuple(threshold.shape)}")
+    if item_xyz.dtype != F64 or tuple(item_xyz.shape) != (nI, 3):
+        raise ValueError(f"recommend_geo_topk: item_xyz must be float64 [{nI} x 3]")
+    if cell_keys.dtype != I64 or cell_ptr.dtype != I32 or cell_items.dtype != I32 or cell_keys.dim() != 1 or \
+            cell_ptr.numel() != cell_keys.numel() + 1 or cell_items.numel() != nI:
+        raise ValueError("recommend_geo_topk: the item grid must be cell_keys int64 [C], cell_ptr int32 [C + 1] and "
+                         f"cell_items int32 [{nI}]")
+    if any(x.device != dev for x in (cell_keys, cell_ptr, cell_items, item_xyz, centre_xyz, threshold)):
+        raise ValueError("recommend_geo_topk: the item grid, item_xyz, centre_xyz and threshold must live on the device "
+                         "of the embeddings")
+    cell_deg = float(cell_deg)
+    if not 0.0 < cell_deg <= 360.0:
+        raise ValueError(f"recommend_geo_topk: cell_deg must be in (0, 360], got {cell_deg}")
+    nlat, nlon = geo_grid_shape(cell_deg)
+    if (seen_ptr is None) != (seen_idx is None):
+        raise ValueError("recommend_geo_topk: seen_ptr and seen_idx go together")
+    bias = _item_bias(item_bias, nI, dev, "recommend_geo_topk")
+    if seen_ptr is not None:
+        if seen_ptr.dtype != I32 or seen_idx.dtype != I32 or seen_ptr.numel() != nU + 1:
+            raise ValueError(f"recommend_geo_topk: seen lists must be int32 CSR with {nU + 1} offsets")
+        if seen_ptr.device != dev or seen_idx.device != dev:
+            raise ValueError("recommend_geo_topk: seen lists must live on the device of the embeddings")
+        seen_ptr = seen_ptr.contiguous()
+        seen_idx = seen_idx.contiguous() if seen_idx.numel() else torch.zeros(1, dtype=I32, device=dev)
+    uid = user_ids.to(I64).contiguous()
+    keys = cell_keys.contiguous() if cell_keys.numel() else torch.zeros(1, dtype=I64, device=dev)
+    cptr, citems, P = cell_ptr.contiguous(), cell_items.contiguous(), item_xyz.contiguous()
+    c, t = centre_xyz.contiguous(), threshold.contiguous()
+    lib = _cabi.load()
+    Uc, Vc = U.detach().contiguous(), V.detach().contiguous()
+    ids = torch.empty(B, K, device=dev, dtype=I64)
+    scores = torch.empty(B, K, device=dev, dtype=F32)
+    if B == 0:
+        return ids, scores
+    err = torch.zeros(1, device=dev, dtype=I32)
+    nbytes = lib.yr_recommend_geo_ws_bytes(B, nI, K)
+    ws = torch.empty(max(nbytes, 1), device=dev, dtype=torch.uint8)
+    check(lib.yr_recommend_geo_topk(Uc.data_ptr(), nU, Vc.data_ptr(), nI, d, _RT_DTYPES[U.dtype], dptr(uid, I64), B,
+                                    dptr(keys, I64), dptr(cptr, I32), int(cell_keys.numel()), dptr(citems, I32),
+                                    dptr(P, F64), cell_deg, nlat, nlon, dptr(c, F64), dptr(t, F64), dptr(seen_ptr),
+                                    dptr(seen_idx), K, dptr(ids), dptr(scores), dptr(ws), nbytes, dptr(err),
+                                    stream_ptr(dev), dptr(bias)), "yr_recommend_geo_topk")
+    e = int(err.item())
+    if e & 1:
+        raise IndexError(f"recommend_geo_topk: user id out of range [0, {nU})")
+    if e & 2:
+        raise ValueError("recommend_geo_topk: a centre is not finite or a threshold is NaN or +inf")
+    return ids, scores

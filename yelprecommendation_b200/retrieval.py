@@ -23,6 +23,17 @@ ids and scores equal what the unrestricted kernel returns with every item outsid
 
 A CDAE user is encoded from their interaction list (yr_cdae_encode), and the output bias enters the retrieval kernels as a
 per-item bias added after the dot product.
+
+    places = ItemLocations.from_degrees(item_lat, item_lon)    # where each item is
+    rec = Recommender(user_emb, item_emb, seen, locations=places)
+    ids, scores = rec.recommend(user_ids, k=20, near=(lat, lon), radius_km=5)   # only items within 5 km
+
+With `near`, row b ranks only the items inside its radius, decided by one exact float64 predicate shared by the kernel
+(yr_recommend_geo_topk) and the reference: item i is inside iff ((c_x * p_x) + (c_y * p_y)) + (c_z * p_z) >= t, each
+product and sum rounded on its own, with p = ItemLocations.P[i], c the centre's unit vector and t = cos(radius_km /
+EARTH_RADIUS_KM) (-inf from half the Earth's circumference on), all computed on the host by geo_query. The kernel reads
+only the items of the grid cells around each centre; ids and scores equal what the unrestricted kernel returns with every
+item outside the radius excluded.
 """
 from __future__ import annotations
 
@@ -34,6 +45,125 @@ import torch
 from . import ops
 
 I32, I64, F32 = torch.int32, torch.int64, torch.float32
+
+
+EARTH_RADIUS_KM = 6371.0088          # mean Earth radius (IUGG)
+GEO_MIN_CELL_KM = 0.01               # grid cells at least 10 m wide: the window's one-cell margin covers float64 rounding
+
+
+def _unit_xyz(lat: np.ndarray, lon: np.ndarray) -> np.ndarray:
+    """float64 [n x 3] unit vectors (cos(phi) cos(lam), cos(phi) sin(lam), sin(phi)) of (lat, lon) in degrees."""
+    phi, lam = np.radians(lat), np.radians(lon)
+    return np.stack([np.cos(phi) * np.cos(lam), np.cos(phi) * np.sin(lam), np.sin(phi)], axis=1)
+
+
+def _check_degrees(lat: np.ndarray, lon: np.ndarray, what: str) -> None:
+    if not (np.isfinite(lat).all() and np.isfinite(lon).all()):
+        raise ValueError(f"{what}: coordinates must be finite")
+    if lat.size and np.abs(lat).max() > 90.0:
+        raise ValueError(f"{what}: latitude outside [-90, 90]")
+    if lon.size and np.abs(lon).max() > 180.0:
+        raise ValueError(f"{what}: longitude outside [-180, 180]")
+
+
+def _as_f64(x) -> np.ndarray:
+    return np.asarray(x.detach().cpu().numpy() if torch.is_tensor(x) else x, dtype=np.float64)
+
+
+class ItemLocations:
+    """Item positions on the sphere and a grid index over them, for radius-restricted retrieval.
+
+    P: float64 [num_items x 3], the unit vector of each item's (lat, lon). The grid: cells of cell_deg degrees of latitude
+    and longitude (cell_km of arc along a meridian); an item is in lat band floor((lat + 90) / cell_deg) and lon band
+    floor((lon + 180) / cell_deg), each clamped to the grid, cell key = lat band * num_lon + lon band. cell_items int32
+    [num_items] holds the item ids sorted by (key, id), cell_keys int64 the ascending keys of the non-empty cells and
+    cell_ptr int32 their offsets into cell_items. The cell size sets how many items a request reads, never its result."""
+
+    def __init__(self, lat, lon, cell_km: float = 2.0):
+        lat, lon = _as_f64(lat).reshape(-1), _as_f64(lon).reshape(-1)
+        if lat.shape != lon.shape:
+            raise ValueError(f"ItemLocations: {lat.size} latitudes but {lon.size} longitudes")
+        _check_degrees(lat, lon, "ItemLocations")
+        cell_km = float(cell_km)
+        if not cell_km >= GEO_MIN_CELL_KM or not np.isfinite(cell_km):
+            raise ValueError(f"ItemLocations: cell_km must be finite and at least {GEO_MIN_CELL_KM}, got {cell_km}")
+        n = lat.size
+        self.num_items, self.cell_km = n, cell_km
+        self.cell_deg = min(float(np.degrees(cell_km / EARTH_RADIUS_KM)), 360.0)
+        self.num_lat, self.num_lon = ops.geo_grid_shape(self.cell_deg)
+        self.P = torch.from_numpy(_unit_xyz(lat, lon))
+        lat_band = np.clip(np.floor((lat + 90.0) / self.cell_deg), 0, self.num_lat - 1).astype(np.int64)
+        lon_band = np.clip(np.floor((lon + 180.0) / self.cell_deg), 0, self.num_lon - 1).astype(np.int64)
+        key = lat_band * self.num_lon + lon_band
+        order = np.lexsort((np.arange(n), key))
+        keys, first = np.unique(key[order], return_index=True)
+        self.cell_items = torch.from_numpy(order.astype(np.int32))
+        self.cell_keys = torch.from_numpy(keys.astype(np.int64))
+        self.cell_ptr = torch.from_numpy(np.append(first, n).astype(np.int32))
+        self._on = {}
+
+    @classmethod
+    def from_degrees(cls, lat, lon, cell_km: float = 2.0) -> "ItemLocations":
+        """From each item's latitude and longitude in degrees (item i at (lat[i], lon[i])). ValueError on non-finite
+        coordinates, |lat| > 90 or |lon| > 180."""
+        return cls(lat, lon, cell_km)
+
+    def on(self, device) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+        """(cell_keys, cell_ptr, cell_items, P) on `device`, copied once per device."""
+        device = torch.device(device)
+        if device.type == "cuda" and device.index is None:
+            device = torch.device("cuda", torch.cuda.current_device())
+        if device not in self._on:
+            self._on[device] = tuple(x.to(device) for x in (self.cell_keys, self.cell_ptr, self.cell_items, self.P))
+        return self._on[device]
+
+
+def geo_query(near, radius_km, B: int) -> Tuple[np.ndarray, np.ndarray]:
+    """(c float64 [B x 3], t float64 [B]) of B radius requests: near = one (lat, lon) pair in degrees for every row, or
+    two length-B sequences; radius_km = one value or B values, each > 0. c is the centre's unit vector, t =
+    cos(radius_km / EARTH_RADIUS_KM), or -inf when radius_km >= pi * EARTH_RADIUS_KM (every item). The one place where
+    requests become the predicate's operands, for the kernel and the reference alike."""
+    if near is None or radius_km is None:
+        raise ValueError("recommend: near and radius_km go together")
+    try:
+        lat, lon = near
+    except (TypeError, ValueError):
+        raise ValueError("recommend: near must be a (lat, lon) pair, or two sequences of B values") from None
+    lat, lon = _as_f64(lat), _as_f64(lon)
+    if lat.ndim == 0 and lon.ndim == 0:
+        lat, lon = np.full(B, float(lat)), np.full(B, float(lon))
+    elif lat.shape != (B,) or lon.shape != (B,):
+        raise ValueError(f"recommend: near must be one (lat, lon) pair or two sequences of {B} values, got shapes "
+                         f"{lat.shape} and {lon.shape}")
+    _check_degrees(lat, lon, "recommend")
+    r = _as_f64(radius_km)
+    if r.ndim == 0:
+        r = np.full(B, float(r))
+    elif r.shape != (B,):
+        raise ValueError(f"recommend: radius_km must be one value or {B} values, got shape {r.shape}")
+    if np.isnan(r).any() or (r <= 0).any():
+        raise ValueError("recommend: radius_km must be > 0")
+    whole = r >= np.pi * EARTH_RADIUS_KM
+    t = np.where(whole, -np.inf, np.cos(np.where(whole, 0.0, r) / EARTH_RADIUS_KM))
+    return _unit_xyz(lat, lon).reshape(B, 3), t
+
+
+def _geo_inside(P: torch.Tensor, c: torch.Tensor, t: torch.Tensor) -> torch.Tensor:
+    """bool [B x nI]: ((c_x * p_x) + (c_y * p_y)) + (c_z * p_z) >= t_b, float64, one rounded operation at a time."""
+    return ((c[:, 0:1] * P[None, :, 0]) + (c[:, 1:2] * P[None, :, 1])) + (c[:, 2:3] * P[None, :, 2]) >= t[:, None]
+
+
+def _geo_args(subset, near, radius_km, locations: Optional[ItemLocations], nI: int, what: str) -> bool:
+    """Whether a request is radius-restricted, after checking that it can be."""
+    if near is None and radius_km is None:
+        return False
+    if subset is not None:
+        raise ValueError("recommend: subset and near cannot be combined")
+    if locations is None:
+        raise ValueError(f"recommend: near needs the item locations ({what}(..., locations=ItemLocations...))")
+    if locations.num_items != nI:
+        raise ValueError(f"recommend: locations cover {locations.num_items} items, the item table {nI}")
+    return True
 
 
 class ItemLists:
@@ -164,10 +294,13 @@ def _subset_rows(subset, B: int, subsets: Optional[ItemSubsets]):
 
 def recommend_reference(user_emb: torch.Tensor, item_emb: torch.Tensor, user_ids, k: int,
                         seen: Optional[SeenItems] = None, subsets: Optional[ItemSubsets] = None,
-                        subset=None, item_bias: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
-    """Plain PyTorch on the tables' device: dense [B x num_items] scores (+ item_bias [num_items], fp32), seen items and
-    items outside the row's subset (subsets[subset[b]]; -1 = whole catalog) set to -inf, a stable descending sort
-    (torch.topk does not fix the order of ties), and slots holding -inf turned into padding (id -1)."""
+                        subset=None, item_bias: Optional[torch.Tensor] = None,
+                        locations: Optional[ItemLocations] = None, near=None,
+                        radius_km=None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Plain PyTorch on the tables' device: dense [B x num_items] scores (+ item_bias [num_items], fp32), seen items,
+    items outside the row's subset (subsets[subset[b]]; -1 = whole catalog) and items outside the row's radius (near,
+    radius_km: geo_query's predicate over locations.P) set to -inf, a stable descending sort (torch.topk does not fix the
+    order of ties), and slots holding -inf turned into padding (id -1)."""
     k = _check_k(k)
     dev = user_emb.device
     uid = torch.as_tensor(user_ids).to(device=dev, dtype=I64).reshape(-1)
@@ -175,6 +308,7 @@ def recommend_reference(user_emb: torch.Tensor, item_emb: torch.Tensor, user_ids
     if uid.numel() and (int(uid.min()) < 0 or int(uid.max()) >= nU):
         raise IndexError(f"recommend: user id out of range [0, {nU})")
     B = uid.numel()
+    geo = _geo_args(subset, near, radius_km, locations, nI, "Recommender")
     scores = user_emb[uid].to(F32) @ item_emb.to(F32).T
     if item_bias is not None:
         scores = scores + item_bias.to(device=dev, dtype=F32)[None, :]
@@ -193,6 +327,11 @@ def recommend_reference(user_emb: torch.Tensor, item_emb: torch.Tensor, user_ids
         row, item = _list_entries(subsets, sid[limited], dev)
         outside[limited[row], item] = False
         scores[outside] = float("-inf")
+    if geo:
+        c, t = geo_query(near, radius_km, B)
+        P = locations.P.to(dev)
+        inside = _geo_inside(P, torch.from_numpy(c).to(dev), torch.from_numpy(t).to(dev))
+        scores[~inside] = float("-inf")
     kk = min(k, nI)
     sc, order = torch.sort(scores, dim=1, descending=True, stable=True)
     sc, order = sc[:, :kk].contiguous(), order[:, :kk].contiguous()
@@ -205,10 +344,10 @@ def recommend_reference(user_emb: torch.Tensor, item_emb: torch.Tensor, user_ids
 
 class Recommender:
     """Top-K retrieval over fixed user / item tables ([num_users x d], [num_items x d], fp32 or bf16, same device),
-    optionally restricted per request to one of the item subsets."""
+    optionally restricted per request to one of the item subsets or to the items within a radius (locations)."""
 
     def __init__(self, user_emb: torch.Tensor, item_emb: torch.Tensor, seen: Optional[SeenItems] = None,
-                 subsets: Optional[ItemSubsets] = None):
+                 subsets: Optional[ItemSubsets] = None, locations: Optional[ItemLocations] = None):
         if user_emb.device != item_emb.device:
             raise ValueError(f"Recommender: user and item tables on different devices ({user_emb.device}, {item_emb.device})")
         if seen is not None and (seen.num_users != user_emb.shape[0] or seen.num_items != item_emb.shape[0]):
@@ -216,31 +355,48 @@ class Recommender:
                              f"{user_emb.shape[0]} x {item_emb.shape[0]}")
         if subsets is not None and subsets.num_items != item_emb.shape[0]:
             raise ValueError(f"Recommender: subsets cover {subsets.num_items} items, the item table {item_emb.shape[0]}")
+        if locations is not None and locations.num_items != item_emb.shape[0]:
+            raise ValueError(f"Recommender: locations cover {locations.num_items} items, the item table "
+                             f"{item_emb.shape[0]}")
         self.user_emb, self.item_emb, self.seen, self.subsets = user_emb.detach(), item_emb.detach(), seen, subsets
+        self.locations = locations
 
-    def recommend(self, user_ids, k: int, exclude_seen: bool = True, subset=None) -> Tuple[torch.Tensor, torch.Tensor]:
+    def recommend(self, user_ids, k: int, exclude_seen: bool = True, subset=None, near=None,
+                  radius_km=None) -> Tuple[torch.Tensor, torch.Tensor]:
         """(item ids int64 [B x k], scores float32 [B x k]) on the tables' device, best first. subset: None (the whole
         catalog), an int for every row, or B ints (-1 = whole catalog for that row): row b then ranks only the items of
         subsets[subset[b]]. Host-side subset ids let the number of item splits follow the requested subsets; on a CUDA
-        tensor it follows the whole catalog (no device read)."""
+        tensor it follows the whole catalog (no device read). near = (lat, lon) in degrees (one pair, or two sequences
+        of B values) with radius_km (one value or B values, > 0): row b ranks only the items within radius_km[b] of
+        near[b] (geo_query); not combined with subset."""
         if exclude_seen and self.seen is None:
             raise ValueError("recommend: exclude_seen=True needs the seen items (Recommender(..., seen=SeenItems...))")
         seen = self.seen if exclude_seen else None
         dev = self.user_emb.device
         if subset is not None and self.subsets is None:
             raise ValueError("recommend: subset needs the item subsets (Recommender(..., subsets=ItemSubsets...))")
+        _geo_args(subset, near, radius_km, self.locations, self.item_emb.shape[0], "Recommender")
         if dev.type != "cuda":
-            return recommend_reference(self.user_emb, self.item_emb, user_ids, k, seen, self.subsets, subset)
+            return recommend_reference(self.user_emb, self.item_emb, user_ids, k, seen, self.subsets, subset,
+                                       locations=self.locations, near=near, radius_km=radius_km)
         uid = user_ids if torch.is_tensor(user_ids) else torch.as_tensor(np.asarray(user_ids, dtype=np.int64))
         uid = uid.to(dev).reshape(-1)
         ptr, idx = seen.on(dev) if seen is not None else (None, None)
-        return _recommend_kernel(self.user_emb, self.item_emb, uid, k, ptr, idx, self.subsets, subset)
+        return _recommend_kernel(self.user_emb, self.item_emb, uid, k, ptr, idx, self.subsets, subset,
+                                 locations=self.locations, near=near, radius_km=radius_km)
 
 
-def _recommend_kernel(U, V, uid, k, seen_ptr, seen_idx, subsets: Optional[ItemSubsets], subset, item_bias=None):
-    """ops.recommend_topk, or with `subset` ops.recommend_subset_topk: seen lists indexed by uid, which is on U's device.
-    Host-side subset ids let the number of item splits follow the requested subsets; on a CUDA tensor it follows the whole
-    catalog (no device read)."""
+def _recommend_kernel(U, V, uid, k, seen_ptr, seen_idx, subsets: Optional[ItemSubsets], subset, item_bias=None,
+                      locations: Optional[ItemLocations] = None, near=None, radius_km=None):
+    """ops.recommend_topk, with `subset` ops.recommend_subset_topk, with `near` ops.recommend_geo_topk: seen lists indexed
+    by uid, which is on U's device. Host-side subset ids let the number of item splits follow the requested subsets; on a
+    CUDA tensor it follows the whole catalog (no device read)."""
+    if _geo_args(subset, near, radius_km, locations, V.shape[0], "Recommender"):
+        c, t = geo_query(near, radius_km, uid.numel())
+        keys, cptr, items, P = locations.on(U.device)
+        return ops.recommend_geo_topk(U, V, uid, k, keys, cptr, items, P, locations.cell_deg,
+                                      torch.from_numpy(c).to(U.device), torch.from_numpy(t).to(U.device), seen_ptr,
+                                      seen_idx, item_bias=item_bias)
     if subset is None:
         return ops.recommend_topk(U, V, uid, k, seen_ptr, seen_idx, item_bias=item_bias)
     sid = _subset_rows(subset, uid.numel(), subsets)
@@ -268,7 +424,9 @@ def _cdae_check(model, seen: Optional[SeenItems], subsets: Optional[ItemSubsets]
 
 
 def cdae_recommend_reference(model, user_ids, k: int, seen: SeenItems, exclude_seen: bool = True,
-                             subsets: Optional[ItemSubsets] = None, subset=None) -> Tuple[torch.Tensor, torch.Tensor]:
+                             subsets: Optional[ItemSubsets] = None, subset=None,
+                             locations: Optional[ItemLocations] = None, near=None,
+                             radius_km=None) -> Tuple[torch.Tensor, torch.Tensor]:
     """Plain PyTorch restatement of CDAERecommender.recommend on the model's device: the dense multi-hot x of the users'
     seen items, z = act(x @ W_h^T + b_h + V_u[u]), then recommend_reference over the logits z . W_o[i] + b_o[i]."""
     _cdae_check(model, seen, subsets, "cdae_recommend_reference")
@@ -285,7 +443,8 @@ def cdae_recommend_reference(model, user_ids, k: int, seen: SeenItems, exclude_s
     z = pre if model.hidden_act == 1 else torch.sigmoid(pre)
     rows = SeenItems(*_batch_lists(seen, uid), B, model.num_items) if exclude_seen else None
     return recommend_reference(z, model.output_layer.weight.data, torch.arange(B, device=dev), k, rows, subsets, subset,
-                               item_bias=model.output_layer.bias.data)
+                               item_bias=model.output_layer.bias.data, locations=locations, near=near,
+                               radius_km=radius_km)
 
 
 def _batch_lists(seen: SeenItems, uid: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
@@ -304,19 +463,24 @@ class CDAERecommender:
     B x num_items input or output: z = act(W_h[:, seen[u]].sum(1) + b_h + V_u[u]) (yr_cdae_encode), then the fused
     retrieval kernel ranks the logits z . W_o[i] + b_o[i] (b_o as the per-item bias).
 
-    recommend(user_ids, k, exclude_seen=True, subset=None) has Recommender.recommend's contract: (item ids int64 [B x k],
-    scores float32 [B x k]), best first, ties to the lower id, short rows padded with -1 / -inf, the same subset semantics.
+    recommend(user_ids, k, exclude_seen=True, subset=None, near=None, radius_km=None) has Recommender.recommend's
+    contract: (item ids int64 [B x k], scores float32 [B x k]), best first, ties to the lower id, short rows padded with
+    -1 / -inf, the same subset and radius semantics.
     The scores are logits, the values CDAETrainer.evaluate ranks by; sigmoid(score) is the model's predicted probability.
     """
 
-    def __init__(self, model, seen: SeenItems, subsets: Optional[ItemSubsets] = None):
+    def __init__(self, model, seen: SeenItems, subsets: Optional[ItemSubsets] = None,
+                 locations: Optional[ItemLocations] = None):
         _cdae_check(model, seen, subsets, "CDAERecommender")
+        if locations is not None and locations.num_items != model.num_items:
+            raise ValueError(f"CDAERecommender: locations cover {locations.num_items} items, the model {model.num_items}")
         if model.hidden_layer.weight.device.type != "cuda":
             raise ops.YelprecError("CDAERecommender: the model must be on a CUDA device (the reference path is "
                                    "retrieval.cdae_recommend_reference)")
-        self.model, self.seen, self.subsets = model, seen, subsets
+        self.model, self.seen, self.subsets, self.locations = model, seen, subsets, locations
 
-    def recommend(self, user_ids, k: int, exclude_seen: bool = True, subset=None) -> Tuple[torch.Tensor, torch.Tensor]:
+    def recommend(self, user_ids, k: int, exclude_seen: bool = True, subset=None, near=None,
+                  radius_km=None) -> Tuple[torch.Tensor, torch.Tensor]:
         """(item ids int64 [B x k], logits float32 [B x k]) on the model's device, best first; see the class docstring."""
         m = self.model
         dev = m.hidden_layer.weight.device
@@ -328,6 +492,8 @@ class CDAERecommender:
         B = uid.numel()
         if subset is not None:
             _subset_rows(subset, B, self.subsets)
+        if _geo_args(subset, near, radius_km, self.locations, m.num_items, "CDAERecommender"):
+            geo_query(near, radius_km, B)
         if B == 0:
             return torch.empty(0, k, device=dev, dtype=I64), torch.empty(0, k, device=dev, dtype=F32)
         ptr, idx = self.seen.on(dev)
@@ -335,4 +501,5 @@ class CDAERecommender:
         rows = torch.arange(B, device=dev, dtype=I64)
         bptr, bidx = _batch_lists(self.seen, uid) if exclude_seen else (None, None)
         return _recommend_kernel(z, m.output_layer.weight.data, rows, k, bptr, bidx, self.subsets, subset,
-                                 item_bias=m.output_layer.bias.data)
+                                 item_bias=m.output_layer.bias.data, locations=self.locations, near=near,
+                                 radius_km=radius_km)

@@ -219,11 +219,12 @@ class CDAETrainer(BaseTrainer):
                     f"MAP@{k}: {result[2]:.4f} / NDCG@{k}: {result[3]:.4f}")
         return result
 
-    def recommender(self, seen=None, subsets=None):
+    def recommender(self, seen=None, subsets=None, locations=None):
         """retrieval.CDAERecommender over the model's live parameters (recommend(user_ids, k, exclude_seen=True,
-        subset=None); scores are output logits). `seen` is required: it is the users' input as well as what is excluded."""
+        subset=None, near=None, radius_km=None); scores are output logits). `seen` is required: it is the users' input as
+        well as what is excluded."""
         from ..retrieval import CDAERecommender
-        return CDAERecommender(self.model, seen, subsets)
+        return CDAERecommender(self.model, seen, subsets, locations)
 
     def run(self, train_dataloader, valid_dataloader):
         """Epoch loop of trainers/base_trainer.py:49-115 (validate returns the 5-tuple for CDAE)."""

@@ -177,10 +177,12 @@ class MFTrainer(BaseTrainer):
                         f"MAP@{k}: {result[2]:.4f} / NDCG@{k}: {result[3]:.4f}")
         return result
 
-    def recommender(self, seen=None, subsets=None):
-        """retrieval.Recommender over the current user / item tables (recommend(user_ids, k, exclude_seen=True, subset=None))."""
+    def recommender(self, seen=None, subsets=None, locations=None):
+        """retrieval.Recommender over the current user / item tables (recommend(user_ids, k, exclude_seen=True, subset=None,
+        near=None, radius_km=None))."""
         from ..retrieval import Recommender
-        return Recommender(self.model.user_embedding.weight.data, self.model.item_embedding.weight.data, seen, subsets)
+        return Recommender(self.model.user_embedding.weight.data, self.model.item_embedding.weight.data, seen, subsets,
+                           locations)
 
     def _generate_top_k_recommendation(self, pred: torch.Tensor, mask_items) -> np.ndarray:
         """One score row -> top-K item ids, best first (mf_trainer.py:163-178). Ties: (score desc, id asc)."""

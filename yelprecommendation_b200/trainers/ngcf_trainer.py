@@ -270,11 +270,11 @@ class NGCFTrainer(BaseTrainer):
                         f"MAP@{k}: {result[2]:.4f} / NDCG@{k}: {result[3]:.4f}")
         return result
 
-    def recommender(self, seen=None, subsets=None):
+    def recommender(self, seen=None, subsets=None, locations=None):
         """retrieval.Recommender over the propagated, layer-concatenated user / item embeddings that evaluate() ranks with."""
         from ..retrieval import Recommender
         cat = ops.ngcf_concat(self.propagate()[0])
-        return Recommender(cat[: self.num_users], cat[self.num_users:], seen, subsets)
+        return Recommender(cat[: self.num_users], cat[self.num_users:], seen, subsets, locations)
 
     def _generate_top_k_recommendation(self, pred: torch.Tensor, mask_items) -> np.ndarray:
         if not pred.is_cuda:
