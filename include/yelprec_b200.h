@@ -212,7 +212,8 @@ int yr_ngcf_tail(const float* const* E_layers, float* const* G_layers, int n_lay
                  int32_t* err, yr_stream stream);
 
 /* One dense torch.optim step over a flat parameter (Adam / AdamW / SGD, single-tensor op order of
- * torch.optim, trainers/base_trainer.py:34-40). m, v may be NULL for SGD. */
+ * torch.optim, trainers/base_trainer.py:34-40). m, v may be NULL for SGD. Any n and any 4-byte-aligned pointers
+ * (a view that starts inside a tensor); with 16-byte-aligned pointers the step runs on float4 accesses, same bits. */
 int yr_dense_opt_step(float* p, const float* g, float* m, float* v, int64_t n, const yr_opt* opt,
                       yr_stream stream);
 

@@ -422,15 +422,16 @@ __global__ void tail_finish_kernel(double* loss_acc, int64_t B, double* loss_sum
 }
 
 // ---------------------------------------------------------------------------------------------
-// Dense optimizer step, float4 vectorised with scalar tail.
+// Dense optimizer step, float4 vectorised with scalar tail. vec == 0 (a pointer that is not 16-byte aligned, e.g. a view
+// that starts inside a tensor): every element takes the scalar loop — same per-element arithmetic, same bits.
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
 dense_opt_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
-                 float* __restrict__ v, int64_t n, yr_opt opt) {
+                 float* __restrict__ v, int64_t n, yr_opt opt, int vec) {
   OptScalars os;
   opt_scalars_for_step(os, opt, opt.step);
   const bool adam = opt.kind != YR_OPT_SGD;
-  const int64_t n4 = n >> 2;
+  const int64_t n4 = vec ? n >> 2 : 0;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
     float4 pv = reinterpret_cast<float4*>(p)[i];
@@ -758,7 +759,9 @@ extern "C" int yr_dense_opt_step(float* p, const float* g, float* m, float* v, i
   if (blocks < 1) blocks = 1;
   const int64_t cap = (int64_t)yr_sm_count() * 8;
   if (blocks > cap) blocks = cap;
-  dense_opt_kernel<<<(unsigned)blocks, threads, 0, (cudaStream_t)stream>>>(p, g, m, v, n, *opt);
+  const bool adam = opt->kind != YR_OPT_SGD;
+  const int vec = (((uintptr_t)p | (uintptr_t)g | (adam ? ((uintptr_t)m | (uintptr_t)v) : 0)) & 15) == 0;
+  dense_opt_kernel<<<(unsigned)blocks, threads, 0, (cudaStream_t)stream>>>(p, g, m, v, n, *opt, vec);
   YR_CHECK_LAUNCH();
   return YR_OK;
 }
