@@ -104,15 +104,16 @@ def test_kernel_rejects_cpu_tensors():
         ops.recommend_topk(U, V, torch.zeros(2, dtype=I64), 3)
 
 
-def test_kernel_is_built_for_sm100a():
-    """The retrieval kernels are in the library as sm_100a SASS (one instance per table dtype and users-per-block)."""
+def test_kernel_instances_are_built_for_sm100a():
+    """The retrieval kernels are in the library as sm_100a SASS (one instance per table dtype, users-per-block and bias)."""
     from yelprecommendation_b200 import _cabi
     import __graft_entry__ as ge
     if not os.path.exists(_cabi.lib_path()):
         ge.build()
     out = subprocess.run(["cuobjdump", "-sass", _cabi.lib_path()], capture_output=True, text=True).stdout
     names = set(re.findall(r"Function : (\S*recommend\S*)", out))
-    assert len([n for n in names if "recommend_topk_kernel" in n]) == 6, names
+    assert len([n for n in names if "recommend_topk_kernel" in n]) == 12, names   # fp32 / bf16 x TU x bias
+    assert not any("_bias_kernel" in n for n in names), names
     assert any("recommend_merge_kernel" in n for n in names), names
     lib = _cabi.load()
     assert lib.yr_recommend_ws_bytes(0, 10, 5) == 0

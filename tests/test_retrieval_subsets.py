@@ -122,16 +122,17 @@ def test_subset_kernel_rejects_cpu_tensors():
         ops.recommend_subset_topk(U, V, z, 3, torch.zeros(2, dtype=I32), torch.zeros(1, dtype=I32), z, 9)
 
 
-def test_subset_kernel_is_built_for_sm100a():
-    """One subset kernel instance per table dtype and users-per-block, next to the 6 unrestricted ones."""
+def test_subset_kernel_instances_are_built_for_sm100a():
+    """One subset kernel instance per table dtype, users-per-block and bias, next to the 12 unrestricted ones."""
     from yelprecommendation_b200 import _cabi
     import __graft_entry__ as ge
     if not os.path.exists(_cabi.lib_path()):
         ge.build()
     out = subprocess.run(["cuobjdump", "-sass", _cabi.lib_path()], capture_output=True, text=True).stdout
     names = set(re.findall(r"Function : (\S*recommend\S*)", out))
-    assert len([n for n in names if "recommend_subset_kernel" in n]) == 6, names
-    assert len([n for n in names if "recommend_topk_kernel" in n]) == 6, names
+    assert len([n for n in names if "recommend_subset_kernel" in n]) == 12, names
+    assert len([n for n in names if "recommend_topk_kernel" in n]) == 12, names   # fp32 / bf16 x TU x bias
+    assert not any("_bias_kernel" in n for n in names), names
     assert any("recommend_subset_plan_kernel" in n for n in names), names
     assert _cabi.load().yr_recommend_subset_ws_bytes(0, 3, 10, 5) == 0
 

@@ -12,9 +12,10 @@
 //
 // recommend_subset_kernel restricts each row to one subset of the catalog (an ascending item-id list): the same scores,
 // masking and selection over the gathered ids of the row's subset, with rows grouped by subset on the device first.
+// recommend_geo_kernel restricts each row to the items within a radius (see below).
 //
-// The _bias kernels add a per-item fp32 bias to each score after the fma chain (a CDAE output layer: z . W_o[i] + b_o[i]);
-// they share their bodies with the unbiased kernels, whose code the bias does not touch.
+// Every scoring kernel takes kBias: with it, a per-item fp32 bias is added to each score after the fma chain (a CDAE
+// output layer: z . W_o[i] + b_o[i]); without it, item_bias is not read.
 #include <float.h>
 #include <algorithm>
 #include <cuda_bf16.h>
@@ -100,6 +101,40 @@ __device__ void rt_compact(uint64_t* keys, int* cnt, uint64_t* thr, int K) {
   __syncthreads();
 }
 
+// Dynamic shared memory of the scoring kernels: the byte offset of each array, laid end to end from (TU, d), and the
+// total. A kernel carves its arrays from its layout and the host takes the launch's byte count from the same layout.
+struct RtSmem {   // recommend_topk_kernel; keys [TU][kRtEntries / TU] at 0
+  size_t thr, Us, bits, cnt, mcur, mend, bytes;
+  __host__ __device__ RtSmem(int TU, int d)
+      : thr((size_t)kRtEntries * 8), Us(thr + (size_t)TU * 8), bits(Us + (size_t)TU * d * 4),
+        cnt(bits + (size_t)TU * (kRtTile / 32) * 4), mcur(cnt + (size_t)TU * 4), mend(mcur + (size_t)TU * 4),
+        bytes(mend + (size_t)TU * 4) {}
+};
+
+struct RsSmem : RtSmem {   // recommend_subset_kernel: RtSmem's arrays, then rowb and sid
+  size_t rowb, sid;
+  __host__ __device__ RsSmem(int TU, int d) : RtSmem(TU, d), rowb(bytes), sid(rowb + (size_t)TU * 4) {
+    bytes = sid + (size_t)kRtTile * 4;
+  }
+};
+
+template <typename E>
+__device__ __forceinline__ E* rt_at(uint64_t* smem, size_t offset) {
+  return reinterpret_cast<E*>(reinterpret_cast<char*>(smem) + offset);
+}
+
+// Us[u][0..d) = the row of U of each of the TU users that has one (has_row(u, uid)) as floats, zeros for the others.
+template <typename T, int TU, typename HasRow>
+__device__ __forceinline__ void rt_stage_users(float* Us, const T* U, int d, HasRow has_row) {
+  for (int i = threadIdx.x; i < TU * d; i += kRtThreads) {
+    const int u = i / d, k = i - u * d;
+    float x = 0.f;
+    int64_t uid;
+    if (has_row(u, uid)) x = rt_to_float(U[uid * d + k]);
+    Us[i] = x;
+  }
+}
+
 // acc[u] = Us[u] . vrow for the TU staged users, one fma chain each, k ascending (acc = 0 when vrow is null).
 template <typename T, int TU>
 __device__ __forceinline__ void rt_score(const T* __restrict__ vrow, const float* Us, int d, float (&acc)[TU]) {
@@ -121,36 +156,62 @@ __device__ __forceinline__ void rt_score(const T* __restrict__ vrow, const float
   }
 }
 
-// Append (s, item) to user u's candidate buffer if it beats the user's current K-th best.
-template <int TU>
-__device__ __forceinline__ void rt_offer(uint64_t* keys, int* cnt, const uint64_t* thr, int u, float s, uint32_t item) {
+struct RtKeepAll {
+  __device__ bool operator()() const { return true; }
+};
+
+// Append (s, item) to user u's candidate buffer if it beats the user's current K-th best and keep() (asked only then).
+template <int TU, typename Keep = RtKeepAll>
+__device__ __forceinline__ void rt_offer(uint64_t* keys, int* cnt, const uint64_t* thr, int u, float s, uint32_t item,
+                                         Keep keep = {}) {
   if (s == 0.f) s = 0.f;                       // -0 ranks like +0
   if (!(s > -INFINITY)) return;                // excluded (-inf) or NaN: never returned
   const uint64_t key = rt_key(s, item);
-  if (key > thr[u]) {
+  if (key > thr[u] && keep()) {
     const int p = atomicAdd(cnt + u, 1);
     keys[(size_t)u * (kRtEntries / TU) + p] = key;
   }
 }
 
-// The body of recommend_topk_kernel (kBias = false) and recommend_topk_bias_kernel (kBias: score + item_bias[item]).
+// Each user's K keys key_of(u, j) (zero: padding) to its batch row b (row_of(u, b); false: none): the split's per-split
+// list in partial, or decoded ids and scores when partial is null. Row: the type of b.
+template <int TU, typename Row, typename RowOf, typename KeyOf>
+__device__ __forceinline__ void rt_write_rows(int K, int split, int64_t B, uint64_t* partial, int64_t* out_ids,
+                                              float* out_scores, RowOf row_of, KeyOf key_of) {
+  for (int i = threadIdx.x; i < TU * K; i += kRtThreads) {
+    const int u = i / K, j = i - u * K;
+    Row b;
+    if (!row_of(u, b)) continue;
+    const uint64_t key = key_of(u, j);
+    if (partial) {
+      partial[((int64_t)split * B + b) * K + j] = key;
+    } else {
+      int64_t id; float s;
+      rt_decode(key, id, s);
+      out_ids[(int64_t)b * K + j] = id;
+      out_scores[(int64_t)b * K + j] = s;
+    }
+  }
+}
+
 template <typename T, int TU, bool kBias>
-__device__ __forceinline__ void
-recommend_topk_body(const T* __restrict__ U, int64_t nU, const T* __restrict__ V, int64_t nI, int d,
-                    const int64_t* __restrict__ uids, int64_t B, const int32_t* __restrict__ seen_ptr,
-                    const int32_t* __restrict__ seen_idx, int seen_by_row, float masked_score, int K, int64_t per_split,
-                    uint64_t* __restrict__ partial, int64_t* __restrict__ out_ids, float* __restrict__ out_scores,
-                    int32_t* err, const float* __restrict__ item_bias) {
+__global__ void __launch_bounds__(kRtThreads)
+recommend_topk_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ V, int64_t nI, int d,
+                      const int64_t* __restrict__ uids, int64_t B, const int32_t* __restrict__ seen_ptr,
+                      const int32_t* __restrict__ seen_idx, int seen_by_row, float masked_score, int K, int64_t per_split,
+                      uint64_t* __restrict__ partial, int64_t* __restrict__ out_ids, float* __restrict__ out_scores,
+                      int32_t* err, const float* __restrict__ item_bias) {
   constexpr int CAP = kRtEntries / TU;
   constexpr int kWords = kRtTile / 32;
   extern __shared__ __align__(16) uint64_t rt_smem[];
+  const RtSmem lay(TU, d);
   uint64_t* keys = rt_smem;                                    // [TU][CAP]
-  uint64_t* thr = keys + kRtEntries;                           // [TU]; ~0 = inactive row (no candidate beats it)
-  float* Us = reinterpret_cast<float*>(thr + TU);              // [TU][d]
-  uint32_t* bits = reinterpret_cast<uint32_t*>(Us + (size_t)TU * d);   // [TU][kWords]: seen items of the tile
-  int* cnt = reinterpret_cast<int*>(bits + TU * kWords);       // [TU]
-  int* mcur = cnt + TU;                                        // [TU]: next unconsumed entry of the seen list
-  int* mend = mcur + TU;                                       // [TU]
+  uint64_t* thr = rt_at<uint64_t>(rt_smem, lay.thr);           // [TU]; ~0 = inactive row (no candidate beats it)
+  float* Us = rt_at<float>(rt_smem, lay.Us);                   // [TU][d]
+  uint32_t* bits = rt_at<uint32_t>(rt_smem, lay.bits);         // [TU][kWords]: seen items of the tile
+  int* cnt = rt_at<int>(rt_smem, lay.cnt);                     // [TU]
+  int* mcur = rt_at<int>(rt_smem, lay.mcur);                   // [TU]: next unconsumed entry of the seen list
+  int* mend = rt_at<int>(rt_smem, lay.mend);                   // [TU]
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int64_t b0 = (int64_t)blockIdx.x * TU;
@@ -158,16 +219,12 @@ recommend_topk_body(const T* __restrict__ U, int64_t nU, const T* __restrict__ V
   const int64_t ib = (int64_t)split * per_split;
   const int64_t ie = min(nI, ib + per_split);
 
-  for (int i = tid; i < TU * d; i += kRtThreads) {
-    const int u = i / d, k = i - u * d;
+  rt_stage_users<T, TU>(Us, U, d, [&](int u, int64_t& uid) {
     const int64_t b = b0 + u;
-    float x = 0.f;
-    if (b < B) {
-      const int64_t uid = uids[b];
-      if (uid >= 0 && uid < nU) x = rt_to_float(U[uid * d + k]);
-    }
-    Us[i] = x;
-  }
+    if (b >= B) return false;
+    uid = uids[b];
+    return uid >= 0 && uid < nU;
+  });
   if (tid < TU) {
     const int64_t b = b0 + tid;
     bool active = false;
@@ -215,6 +272,7 @@ recommend_topk_body(const T* __restrict__ U, int64_t nU, const T* __restrict__ V
       }
     }
     // ---- scores of my item against every user of the tile: one fma chain each, k ascending ----
+    // (rt_score's chain, written out: calling rt_score here changes this kernel's register allocation and spills)
     const int64_t item = i0 + tid;
     const bool have = item < ie;
     float acc[TU];
@@ -245,13 +303,7 @@ recommend_topk_body(const T* __restrict__ U, int64_t nU, const T* __restrict__ V
         float s = acc[u];
         if constexpr (kBias) s += bias;
         if (seen_ptr && ((bits[u * kWords + warp] >> lane) & 1u)) s = masked_score;
-        if (s == 0.f) s = 0.f;                       // -0 ranks like +0
-        if (!(s > -INFINITY)) continue;              // excluded (-inf) or NaN: never returned
-        const uint64_t key = rt_key(s, (uint32_t)item);
-        if (key > thr[u]) {
-          const int p = atomicAdd(cnt + u, 1);
-          keys[(size_t)u * CAP + p] = key;
-        }
+        rt_offer<TU>(keys, cnt, thr, u, s, (uint32_t)item);
       }
     }
     __syncthreads();
@@ -262,42 +314,9 @@ recommend_topk_body(const T* __restrict__ U, int64_t nU, const T* __restrict__ V
   }
   rt_compact<TU>(keys, cnt, thr, K);
 
-  for (int i = tid; i < TU * K; i += kRtThreads) {
-    const int u = i / K, j = i - u * K;
-    const int64_t b = b0 + u;
-    if (b >= B) continue;
-    const uint64_t key = keys[(size_t)u * CAP + j];     // zero beyond the user's count: padding
-    if (partial) {
-      partial[((int64_t)split * B + b) * K + j] = key;
-    } else {
-      int64_t id; float s;
-      rt_decode(key, id, s);
-      out_ids[b * K + j] = id;
-      out_scores[b * K + j] = s;
-    }
-  }
-}
-
-template <typename T, int TU>
-__global__ void __launch_bounds__(kRtThreads)
-recommend_topk_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ V, int64_t nI, int d,
-                      const int64_t* __restrict__ uids, int64_t B, const int32_t* __restrict__ seen_ptr,
-                      const int32_t* __restrict__ seen_idx, int seen_by_row, float masked_score, int K, int64_t per_split,
-                      uint64_t* __restrict__ partial, int64_t* __restrict__ out_ids, float* __restrict__ out_scores,
-                      int32_t* err) {
-  recommend_topk_body<T, TU, false>(U, nU, V, nI, d, uids, B, seen_ptr, seen_idx, seen_by_row, masked_score, K, per_split,
-                                    partial, out_ids, out_scores, err, nullptr);
-}
-
-template <typename T, int TU>
-__global__ void __launch_bounds__(kRtThreads)
-recommend_topk_bias_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ V, int64_t nI, int d,
-                           const int64_t* __restrict__ uids, int64_t B, const int32_t* __restrict__ seen_ptr,
-                           const int32_t* __restrict__ seen_idx, int seen_by_row, float masked_score, int K,
-                           int64_t per_split, uint64_t* __restrict__ partial, int64_t* __restrict__ out_ids,
-                           float* __restrict__ out_scores, int32_t* err, const float* __restrict__ item_bias) {
-  recommend_topk_body<T, TU, true>(U, nU, V, nI, d, uids, B, seen_ptr, seen_idx, seen_by_row, masked_score, K, per_split,
-                                   partial, out_ids, out_scores, err, item_bias);
+  rt_write_rows<TU, int64_t>(
+      K, split, B, partial, out_ids, out_scores, [&](int u, int64_t& b) { b = b0 + u; return b < B; },
+      [&](int u, int j) { return keys[(size_t)u * CAP + j]; });   // zero beyond the user's count: padding
 }
 
 // Row b: the K best of the S per-split lists partial[s][b][0..K).
@@ -414,22 +433,39 @@ recommend_subset_plan_kernel(const int64_t* __restrict__ subset_ids, int B, int 
   }
 }
 
+// The plan's group g of scoring block blk (the last g with blocks_at[g] <= blk, ng groups) and the rows it takes,
+// order[r0, r0 + nr); false for a block past the plan's last.
+template <int TU>
+__device__ __forceinline__ bool rs_block_rows(const int32_t* blocks_at, const int32_t* rows_at, int ng, int blk, int& g,
+                                              int& r0, int& nr) {
+  if (blk >= blocks_at[ng]) return false;
+  int lo = 0, hi = ng;
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (blocks_at[mid] <= blk) lo = mid + 1; else hi = mid;
+  }
+  g = lo - 1;
+  r0 = rows_at[g] + (blk - blocks_at[g]) * TU;
+  nr = min(TU, rows_at[g + 1] - r0);
+  return true;
+}
+
 // Grid (upper bound on the plan's block count, S). Block x takes TU rows of one group and split y of the group's list:
 // a slice of at least kRtMinSplit ids (a multiple of the tile) so that groups shorter than the longest use fewer splits;
 // a split past the end of its list writes padding keys.
-// kBias: score + item_bias[item] (recommend_subset_bias_kernel).
 template <typename T, int TU, bool kBias>
-__device__ __forceinline__ void
-recommend_subset_body(const T* __restrict__ U, int64_t nU, const T* __restrict__ V, int64_t nI, int d,
-                      const int64_t* __restrict__ uids, int64_t B, const int32_t* __restrict__ sub_ptr,
-                      const int32_t* __restrict__ sub_idx, int G, const int32_t* __restrict__ rows_at,
-                      const int32_t* __restrict__ blocks_at, const int32_t* __restrict__ order,
-                      const int32_t* __restrict__ seen_ptr, const int32_t* __restrict__ seen_idx, int K, int S,
-                      uint64_t* __restrict__ partial, int64_t* __restrict__ out_ids, float* __restrict__ out_scores,
-                      int32_t* err, const float* __restrict__ item_bias) {
+__global__ void __launch_bounds__(kRtThreads, 2)   // 2 blocks an SM: up to 128 registers, no spills
+recommend_subset_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ V, int64_t nI, int d,
+                        const int64_t* __restrict__ uids, int64_t B, const int32_t* __restrict__ sub_ptr,
+                        const int32_t* __restrict__ sub_idx, int G, const int32_t* __restrict__ rows_at,
+                        const int32_t* __restrict__ blocks_at, const int32_t* __restrict__ order,
+                        const int32_t* __restrict__ seen_ptr, const int32_t* __restrict__ seen_idx, int K, int S,
+                        uint64_t* __restrict__ partial, int64_t* __restrict__ out_ids, float* __restrict__ out_scores,
+                        int32_t* err, const float* __restrict__ item_bias) {
   constexpr int CAP = kRtEntries / TU;
   constexpr int kWords = kRtTile / 32;
   extern __shared__ __align__(16) uint64_t rt_smem[];
+  // RsSmem's arrays, carved by pointer arithmetic: carving through its offsets changes this kernel's register allocation
   uint64_t* keys = rt_smem;                                    // [TU][CAP]
   uint64_t* thr = keys + kRtEntries;                           // [TU]; ~0 = inactive row (no candidate beats it)
   float* Us = reinterpret_cast<float*>(thr + TU);              // [TU][d]
@@ -442,15 +478,8 @@ recommend_subset_body(const T* __restrict__ U, int64_t nU, const T* __restrict__
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int blk = blockIdx.x, split = blockIdx.y;
-  if (blk >= blocks_at[G + 2]) return;
-  int lo = 0, hi = G + 2;                                      // group: the last g with blocks_at[g] <= blk
-  while (lo < hi) {
-    const int mid = (lo + hi) >> 1;
-    if (blocks_at[mid] <= blk) lo = mid + 1; else hi = mid;
-  }
-  const int g = lo - 1;
-  const int r0 = rows_at[g] + (blk - blocks_at[g]) * TU;
-  const int nr = min(TU, rows_at[g + 1] - r0);
+  int g, r0, nr;
+  if (!rs_block_rows<TU>(blocks_at, rows_at, G + 2, blk, g, r0, nr)) return;
   const int32_t* list = g < G ? sub_idx + sub_ptr[g] : nullptr;   // null: the identity (whole catalog)
   const int64_t len = g < G ? sub_ptr[g + 1] - sub_ptr[g] : g == G ? nI : 0;
   int64_t per = max((len + S - 1) / S, (int64_t)kRtMinSplit);
@@ -484,12 +513,11 @@ recommend_subset_body(const T* __restrict__ U, int64_t nU, const T* __restrict__
   }
   __syncthreads();
   if (pb < pe) {
-    for (int i = tid; i < TU * d; i += kRtThreads) {
-      const int u = i / d, k = i - u * d;
-      float x = 0.f;
-      if (thr[u] == 0ull) x = rt_to_float(U[uids[rowb[u]] * d + k]);
-      Us[i] = x;
-    }
+    rt_stage_users<T, TU>(Us, U, d, [&](int u, int64_t& uid) {
+      if (thr[u] != 0ull) return false;
+      uid = uids[rowb[u]];
+      return true;
+    });
     for (int64_t p0 = pb; p0 < pe; p0 += kRtTile) {
       const int n = (int)min((int64_t)kRtTile, pe - p0);
       for (int i = tid; i < TU * kWords; i += kRtThreads) bits[i] = 0;
@@ -557,32 +585,6 @@ recommend_subset_body(const T* __restrict__ U, int64_t nU, const T* __restrict__
       out_scores[(int64_t)b * K + j] = s;
     }
   }
-}
-
-template <typename T, int TU>
-__global__ void __launch_bounds__(kRtThreads, 2)   // 2 blocks an SM: up to 128 registers, no spills
-recommend_subset_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ V, int64_t nI, int d,
-                        const int64_t* __restrict__ uids, int64_t B, const int32_t* __restrict__ sub_ptr,
-                        const int32_t* __restrict__ sub_idx, int G, const int32_t* __restrict__ rows_at,
-                        const int32_t* __restrict__ blocks_at, const int32_t* __restrict__ order,
-                        const int32_t* __restrict__ seen_ptr, const int32_t* __restrict__ seen_idx, int K, int S,
-                        uint64_t* __restrict__ partial, int64_t* __restrict__ out_ids, float* __restrict__ out_scores,
-                        int32_t* err) {
-  recommend_subset_body<T, TU, false>(U, nU, V, nI, d, uids, B, sub_ptr, sub_idx, G, rows_at, blocks_at, order, seen_ptr,
-                                      seen_idx, K, S, partial, out_ids, out_scores, err, nullptr);
-}
-
-template <typename T, int TU>
-__global__ void __launch_bounds__(kRtThreads, 2)
-recommend_subset_bias_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ V, int64_t nI, int d,
-                             const int64_t* __restrict__ uids, int64_t B, const int32_t* __restrict__ sub_ptr,
-                             const int32_t* __restrict__ sub_idx, int G, const int32_t* __restrict__ rows_at,
-                             const int32_t* __restrict__ blocks_at, const int32_t* __restrict__ order,
-                             const int32_t* __restrict__ seen_ptr, const int32_t* __restrict__ seen_idx, int K, int S,
-                             uint64_t* __restrict__ partial, int64_t* __restrict__ out_ids,
-                             float* __restrict__ out_scores, int32_t* err, const float* __restrict__ item_bias) {
-  recommend_subset_body<T, TU, true>(U, nU, V, nI, d, uids, B, sub_ptr, sub_idx, G, rows_at, blocks_at, order, seen_ptr,
-                                     seen_idx, K, S, partial, out_ids, out_scores, err, item_bias);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -687,13 +689,21 @@ __device__ __forceinline__ bool geo_listed(const int32_t* __restrict__ idx, int 
   return lo < end && idx[lo] == item;
 }
 
+struct GeoSmem {   // recommend_geo_kernel; keys [TU][kRtEntries / TU] at 0
+  size_t thr, cq, Us, cnt, sb, se, rowb, pass, wv, seg, pref, misc, bytes;
+  __host__ __device__ GeoSmem(int TU, int d)
+      : thr((size_t)kRtEntries * 8), cq(thr + (size_t)TU * 8), Us(cq + (size_t)TU * 4 * 8), cnt(Us + (size_t)TU * d * 4),
+        sb(cnt + (size_t)TU * 4), se(sb + (size_t)TU * 4), rowb(se + (size_t)TU * 4), pass(rowb + (size_t)TU * 4),
+        wv(pass + (size_t)TU * 4), seg(wv + 8 * 4), pref(seg + (size_t)kGeoMaxSegs * 4),
+        misc(pref + (size_t)(kGeoMaxSegs + 1) * 4), bytes(misc + 16 * 4) {}
+};
+
 // Grid (upper bound on the plan's block count, S), as recommend_subset_kernel: block x takes up to TU rows of one hash
 // bucket (group H: rows with a non-finite centre or threshold, all padding), split y of each window. Rows of a bucket
 // normally share one window; on a hash collision the block streams each distinct window of its rows in turn, and a row
 // takes offers only during its own window. Window items come in cell order, not id order, so instead of the ascending
 // seen cursor of the subset kernel a candidate that beats the row's current K-th best is looked up in the row's seen
 // list (a binary search) before it enters the buffer: few items get that far once the thresholds settle.
-// kBias: score + item_bias[item].
 template <typename T, int TU, bool kBias>
 __global__ void __launch_bounds__(kRtThreads, 2)   // 2 blocks an SM: up to 128 registers, no spills
 recommend_geo_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ V, int d, const int64_t* __restrict__ uids,
@@ -707,31 +717,25 @@ recommend_geo_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ 
                      const float* __restrict__ item_bias) {
   constexpr int CAP = kRtEntries / TU;
   extern __shared__ __align__(16) uint64_t rt_smem[];
+  const GeoSmem lay(TU, d);
   uint64_t* keys = rt_smem;                                    // [TU][CAP]
-  uint64_t* thr = keys + kRtEntries;                           // [TU]; ~0 = inactive row (no candidate beats it)
-  double* cq = reinterpret_cast<double*>(thr + TU);            // [TU][4]: c_x, c_y, c_z, t of each row
-  float* Us = reinterpret_cast<float*>(cq + 4 * TU);           // [TU][d]
-  int* cnt = reinterpret_cast<int*>(Us + (size_t)TU * d);      // [TU]
-  int* sb = cnt + TU;                                          // [TU]: the row's seen list, seen_idx[sb, se)
-  int* se = sb + TU;                                           // [TU]
-  int* rowb = se + TU;                                         // [TU]: batch row of each user, -1 = none
-  int* pass = rowb + TU;                                       // [TU]: 0 to stream, 1 in the current window, 2 done
-  int* wv = pass + TU;                                         // [8]: the current window
-  int* seg = wv + 8;                                           // [kGeoMaxSegs]: first cell_items position of each run
-  int* pref = seg + kGeoMaxSegs;                               // [kGeoMaxSegs + 1]: window position of each run
-  int* misc = pref + kGeoMaxSegs + 1;                          // [16]: leader row, warp sums of the scan
+  uint64_t* thr = rt_at<uint64_t>(rt_smem, lay.thr);           // [TU]; ~0 = inactive row (no candidate beats it)
+  double* cq = rt_at<double>(rt_smem, lay.cq);                 // [TU][4]: c_x, c_y, c_z, t of each row
+  float* Us = rt_at<float>(rt_smem, lay.Us);                   // [TU][d]
+  int* cnt = rt_at<int>(rt_smem, lay.cnt);                     // [TU]
+  int* sb = rt_at<int>(rt_smem, lay.sb);                       // [TU]: the row's seen list, seen_idx[sb, se)
+  int* se = rt_at<int>(rt_smem, lay.se);                       // [TU]
+  int* rowb = rt_at<int>(rt_smem, lay.rowb);                   // [TU]: batch row of each user, -1 = none
+  int* pass = rt_at<int>(rt_smem, lay.pass);                   // [TU]: 0 to stream, 1 in the current window, 2 done
+  int* wv = rt_at<int>(rt_smem, lay.wv);                       // [8]: the current window
+  int* seg = rt_at<int>(rt_smem, lay.seg);                     // [kGeoMaxSegs]: first cell_items position of each run
+  int* pref = rt_at<int>(rt_smem, lay.pref);                   // [kGeoMaxSegs + 1]: window position of each run
+  int* misc = rt_at<int>(rt_smem, lay.misc);                   // [16]: leader row, warp sums of the scan
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int blk = blockIdx.x, split = blockIdx.y;
-  if (blk >= blocks_at[H + 2]) return;
-  int lo = 0, hi = H + 2;                                      // group: the last g with blocks_at[g] <= blk
-  while (lo < hi) {
-    const int mid = (lo + hi) >> 1;
-    if (blocks_at[mid] <= blk) lo = mid + 1; else hi = mid;
-  }
-  const int g = lo - 1;
-  const int r0 = rows_at[g] + (blk - blocks_at[g]) * TU;
-  const int nr = min(TU, rows_at[g + 1] - r0);
+  int g, r0, nr;
+  if (!rs_block_rows<TU>(blocks_at, rows_at, H + 2, blk, g, r0, nr)) return;
 
   if (tid < TU) {
     const int b = tid < nr ? order[r0 + tid] : -1;
@@ -754,12 +758,11 @@ recommend_geo_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ 
     pass[tid] = active ? 0 : 2;
   }
   __syncthreads();
-  for (int i = tid; i < TU * d; i += kRtThreads) {
-    const int u = i / d, k = i - u * d;
-    float x = 0.f;
-    if (thr[u] == 0ull) x = rt_to_float(U[uids[rowb[u]] * d + k]);
-    Us[i] = x;
-  }
+  rt_stage_users<T, TU>(Us, U, d, [&](int u, int64_t& uid) {
+    if (thr[u] != 0ull) return false;
+    uid = uids[rowb[u]];
+    return true;
+  });
 
   for (;;) {
     if (tid == 0) {
@@ -845,14 +848,8 @@ recommend_geo_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ 
 #pragma unroll
         for (int u = 0; u < TU; ++u) {
           if (!((in >> u) & 1u)) continue;
-          float s = kBias ? acc[u] + bias : acc[u];
-          if (s == 0.f) s = 0.f;                   // -0 ranks like +0
-          if (!(s > -INFINITY)) continue;          // -inf or NaN: never returned
-          const uint64_t key = rt_key(s, (uint32_t)item);
-          if (key <= thr[u]) continue;
-          if (seen_ptr && geo_listed(seen_idx, sb[u], se[u], item)) continue;
-          const int q = atomicAdd(cnt + u, 1);
-          keys[(size_t)u * CAP + q] = key;
+          rt_offer<TU>(keys, cnt, thr, u, kBias ? acc[u] + bias : acc[u], (uint32_t)item,
+                       [&] { return !(seen_ptr && geo_listed(seen_idx, sb[u], se[u], item)); });
         }
       }
       __syncthreads();
@@ -866,20 +863,9 @@ recommend_geo_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ 
   }
 
   // every buffer that took an offer was truncated after its window's last tile: its first cnt keys are its K best
-  for (int i = tid; i < TU * K; i += kRtThreads) {
-    const int u = i / K, j = i - u * K;
-    const int b = rowb[u];
-    if (b < 0) continue;
-    const uint64_t key = j < cnt[u] ? keys[(size_t)u * CAP + j] : 0;   // zero beyond the user's count: padding
-    if (partial) {
-      partial[((int64_t)split * B + b) * K + j] = key;
-    } else {
-      int64_t id; float s;
-      rt_decode(key, id, s);
-      out_ids[(int64_t)b * K + j] = id;
-      out_scores[(int64_t)b * K + j] = s;
-    }
-  }
+  rt_write_rows<TU, int>(
+      K, split, B, partial, out_ids, out_scores, [&](int u, int& b) { b = rowb[u]; return b >= 0; },
+      [&](int u, int j) { return j < cnt[u] ? keys[(size_t)u * CAP + j] : 0; });   // zero beyond the count: padding
 }
 
 }  // namespace yr
@@ -919,81 +905,23 @@ int rt_splits(int64_t B, int64_t nI, int K, int TU, int sm, int64_t* per_split) 
   return (int)((nI + per - 1) / per);
 }
 
-size_t rt_smem_bytes(int TU, int d) {
-  return (size_t)kRtEntries * 8 + (size_t)TU * 8 + (size_t)TU * d * 4 + (size_t)TU * (kRtTile / 32) * 4 + 3 * (size_t)TU * 4;
-}
-
-template <typename T, int TU, bool kBias>
-int rt_launch(const void* U, int64_t nU, const void* V, int64_t nI, int d, const int64_t* uids, int64_t B,
-              const int32_t* seen_ptr, const int32_t* seen_idx, int seen_by_row, float masked_score, int K, int S,
-              int64_t per_split, uint64_t* partial, int64_t* out_ids, float* out_scores, int32_t* err,
-              const float* item_bias, cudaStream_t s) {
-  static AttrOnce attr;
-  const size_t smem = rt_smem_bytes(TU, d);
-  const int max_smem = (int)rt_smem_bytes(TU, rt_max_d(TU));
-  dim3 grid((unsigned)((B + TU - 1) / TU), (unsigned)S);
-  const T* Ut = reinterpret_cast<const T*>(U);
-  const T* Vt = reinterpret_cast<const T*>(V);
-  if constexpr (kBias) {
-    int rc = attr.set(recommend_topk_bias_kernel<T, TU>, max_smem);
-    if (rc) return rc;
-    recommend_topk_bias_kernel<T, TU><<<grid, kRtThreads, smem, s>>>(Ut, nU, Vt, nI, d, uids, B, seen_ptr, seen_idx,
-                                                                     seen_by_row, masked_score, K, per_split, partial,
-                                                                     out_ids, out_scores, err, item_bias);
-  } else {
-    int rc = attr.set(recommend_topk_kernel<T, TU>, max_smem);
-    if (rc) return rc;
-    recommend_topk_kernel<T, TU><<<grid, kRtThreads, smem, s>>>(Ut, nU, Vt, nI, d, uids, B, seen_ptr, seen_idx,
-                                                                seen_by_row, masked_score, K, per_split, partial, out_ids,
-                                                                out_scores, err);
-  }
-  YR_CHECK_LAUNCH();
-  return YR_OK;
-}
-
-size_t rs_smem_bytes(int TU, int d) { return rt_smem_bytes(TU, d) + (size_t)TU * 4 + (size_t)kRtTile * 4; }
-
-template <typename T, int TU, bool kBias>
-int rs_launch(const void* U, int64_t nU, const void* V, int64_t nI, int d, const int64_t* uids, int64_t B,
-              const int32_t* sub_ptr, const int32_t* sub_idx, int G, const int32_t* rows_at, const int32_t* blocks_at,
-              const int32_t* order, const int32_t* seen_ptr, const int32_t* seen_idx, int K, int S, uint64_t* partial,
-              int64_t* out_ids, float* out_scores, int32_t* err, const float* item_bias, cudaStream_t s) {
-  static AttrOnce attr;
-  const int max_smem = (int)rs_smem_bytes(TU, rt_max_d(TU));
-  // the plan makes sum over groups of ceil(rows / TU) blocks: at most ceil(B / TU) + one per non-empty group
-  dim3 grid((unsigned)((B + TU - 1) / TU + std::min<int64_t>((int64_t)G + 2, B)), (unsigned)S);
-  const size_t smem = rs_smem_bytes(TU, d);
-  const T* Ut = reinterpret_cast<const T*>(U);
-  const T* Vt = reinterpret_cast<const T*>(V);
-  if constexpr (kBias) {
-    int rc = attr.set(recommend_subset_bias_kernel<T, TU>, max_smem);
-    if (rc) return rc;
-    recommend_subset_bias_kernel<T, TU><<<grid, kRtThreads, smem, s>>>(Ut, nU, Vt, nI, d, uids, B, sub_ptr, sub_idx, G,
-                                                                       rows_at, blocks_at, order, seen_ptr, seen_idx, K,
-                                                                       S, partial, out_ids, out_scores, err, item_bias);
-  } else {
-    int rc = attr.set(recommend_subset_kernel<T, TU>, max_smem);
-    if (rc) return rc;
-    recommend_subset_kernel<T, TU><<<grid, kRtThreads, smem, s>>>(Ut, nU, Vt, nI, d, uids, B, sub_ptr, sub_idx, G,
-                                                                  rows_at, blocks_at, order, seen_ptr, seen_idx, K, S,
-                                                                  partial, out_ids, out_scores, err);
-  }
-  YR_CHECK_LAUNCH();
-  return YR_OK;
-}
-
-int rs_splits(int64_t B, int64_t max_len, int K, int TU) {
-  int64_t per = 0;
-  return rt_splits(B, std::max<int64_t>(max_len, 1), K, TU, yr_sm_count(), &per);
-}
-
 size_t rs_partial_bytes(int S, int64_t B, int K) { return S > 1 ? (size_t)S * (size_t)B * (size_t)K * sizeof(uint64_t) : 0; }
 
 size_t rs_plan_bytes(int64_t B, int G) { return ((size_t)3 * G + 8 + (size_t)B) * sizeof(int32_t); }
 
-size_t geo_smem_bytes(int TU, int d) {
-  return (size_t)kRtEntries * 8 + (size_t)TU * 8 + (size_t)TU * 4 * 8 + (size_t)TU * d * 4 + 5 * (size_t)TU * 4 +
-         (size_t)(8 + 2 * kGeoMaxSegs + 1 + 16) * 4;
+// The row plan of recommend_subset_plan_kernel for B rows in G groups, carved from rs_plan_bytes(B, G) bytes at p.
+struct RsPlan {
+  int32_t* cursor;      // [G + 2]
+  int32_t* rows_at;     // [G + 3]
+  int32_t* blocks_at;   // [G + 3]
+  int32_t* order;       // [B]
+  RsPlan(void* p, int G)
+      : cursor(static_cast<int32_t*>(p)), rows_at(cursor + G + 2), blocks_at(rows_at + G + 3), order(blocks_at + G + 3) {}
+};
+
+int rs_splits(int64_t B, int64_t max_len, int K, int TU) {
+  int64_t per = 0;
+  return rt_splits(B, std::max<int64_t>(max_len, 1), K, TU, yr_sm_count(), &per);
 }
 
 // Hash buckets of the row grouping: about two per row (few collisions), at most 2^16 (the plan scans them all).
@@ -1008,33 +936,61 @@ size_t geo_ws_bytes(int S, int64_t B, int K) {
   return rs_partial_bytes(S, B, K) + (size_t)B * 8 + rs_plan_bytes(B, geo_buckets(B)) + (size_t)B * kGeoWin * 4;
 }
 
-template <typename T, int TU, bool kBias>
-int geo_launch(const void* U, int64_t nU, const void* V, int d, const int64_t* uids, int64_t B, const int64_t* cell_keys,
-               const int32_t* cell_ptr, int64_t nC, const int32_t* cell_items, const double* P, int nlon, const double* c,
-               const double* t, const int32_t* win, int H, const int32_t* rows_at, const int32_t* blocks_at,
-               const int32_t* order, const int32_t* seen_ptr, const int32_t* seen_idx, int K, int S, uint64_t* partial,
-               int64_t* out_ids, float* out_scores, int32_t* err, const float* item_bias, cudaStream_t s) {
+// kernel<<<grid, kRtThreads, bytes, s>>>(args...), its dynamic shared memory limit raised to max_bytes first (once per
+// device: one AttrOnce per kernel instance).
+template <auto kernel, typename... A>
+int rt_launch(dim3 grid, size_t bytes, size_t max_bytes, cudaStream_t s, A... args) {
   static AttrOnce attr;
-  int rc = attr.set(recommend_geo_kernel<T, TU, kBias>, (int)geo_smem_bytes(TU, rt_max_d(TU)));
+  int rc = attr.set(kernel, (int)max_bytes);
   if (rc) return rc;
-  dim3 grid((unsigned)((B + TU - 1) / TU + std::min<int64_t>((int64_t)H + 2, B)), (unsigned)S);
-  recommend_geo_kernel<T, TU, kBias><<<grid, kRtThreads, geo_smem_bytes(TU, d), s>>>(
-      reinterpret_cast<const T*>(U), nU, reinterpret_cast<const T*>(V), d, uids, B, cell_keys, cell_ptr, nC, cell_items,
-      P, nlon, c, t, win, H, rows_at, blocks_at, order, seen_ptr, seen_idx, K, S, partial, out_ids, out_scores, err,
-      item_bias);
+  kernel<<<grid, kRtThreads, bytes, s>>>(args...);
   YR_CHECK_LAUNCH();
+  return YR_OK;
+}
+
+// Shared memory of a scoring launch with TU users per block, d wide (bytes), and at the widest d it can have (max).
+template <typename Layout>
+struct RtBytes {
+  size_t bytes, max;
+  RtBytes(int TU, int d) : bytes(Layout(TU, d).bytes), max(Layout(TU, rt_max_d(TU)).bytes) {}
+};
+
+// The scoring kernel instance of a launch: table type, users per block, bias.
+template <typename T_, int TU_, bool kBias_>
+struct RtInst {
+  using T = T_;
+  static constexpr int TU = TU_;
+  static constexpr bool kBias = kBias_;
+};
+
+template <typename T, bool kBias, typename F>
+int rt_dispatch_tu(int TU, F& f) {
+  return TU == 16 ? f(RtInst<T, 16, kBias>()) : TU == 8 ? f(RtInst<T, 8, kBias>()) : f(RtInst<T, 4, kBias>());
+}
+
+// f(RtInst<T, TU, kBias>()) for the runtime table dtype, users per block (16, 8 or 4) and bias of a launch.
+template <typename F>
+int rt_dispatch(int dtype, int TU, bool bias, F f) {
+  if (dtype == YR_DTYPE_F32) return bias ? rt_dispatch_tu<float, true>(TU, f) : rt_dispatch_tu<float, false>(TU, f);
+  return bias ? rt_dispatch_tu<__nv_bfloat16, true>(TU, f) : rt_dispatch_tu<__nv_bfloat16, false>(TU, f);
+}
+
+// The arguments every retrieval entry takes: YR_ERR_BAD_ARG for missing pointers, an unpaired seen list, B < 0, an
+// empty user table or K outside [1, kRtMaxK]; then YR_ERR_BAD_DIM for the catalog size or width; then the dtype.
+int rt_check(const void* U, int64_t nU, const void* V, int64_t nI, int d, int dtype, const int64_t* user_ids, int64_t B,
+             const int32_t* seen_ptr, const int32_t* seen_idx, int K, const int64_t* out_ids, const float* out_scores) {
+  if (!U || !V || !out_ids || !out_scores || (B > 0 && !user_ids)) return YR_ERR_BAD_ARG;
+  if ((seen_ptr == nullptr) != (seen_idx == nullptr)) return YR_ERR_BAD_ARG;
+  if (B < 0 || nU <= 0 || K <= 0 || K > kRtMaxK) return YR_ERR_BAD_ARG;
+  if (nI <= 0 || nI >= 0x7fffffffLL || d <= 0 || d > kRtMaxD || (d & 7) != 0) return YR_ERR_BAD_DIM;
+  if (dtype != YR_DTYPE_F32 && dtype != YR_DTYPE_BF16) return YR_ERR_BAD_ARG;
   return YR_OK;
 }
 
 int merge_launch(const uint64_t* partial, int S, int64_t B, int K, int64_t* out_ids, float* out_scores, cudaStream_t s) {
   const int P = rt_pow2(S * K);
-  static AttrOnce attr;
-  int rc = attr.set(recommend_merge_kernel, kRtMergeMax * (int)sizeof(uint64_t));
-  if (rc) return rc;
-  recommend_merge_kernel<<<(unsigned)B, kRtThreads, (size_t)P * sizeof(uint64_t), s>>>(partial, S, B, K, P, out_ids,
-                                                                                     out_scores);
-  YR_CHECK_LAUNCH();
-  return YR_OK;
+  return rt_launch<recommend_merge_kernel>((unsigned)B, (size_t)P * sizeof(uint64_t), kRtMergeMax * sizeof(uint64_t), s,
+                                           partial, S, B, K, P, out_ids, out_scores);
 }
 
 }  // namespace
@@ -1058,11 +1014,7 @@ extern "C" int yr_recommend_topk_ex(const void* U, int64_t nU, const void* V, in
                                     const int64_t* user_ids, int64_t B, const int32_t* seen_ptr, const int32_t* seen_idx,
                                     int seen_by_row, float masked_score, int K, int64_t* out_ids, float* out_scores,
                                     void* ws, size_t ws_bytes, int32_t* err, yr_stream stream, const float* item_bias) {
-  if (!U || !V || !out_ids || !out_scores || (B > 0 && !user_ids)) return YR_ERR_BAD_ARG;
-  if ((seen_ptr == nullptr) != (seen_idx == nullptr)) return YR_ERR_BAD_ARG;
-  if (B < 0 || nU <= 0 || K <= 0 || K > kRtMaxK) return YR_ERR_BAD_ARG;
-  if (nI <= 0 || nI >= 0x7fffffffLL || d <= 0 || d > kRtMaxD || (d & 7) != 0) return YR_ERR_BAD_DIM;
-  if (dtype != YR_DTYPE_F32 && dtype != YR_DTYPE_BF16) return YR_ERR_BAD_ARG;
+  if (int rc = rt_check(U, nU, V, nI, d, dtype, user_ids, B, seen_ptr, seen_idx, K, out_ids, out_scores)) return rc;
   if (B == 0) return YR_OK;
   cudaStream_t s = (cudaStream_t)stream;
   const int TU = rt_users(K, d);
@@ -1073,18 +1025,16 @@ extern "C" int yr_recommend_topk_ex(const void* U, int64_t nU, const void* V, in
     if (!ws || ws_bytes < rs_partial_bytes(S, B, K)) return YR_ERR_WORKSPACE;
     partial = reinterpret_cast<uint64_t*>(ws);
   }
-  int rc;
-#define YR_RT_LAUNCH(T, TU_, BIAS)                                                                                        \
-  rt_launch<T, TU_, BIAS>(U, nU, V, nI, d, user_ids, B, seen_ptr, seen_idx, seen_by_row, masked_score, K, S, per,        \
-                          partial, out_ids, out_scores, err, item_bias, s)
-#define YR_RT_TU(T, BIAS)                                                                                                 \
-  (TU == 16 ? YR_RT_LAUNCH(T, 16, BIAS) : TU == 8 ? YR_RT_LAUNCH(T, 8, BIAS) : YR_RT_LAUNCH(T, 4, BIAS))
-  if (dtype == YR_DTYPE_F32)
-    rc = item_bias ? YR_RT_TU(float, true) : YR_RT_TU(float, false);
-  else
-    rc = item_bias ? YR_RT_TU(__nv_bfloat16, true) : YR_RT_TU(__nv_bfloat16, false);
-#undef YR_RT_TU
-#undef YR_RT_LAUNCH
+  const dim3 grid((unsigned)((B + TU - 1) / TU), (unsigned)S);
+  const RtBytes<RtSmem> smem(TU, d);
+  const int rc = rt_dispatch(dtype, TU, item_bias != nullptr, [&](auto inst) {
+    using I = decltype(inst);
+    using T = typename I::T;
+    return rt_launch<recommend_topk_kernel<T, I::TU, I::kBias>>(
+        grid, smem.bytes, smem.max, s, reinterpret_cast<const T*>(U), nU, reinterpret_cast<const T*>(V), nI, d,
+        user_ids, B, seen_ptr, seen_idx, seen_by_row, masked_score, K, per, partial, out_ids, out_scores, err,
+        item_bias);
+  });
   if (rc || S == 1) return rc;
   return merge_launch(partial, S, B, K, out_ids, out_scores, s);
 }
@@ -1111,14 +1061,9 @@ extern "C" int yr_recommend_subset_topk_ex(const void* U, int64_t nU, const void
                                            const int64_t* subset_ids, const int32_t* seen_ptr, const int32_t* seen_idx,
                                            int K, int64_t* out_ids, float* out_scores, void* ws, size_t ws_bytes,
                                            int32_t* err, yr_stream stream, const float* item_bias) {
-  if (!U || !V || !out_ids || !out_scores || !subset_ptr || !subset_idx) return YR_ERR_BAD_ARG;
-  if (B > 0 && (!user_ids || !subset_ids)) return YR_ERR_BAD_ARG;
-  if ((seen_ptr == nullptr) != (seen_idx == nullptr)) return YR_ERR_BAD_ARG;
-  if (B < 0 || B >= 0x7fffffffLL || G < 0 || G >= 0x7ffffff0 || max_subset_len < 0 || nU <= 0 || K <= 0 ||
-      K > kRtMaxK)
-    return YR_ERR_BAD_ARG;
-  if (nI <= 0 || nI >= 0x7fffffffLL || d <= 0 || d > kRtMaxD || (d & 7) != 0) return YR_ERR_BAD_DIM;
-  if (dtype != YR_DTYPE_F32 && dtype != YR_DTYPE_BF16) return YR_ERR_BAD_ARG;
+  if (!subset_ptr || !subset_idx || (B > 0 && !subset_ids)) return YR_ERR_BAD_ARG;
+  if (B >= 0x7fffffffLL || G < 0 || G >= 0x7ffffff0 || max_subset_len < 0) return YR_ERR_BAD_ARG;
+  if (int rc = rt_check(U, nU, V, nI, d, dtype, user_ids, B, seen_ptr, seen_idx, K, out_ids, out_scores)) return rc;
   if (B == 0) return YR_OK;
   const int TU = rt_users(K, d);
   const int S = rs_splits(B, max_subset_len, K, TU);
@@ -1126,25 +1071,21 @@ extern "C" int yr_recommend_subset_topk_ex(const void* U, int64_t nU, const void
   if (!ws || ws_bytes < pbytes + rs_plan_bytes(B, G)) return YR_ERR_WORKSPACE;
   cudaStream_t s = (cudaStream_t)stream;
   uint64_t* partial = S > 1 ? reinterpret_cast<uint64_t*>(ws) : nullptr;
-  int32_t* cursor = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(ws) + pbytes);   // [G + 2]
-  int32_t* rows_at = cursor + G + 2;                                                      // [G + 3]
-  int32_t* blocks_at = rows_at + G + 3;                                                   // [G + 3]
-  int32_t* order = blocks_at + G + 3;                                                     // [B]
-  recommend_subset_plan_kernel<<<1, kRsPlanThreads, 0, s>>>(subset_ids, (int)B, G, TU, cursor, rows_at, blocks_at, order,
-                                                            err);
+  const RsPlan plan(reinterpret_cast<char*>(ws) + pbytes, G);
+  recommend_subset_plan_kernel<<<1, kRsPlanThreads, 0, s>>>(subset_ids, (int)B, G, TU, plan.cursor, plan.rows_at,
+                                                            plan.blocks_at, plan.order, err);
   YR_CHECK_LAUNCH();
-  int rc;
-#define YR_RS_LAUNCH(T, TU_, BIAS)                                                                                        \
-  rs_launch<T, TU_, BIAS>(U, nU, V, nI, d, user_ids, B, subset_ptr, subset_idx, G, rows_at, blocks_at, order, seen_ptr,  \
-                          seen_idx, K, S, partial, out_ids, out_scores, err, item_bias, s)
-#define YR_RS_TU(T, BIAS)                                                                                                 \
-  (TU == 16 ? YR_RS_LAUNCH(T, 16, BIAS) : TU == 8 ? YR_RS_LAUNCH(T, 8, BIAS) : YR_RS_LAUNCH(T, 4, BIAS))
-  if (dtype == YR_DTYPE_F32)
-    rc = item_bias ? YR_RS_TU(float, true) : YR_RS_TU(float, false);
-  else
-    rc = item_bias ? YR_RS_TU(__nv_bfloat16, true) : YR_RS_TU(__nv_bfloat16, false);
-#undef YR_RS_TU
-#undef YR_RS_LAUNCH
+  // the plan makes sum over groups of ceil(rows / TU) blocks: at most ceil(B / TU) + one per non-empty group
+  const dim3 grid((unsigned)((B + TU - 1) / TU + std::min<int64_t>((int64_t)G + 2, B)), (unsigned)S);
+  const RtBytes<RsSmem> smem(TU, d);
+  const int rc = rt_dispatch(dtype, TU, item_bias != nullptr, [&](auto inst) {
+    using I = decltype(inst);
+    using T = typename I::T;
+    return rt_launch<recommend_subset_kernel<T, I::TU, I::kBias>>(
+        grid, smem.bytes, smem.max, s, reinterpret_cast<const T*>(U), nU, reinterpret_cast<const T*>(V), nI, d,
+        user_ids, B, subset_ptr, subset_idx, G, plan.rows_at, plan.blocks_at, plan.order, seen_ptr, seen_idx, K, S,
+        partial, out_ids, out_scores, err, item_bias);
+  });
   if (rc || S == 1) return rc;
   return merge_launch(partial, S, B, K, out_ids, out_scores, s);
 }
@@ -1161,15 +1102,12 @@ extern "C" int yr_recommend_geo_topk(const void* U, int64_t nU, const void* V, i
                                      const double* centre_xyz, const double* threshold, const int32_t* seen_ptr,
                                      const int32_t* seen_idx, int K, int64_t* out_ids, float* out_scores, void* ws,
                                      size_t ws_bytes, int32_t* err, yr_stream stream, const float* item_bias) {
-  if (!U || !V || !out_ids || !out_scores || !cell_keys || !cell_ptr || !cell_items || !item_xyz) return YR_ERR_BAD_ARG;
-  if (B > 0 && (!user_ids || !centre_xyz || !threshold)) return YR_ERR_BAD_ARG;
-  if ((seen_ptr == nullptr) != (seen_idx == nullptr)) return YR_ERR_BAD_ARG;
-  if (B < 0 || B >= 0x7fffffffLL || nU <= 0 || K <= 0 || K > kRtMaxK) return YR_ERR_BAD_ARG;
-  if (!(cell_deg > 0.0) || !(cell_deg <= 360.0) || num_lat < 1 || num_lon < 1 || num_lat > 0x7fffffffLL ||
-      num_lon > 0x7fffffffLL || num_cells < 0 || num_cells > nI)
+  if (!cell_keys || !cell_ptr || !cell_items || !item_xyz || (B > 0 && (!centre_xyz || !threshold)))
     return YR_ERR_BAD_ARG;
-  if (nI <= 0 || nI >= 0x7fffffffLL || d <= 0 || d > kRtMaxD || (d & 7) != 0) return YR_ERR_BAD_DIM;
-  if (dtype != YR_DTYPE_F32 && dtype != YR_DTYPE_BF16) return YR_ERR_BAD_ARG;
+  if (B >= 0x7fffffffLL || !(cell_deg > 0.0) || !(cell_deg <= 360.0) || num_lat < 1 || num_lon < 1 ||
+      num_lat > 0x7fffffffLL || num_lon > 0x7fffffffLL || num_cells < 0 || num_cells > nI)
+    return YR_ERR_BAD_ARG;
+  if (int rc = rt_check(U, nU, V, nI, d, dtype, user_ids, B, seen_ptr, seen_idx, K, out_ids, out_scores)) return rc;
   if (B == 0) return YR_OK;
   const int TU = rt_users(K, d);
   const int S = rs_splits(B, nI, K, TU);
@@ -1179,30 +1117,25 @@ extern "C" int yr_recommend_geo_topk(const void* U, int64_t nU, const void* V, i
   const size_t pbytes = rs_partial_bytes(S, B, K);
   uint64_t* partial = S > 1 ? reinterpret_cast<uint64_t*>(ws) : nullptr;
   int64_t* bucket = reinterpret_cast<int64_t*>(reinterpret_cast<char*>(ws) + pbytes);   // [B]
-  int32_t* cursor = reinterpret_cast<int32_t*>(bucket + B);                              // [H + 2]
-  int32_t* rows_at = cursor + H + 2;                                                      // [H + 3]
-  int32_t* blocks_at = rows_at + H + 3;                                                   // [H + 3]
-  int32_t* order = blocks_at + H + 3;                                                     // [B]
-  int32_t* win = order + B;                                                               // [B][kGeoWin]
+  const RsPlan plan(bucket + B, H);
+  int32_t* win = plan.order + B;                                                          // [B][kGeoWin]
   recommend_geo_window_kernel<<<(unsigned)((B + kRtThreads - 1) / kRtThreads), kRtThreads, 0, s>>>(
       centre_xyz, threshold, B, cell_deg, (int)num_lat, (int)num_lon, H, win, bucket, err);
   YR_CHECK_LAUNCH();
-  recommend_subset_plan_kernel<<<1, kRsPlanThreads, 0, s>>>(bucket, (int)B, H, TU, cursor, rows_at, blocks_at, order,
-                                                            err);
+  recommend_subset_plan_kernel<<<1, kRsPlanThreads, 0, s>>>(bucket, (int)B, H, TU, plan.cursor, plan.rows_at,
+                                                            plan.blocks_at, plan.order, err);
   YR_CHECK_LAUNCH();
-  int rc;
-#define YR_GEO_LAUNCH(T, TU_, BIAS)                                                                                       \
-  geo_launch<T, TU_, BIAS>(U, nU, V, d, user_ids, B, cell_keys, cell_ptr, num_cells, cell_items, item_xyz, (int)num_lon, \
-                           centre_xyz, threshold, win, H, rows_at, blocks_at, order, seen_ptr, seen_idx, K, S, partial,  \
-                           out_ids, out_scores, err, item_bias, s)
-#define YR_GEO_TU(T, BIAS)                                                                                                \
-  (TU == 16 ? YR_GEO_LAUNCH(T, 16, BIAS) : TU == 8 ? YR_GEO_LAUNCH(T, 8, BIAS) : YR_GEO_LAUNCH(T, 4, BIAS))
-  if (dtype == YR_DTYPE_F32)
-    rc = item_bias ? YR_GEO_TU(float, true) : YR_GEO_TU(float, false);
-  else
-    rc = item_bias ? YR_GEO_TU(__nv_bfloat16, true) : YR_GEO_TU(__nv_bfloat16, false);
-#undef YR_GEO_TU
-#undef YR_GEO_LAUNCH
+  const dim3 grid((unsigned)((B + TU - 1) / TU + std::min<int64_t>((int64_t)H + 2, B)), (unsigned)S);
+  const RtBytes<GeoSmem> smem(TU, d);
+  const int rc = rt_dispatch(dtype, TU, item_bias != nullptr, [&](auto inst) {
+    using I = decltype(inst);
+    using T = typename I::T;
+    return rt_launch<recommend_geo_kernel<T, I::TU, I::kBias>>(
+        grid, smem.bytes, smem.max, s, reinterpret_cast<const T*>(U), nU, reinterpret_cast<const T*>(V), d, user_ids,
+        B, cell_keys, cell_ptr, num_cells, cell_items, item_xyz, (int)num_lon, centre_xyz, threshold, win, H,
+        plan.rows_at, plan.blocks_at, plan.order, seen_ptr, seen_idx, K, S, partial, out_ids, out_scores, err,
+        item_bias);
+  });
   if (rc || S == 1) return rc;
   return merge_launch(partial, S, B, K, out_ids, out_scores, s);
 }

@@ -632,6 +632,65 @@ def _item_bias(item_bias: Optional[torch.Tensor], nI: int, dev, what: str) -> Op
     return item_bias.detach().contiguous()
 
 
+def _rt_tables(what: str, U, V, user_ids, K):
+    """The checks of the embedding tables, k and user_ids every retrieval entry makes: (device, d, nU, nI, K, B)."""
+    if not (torch.is_tensor(U) and torch.is_tensor(V) and torch.is_tensor(user_ids)):
+        raise TypeError(f"{what}: U, V and user_ids must be tensors")
+    if not (U.is_cuda and V.is_cuda and user_ids.is_cuda):
+        raise YelprecError(f"{what}: U, V and user_ids must be CUDA tensors (the reference path is "
+                           "retrieval.recommend_reference)")
+    dev = U.device
+    if V.device != dev or user_ids.device != dev:
+        raise ValueError(f"{what}: tensors on different devices ({U.device}, {V.device}, {user_ids.device})")
+    if U.dtype not in _RT_DTYPES or V.dtype != U.dtype:
+        raise TypeError(f"{what}: U and V must both be float32 or both bfloat16, got {U.dtype} and {V.dtype}")
+    if U.dim() != 2 or V.dim() != 2 or U.shape[1] != V.shape[1]:
+        raise ValueError(f"{what}: U [nU x d] and V [nI x d] expected, got {tuple(U.shape)} and {tuple(V.shape)}")
+    d = int(U.shape[1])
+    if d % 8 != 0 or d > RECOMMEND_MAX_D:
+        raise ValueError(f"{what}: embedding width {d} must be a multiple of 8 and at most {RECOMMEND_MAX_D}")
+    nU, nI = int(U.shape[0]), int(V.shape[0])
+    if nU == 0 or nI == 0 or nI >= 2 ** 31 - 1:
+        raise ValueError(f"{what}: {nU} users x {nI} items is not a valid catalog")
+    if isinstance(K, bool) or int(K) != K or not 1 <= int(K) <= RECOMMEND_MAX_K:
+        raise ValueError(f"{what}: k must be an integer in [1, {RECOMMEND_MAX_K}], got {K}")
+    if user_ids.dtype not in (I64, I32) or user_ids.dim() != 1:
+        raise TypeError(f"{what}: user_ids must be a 1-D int64 or int32 tensor, got {user_ids.dtype} "
+                        f"{tuple(user_ids.shape)}")
+    return dev, d, nU, nI, int(K), int(user_ids.numel())
+
+
+def _rt_seen_and_bias(what: str, seen_ptr, seen_idx, rows: int, item_bias, nI: int, dev):
+    """The seen lists (int32 CSR over `rows` rows) and item_bias, checked and made contiguous: (ptr, idx, bias)."""
+    if (seen_ptr is None) != (seen_idx is None):
+        raise ValueError(f"{what}: seen_ptr and seen_idx go together")
+    bias = _item_bias(item_bias, nI, dev, what)
+    if seen_ptr is not None:
+        if seen_ptr.dtype != I32 or seen_idx.dtype != I32 or seen_ptr.numel() != rows + 1:
+            raise ValueError(f"{what}: seen lists must be int32 CSR with {rows + 1} offsets")
+        if seen_ptr.device != dev or seen_idx.device != dev:
+            raise ValueError(f"{what}: seen lists must live on the device of the embeddings")
+        seen_ptr = seen_ptr.contiguous()
+        seen_idx = seen_idx.contiguous() if seen_idx.numel() else torch.zeros(1, dtype=I32, device=dev)
+    return seen_ptr, seen_idx, bias
+
+
+def _rt_run(U, V, B: int, K: int, dev, ws_bytes, launch):
+    """Allocates the outputs, the workspace (ws_bytes(lib) bytes) and the error word, and calls
+    launch(lib, Uc, Vc, ids, scores, ws, nbytes, err): (ids, scores, error word), the error word 0 when B == 0."""
+    lib = _cabi.load()
+    Uc, Vc = U.detach().contiguous(), V.detach().contiguous()
+    ids = torch.empty(B, K, device=dev, dtype=I64)
+    scores = torch.empty(B, K, device=dev, dtype=F32)
+    if B == 0:
+        return ids, scores, 0
+    err = torch.zeros(1, device=dev, dtype=I32)
+    nbytes = ws_bytes(lib)
+    ws = torch.empty(max(nbytes, 1), device=dev, dtype=torch.uint8)
+    launch(lib, Uc, Vc, ids, scores, ws, nbytes, err)
+    return ids, scores, int(err.item())
+
+
 def recommend_topk(U: torch.Tensor, V: torch.Tensor, user_ids: torch.Tensor, K: int, seen_ptr: Optional[torch.Tensor] = None,
                    seen_idx: Optional[torch.Tensor] = None, seen_by_row: bool = False,
                    masked_score: float = float("-inf"),
@@ -640,57 +699,20 @@ def recommend_topk(U: torch.Tensor, V: torch.Tensor, user_ids: torch.Tensor, K: 
     asc), score = U[uid] . V[item] (+ item_bias[item]) in fp32 (fp32 or bf16 tables, fp32 bias). Seen items (CSR int32,
     ascending per row, rows = user ids, or batch rows with seen_by_row) score `masked_score`; -inf drops them. Short rows
     are padded with id -1 / score -inf."""
-    if not (torch.is_tensor(U) and torch.is_tensor(V) and torch.is_tensor(user_ids)):
-        raise TypeError("recommend_topk: U, V and user_ids must be tensors")
-    if not (U.is_cuda and V.is_cuda and user_ids.is_cuda):
-        raise YelprecError("recommend_topk: U, V and user_ids must be CUDA tensors (the reference path is "
-                           "retrieval.recommend_reference)")
-    dev = U.device
-    if V.device != dev or user_ids.device != dev:
-        raise ValueError(f"recommend_topk: tensors on different devices ({U.device}, {V.device}, {user_ids.device})")
-    if U.dtype not in _RT_DTYPES or V.dtype != U.dtype:
-        raise TypeError(f"recommend_topk: U and V must both be float32 or both bfloat16, got {U.dtype} and {V.dtype}")
-    if U.dim() != 2 or V.dim() != 2 or U.shape[1] != V.shape[1]:
-        raise ValueError(f"recommend_topk: U [nU x d] and V [nI x d] expected, got {tuple(U.shape)} and {tuple(V.shape)}")
-    d = int(U.shape[1])
-    if d % 8 != 0 or d > RECOMMEND_MAX_D:
-        raise ValueError(f"recommend_topk: embedding width {d} must be a multiple of 8 and at most {RECOMMEND_MAX_D}")
-    nU, nI = int(U.shape[0]), int(V.shape[0])
-    if nU == 0 or nI == 0 or nI >= 2 ** 31 - 1:
-        raise ValueError(f"recommend_topk: {nU} users x {nI} items is not a valid catalog")
-    if isinstance(K, bool) or int(K) != K or not 1 <= int(K) <= RECOMMEND_MAX_K:
-        raise ValueError(f"recommend_topk: k must be an integer in [1, {RECOMMEND_MAX_K}], got {K}")
-    K = int(K)
-    if user_ids.dtype not in (I64, I32) or user_ids.dim() != 1:
-        raise TypeError(f"recommend_topk: user_ids must be a 1-D int64 or int32 tensor, got {user_ids.dtype} {tuple(user_ids.shape)}")
-    if (seen_ptr is None) != (seen_idx is None):
-        raise ValueError("recommend_topk: seen_ptr and seen_idx go together")
-    bias = _item_bias(item_bias, nI, dev, "recommend_topk")
+    what = "recommend_topk"
+    dev, d, nU, nI, K, B = _rt_tables(what, U, V, user_ids, K)
+    seen_ptr, seen_idx, bias = _rt_seen_and_bias(what, seen_ptr, seen_idx, B if seen_by_row else nU, item_bias, nI, dev)
     uid = user_ids.to(I64).contiguous()
-    B = int(uid.numel())
-    if seen_ptr is not None:
-        rows = B if seen_by_row else nU
-        if seen_ptr.dtype != I32 or seen_idx.dtype != I32 or seen_ptr.numel() != rows + 1:
-            raise ValueError(f"recommend_topk: seen lists must be int32 CSR with {rows + 1} offsets")
-        if seen_ptr.device != dev or seen_idx.device != dev:
-            raise ValueError("recommend_topk: seen lists must live on the device of the embeddings")
-        seen_ptr = seen_ptr.contiguous()
-        seen_idx = seen_idx.contiguous() if seen_idx.numel() else torch.zeros(1, dtype=I32, device=dev)
-    lib = _cabi.load()
-    Uc, Vc = U.detach().contiguous(), V.detach().contiguous()
-    ids = torch.empty(B, K, device=dev, dtype=I64)
-    scores = torch.empty(B, K, device=dev, dtype=F32)
-    if B == 0:
-        return ids, scores
-    err = torch.zeros(1, device=dev, dtype=I32)
-    nbytes = lib.yr_recommend_ws_bytes(B, nI, K)
-    ws = torch.empty(max(nbytes, 1), device=dev, dtype=torch.uint8)
-    check(lib.yr_recommend_topk_ex(Uc.data_ptr(), nU, Vc.data_ptr(), nI, d, _RT_DTYPES[U.dtype], dptr(uid, I64), B,
-                                   dptr(seen_ptr), dptr(seen_idx), 1 if seen_by_row else 0, float(masked_score), K,
-                                   dptr(ids), dptr(scores), dptr(ws), nbytes, dptr(err), stream_ptr(dev), dptr(bias)),
-          "yr_recommend_topk_ex")
-    if int(err.item()) != 0:
-        raise IndexError(f"recommend_topk: user id out of range [0, {nU})")
+
+    def launch(lib, Uc, Vc, ids, scores, ws, nbytes, err):
+        check(lib.yr_recommend_topk_ex(Uc.data_ptr(), nU, Vc.data_ptr(), nI, d, _RT_DTYPES[U.dtype], dptr(uid, I64), B,
+                                       dptr(seen_ptr), dptr(seen_idx), 1 if seen_by_row else 0, float(masked_score), K,
+                                       dptr(ids), dptr(scores), dptr(ws), nbytes, dptr(err), stream_ptr(dev),
+                                       dptr(bias)), "yr_recommend_topk_ex")
+
+    ids, scores, e = _rt_run(U, V, B, K, dev, lambda lib: lib.yr_recommend_ws_bytes(B, nI, K), launch)
+    if e != 0:
+        raise IndexError(f"{what}: user id out of range [0, {nU})")
     return ids, scores
 
 
@@ -704,78 +726,41 @@ def recommend_subset_topk(U: torch.Tensor, V: torch.Tensor, user_ids: torch.Tens
     streams (the longest subset, num_items if a row is -1); it sets only the number of item splits. Seen lists are indexed
     by user id. (ids int64 [B x K], scores float32 [B x K]), identical to recommend_topk with the items outside each row's
     subset excluded."""
+    what = "recommend_subset_topk"
     if not (torch.is_tensor(subset_ptr) and torch.is_tensor(subset_idx) and torch.is_tensor(subset_ids)):
-        raise TypeError("recommend_subset_topk: subset_ptr, subset_idx and subset_ids must be tensors")
-    if not (torch.is_tensor(U) and torch.is_tensor(V) and torch.is_tensor(user_ids)):
-        raise TypeError("recommend_subset_topk: U, V and user_ids must be tensors")
-    if not (U.is_cuda and V.is_cuda and user_ids.is_cuda):
-        raise YelprecError("recommend_subset_topk: U, V and user_ids must be CUDA tensors (the reference path is "
-                           "retrieval.recommend_reference)")
-    dev = U.device
-    if V.device != dev or user_ids.device != dev:
-        raise ValueError(f"recommend_subset_topk: tensors on different devices ({U.device}, {V.device}, {user_ids.device})")
-    if U.dtype not in _RT_DTYPES or V.dtype != U.dtype:
-        raise TypeError(f"recommend_subset_topk: U and V must both be float32 or both bfloat16, got {U.dtype} and {V.dtype}")
-    if U.dim() != 2 or V.dim() != 2 or U.shape[1] != V.shape[1]:
-        raise ValueError(f"recommend_subset_topk: U [nU x d] and V [nI x d] expected, got {tuple(U.shape)} and "
-                         f"{tuple(V.shape)}")
-    d = int(U.shape[1])
-    if d % 8 != 0 or d > RECOMMEND_MAX_D:
-        raise ValueError(f"recommend_subset_topk: embedding width {d} must be a multiple of 8 and at most {RECOMMEND_MAX_D}")
-    nU, nI = int(U.shape[0]), int(V.shape[0])
-    if nU == 0 or nI == 0 or nI >= 2 ** 31 - 1:
-        raise ValueError(f"recommend_subset_topk: {nU} users x {nI} items is not a valid catalog")
-    if isinstance(K, bool) or int(K) != K or not 1 <= int(K) <= RECOMMEND_MAX_K:
-        raise ValueError(f"recommend_subset_topk: k must be an integer in [1, {RECOMMEND_MAX_K}], got {K}")
-    K = int(K)
-    if user_ids.dtype not in (I64, I32) or user_ids.dim() != 1:
-        raise TypeError(f"recommend_subset_topk: user_ids must be a 1-D int64 or int32 tensor, got {user_ids.dtype} "
-                        f"{tuple(user_ids.shape)}")
-    B = int(user_ids.numel())
+        raise TypeError(f"{what}: subset_ptr, subset_idx and subset_ids must be tensors")
+    dev, d, nU, nI, K, B = _rt_tables(what, U, V, user_ids, K)
     if subset_ids.dtype not in (I64, I32) or subset_ids.dim() != 1:
-        raise TypeError(f"recommend_subset_topk: subset_ids must be a 1-D int64 or int32 tensor, got {subset_ids.dtype} "
+        raise TypeError(f"{what}: subset_ids must be a 1-D int64 or int32 tensor, got {subset_ids.dtype} "
                         f"{tuple(subset_ids.shape)}")
     if subset_ids.numel() != B:
-        raise ValueError(f"recommend_subset_topk: {subset_ids.numel()} subset ids for {B} users")
+        raise ValueError(f"{what}: {subset_ids.numel()} subset ids for {B} users")
     if subset_ptr.dtype != I32 or subset_idx.dtype != I32 or subset_ptr.dim() != 1 or subset_ptr.numel() < 1:
-        raise ValueError("recommend_subset_topk: subsets must be an int32 CSR (subset_ptr [G + 1], subset_idx)")
+        raise ValueError(f"{what}: subsets must be an int32 CSR (subset_ptr [G + 1], subset_idx)")
     if subset_ptr.device != dev or subset_idx.device != dev or subset_ids.device != dev:
-        raise ValueError("recommend_subset_topk: subsets and subset ids must live on the device of the embeddings")
+        raise ValueError(f"{what}: subsets and subset ids must live on the device of the embeddings")
     G = int(subset_ptr.numel()) - 1
     if isinstance(max_len, bool) or int(max_len) != max_len or int(max_len) < 0:
-        raise ValueError(f"recommend_subset_topk: max_len must be a non-negative integer, got {max_len}")
-    if (seen_ptr is None) != (seen_idx is None):
-        raise ValueError("recommend_subset_topk: seen_ptr and seen_idx go together")
-    bias = _item_bias(item_bias, nI, dev, "recommend_subset_topk")
-    if seen_ptr is not None:
-        if seen_ptr.dtype != I32 or seen_idx.dtype != I32 or seen_ptr.numel() != nU + 1:
-            raise ValueError(f"recommend_subset_topk: seen lists must be int32 CSR with {nU + 1} offsets")
-        if seen_ptr.device != dev or seen_idx.device != dev:
-            raise ValueError("recommend_subset_topk: seen lists must live on the device of the embeddings")
-        seen_ptr = seen_ptr.contiguous()
-        seen_idx = seen_idx.contiguous() if seen_idx.numel() else torch.zeros(1, dtype=I32, device=dev)
+        raise ValueError(f"{what}: max_len must be a non-negative integer, got {max_len}")
+    seen_ptr, seen_idx, bias = _rt_seen_and_bias(what, seen_ptr, seen_idx, nU, item_bias, nI, dev)
     uid = user_ids.to(I64).contiguous()
     sid = subset_ids.to(I64).contiguous()
     sptr = subset_ptr.contiguous()
     sidx = subset_idx.contiguous() if subset_idx.numel() else torch.zeros(1, dtype=I32, device=dev)
-    lib = _cabi.load()
-    Uc, Vc = U.detach().contiguous(), V.detach().contiguous()
-    ids = torch.empty(B, K, device=dev, dtype=I64)
-    scores = torch.empty(B, K, device=dev, dtype=F32)
-    if B == 0:
-        return ids, scores
-    err = torch.zeros(1, device=dev, dtype=I32)
-    nbytes = lib.yr_recommend_subset_ws_bytes(B, G, int(max_len), K)
-    ws = torch.empty(max(nbytes, 1), device=dev, dtype=torch.uint8)
-    check(lib.yr_recommend_subset_topk_ex(Uc.data_ptr(), nU, Vc.data_ptr(), nI, d, _RT_DTYPES[U.dtype], dptr(uid, I64),
-                                          B, dptr(sptr, I32), dptr(sidx, I32), G, int(max_len), dptr(sid, I64),
-                                          dptr(seen_ptr), dptr(seen_idx), K, dptr(ids), dptr(scores), dptr(ws), nbytes,
-                                          dptr(err), stream_ptr(dev), dptr(bias)), "yr_recommend_subset_topk_ex")
-    e = int(err.item())
+
+    def launch(lib, Uc, Vc, ids, scores, ws, nbytes, err):
+        check(lib.yr_recommend_subset_topk_ex(Uc.data_ptr(), nU, Vc.data_ptr(), nI, d, _RT_DTYPES[U.dtype],
+                                              dptr(uid, I64), B, dptr(sptr, I32), dptr(sidx, I32), G, int(max_len),
+                                              dptr(sid, I64), dptr(seen_ptr), dptr(seen_idx), K, dptr(ids), dptr(scores),
+                                              dptr(ws), nbytes, dptr(err), stream_ptr(dev), dptr(bias)),
+              "yr_recommend_subset_topk_ex")
+
+    ids, scores, e = _rt_run(U, V, B, K, dev, lambda lib: lib.yr_recommend_subset_ws_bytes(B, G, int(max_len), K),
+                             launch)
     if e & 1:
-        raise IndexError(f"recommend_subset_topk: user id out of range [0, {nU})")
+        raise IndexError(f"{what}: user id out of range [0, {nU})")
     if e & 2:
-        raise IndexError(f"recommend_subset_topk: subset id out of range [-1, {G})")
+        raise IndexError(f"{what}: subset id out of range [-1, {G})")
     return ids, scores
 
 
@@ -798,84 +783,45 @@ def recommend_geo_topk(U: torch.Tensor, V: torch.Tensor, user_ids: torch.Tensor,
     [B x K]), identical to recommend_topk with the items outside each row's radius excluded. A user id out of range
     raises IndexError, a non-finite centre or a NaN / +inf threshold ValueError (both after the launch, from the error
     word: one scalar read per call)."""
+    what = "recommend_geo_topk"
     if not all(torch.is_tensor(x) for x in (cell_keys, cell_ptr, cell_items, item_xyz, centre_xyz, threshold)):
-        raise TypeError("recommend_geo_topk: the item grid, item_xyz, centre_xyz and threshold must be tensors")
-    if not (torch.is_tensor(U) and torch.is_tensor(V) and torch.is_tensor(user_ids)):
-        raise TypeError("recommend_geo_topk: U, V and user_ids must be tensors")
-    if not (U.is_cuda and V.is_cuda and user_ids.is_cuda):
-        raise YelprecError("recommend_geo_topk: U, V and user_ids must be CUDA tensors (the reference path is "
-                           "retrieval.recommend_reference)")
-    dev = U.device
-    if V.device != dev or user_ids.device != dev:
-        raise ValueError(f"recommend_geo_topk: tensors on different devices ({U.device}, {V.device}, {user_ids.device})")
-    if U.dtype not in _RT_DTYPES or V.dtype != U.dtype:
-        raise TypeError(f"recommend_geo_topk: U and V must both be float32 or both bfloat16, got {U.dtype} and {V.dtype}")
-    if U.dim() != 2 or V.dim() != 2 or U.shape[1] != V.shape[1]:
-        raise ValueError(f"recommend_geo_topk: U [nU x d] and V [nI x d] expected, got {tuple(U.shape)} and "
-                         f"{tuple(V.shape)}")
-    d = int(U.shape[1])
-    if d % 8 != 0 or d > RECOMMEND_MAX_D:
-        raise ValueError(f"recommend_geo_topk: embedding width {d} must be a multiple of 8 and at most {RECOMMEND_MAX_D}")
-    nU, nI = int(U.shape[0]), int(V.shape[0])
-    if nU == 0 or nI == 0 or nI >= 2 ** 31 - 1:
-        raise ValueError(f"recommend_geo_topk: {nU} users x {nI} items is not a valid catalog")
-    if isinstance(K, bool) or int(K) != K or not 1 <= int(K) <= RECOMMEND_MAX_K:
-        raise ValueError(f"recommend_geo_topk: k must be an integer in [1, {RECOMMEND_MAX_K}], got {K}")
-    K = int(K)
-    if user_ids.dtype not in (I64, I32) or user_ids.dim() != 1:
-        raise TypeError(f"recommend_geo_topk: user_ids must be a 1-D int64 or int32 tensor, got {user_ids.dtype} "
-                        f"{tuple(user_ids.shape)}")
-    B = int(user_ids.numel())
+        raise TypeError(f"{what}: the item grid, item_xyz, centre_xyz and threshold must be tensors")
+    dev, d, nU, nI, K, B = _rt_tables(what, U, V, user_ids, K)
     if centre_xyz.dtype != F64 or threshold.dtype != F64:
-        raise TypeError(f"recommend_geo_topk: centre_xyz and threshold must be float64, got {centre_xyz.dtype} and "
+        raise TypeError(f"{what}: centre_xyz and threshold must be float64, got {centre_xyz.dtype} and "
                         f"{threshold.dtype}")
     if tuple(centre_xyz.shape) != (B, 3) or tuple(threshold.shape) != (B,):
-        raise ValueError(f"recommend_geo_topk: centre_xyz [{B} x 3] and threshold [{B}] expected, got "
+        raise ValueError(f"{what}: centre_xyz [{B} x 3] and threshold [{B}] expected, got "
                          f"{tuple(centre_xyz.shape)} and {tuple(threshold.shape)}")
     if item_xyz.dtype != F64 or tuple(item_xyz.shape) != (nI, 3):
-        raise ValueError(f"recommend_geo_topk: item_xyz must be float64 [{nI} x 3]")
+        raise ValueError(f"{what}: item_xyz must be float64 [{nI} x 3]")
     if cell_keys.dtype != I64 or cell_ptr.dtype != I32 or cell_items.dtype != I32 or cell_keys.dim() != 1 or \
             cell_ptr.numel() != cell_keys.numel() + 1 or cell_items.numel() != nI:
-        raise ValueError("recommend_geo_topk: the item grid must be cell_keys int64 [C], cell_ptr int32 [C + 1] and "
+        raise ValueError(f"{what}: the item grid must be cell_keys int64 [C], cell_ptr int32 [C + 1] and "
                          f"cell_items int32 [{nI}]")
     if any(x.device != dev for x in (cell_keys, cell_ptr, cell_items, item_xyz, centre_xyz, threshold)):
-        raise ValueError("recommend_geo_topk: the item grid, item_xyz, centre_xyz and threshold must live on the device "
+        raise ValueError(f"{what}: the item grid, item_xyz, centre_xyz and threshold must live on the device "
                          "of the embeddings")
     cell_deg = float(cell_deg)
     if not 0.0 < cell_deg <= 360.0:
-        raise ValueError(f"recommend_geo_topk: cell_deg must be in (0, 360], got {cell_deg}")
+        raise ValueError(f"{what}: cell_deg must be in (0, 360], got {cell_deg}")
     nlat, nlon = geo_grid_shape(cell_deg)
-    if (seen_ptr is None) != (seen_idx is None):
-        raise ValueError("recommend_geo_topk: seen_ptr and seen_idx go together")
-    bias = _item_bias(item_bias, nI, dev, "recommend_geo_topk")
-    if seen_ptr is not None:
-        if seen_ptr.dtype != I32 or seen_idx.dtype != I32 or seen_ptr.numel() != nU + 1:
-            raise ValueError(f"recommend_geo_topk: seen lists must be int32 CSR with {nU + 1} offsets")
-        if seen_ptr.device != dev or seen_idx.device != dev:
-            raise ValueError("recommend_geo_topk: seen lists must live on the device of the embeddings")
-        seen_ptr = seen_ptr.contiguous()
-        seen_idx = seen_idx.contiguous() if seen_idx.numel() else torch.zeros(1, dtype=I32, device=dev)
+    seen_ptr, seen_idx, bias = _rt_seen_and_bias(what, seen_ptr, seen_idx, nU, item_bias, nI, dev)
     uid = user_ids.to(I64).contiguous()
     keys = cell_keys.contiguous() if cell_keys.numel() else torch.zeros(1, dtype=I64, device=dev)
     cptr, citems, P = cell_ptr.contiguous(), cell_items.contiguous(), item_xyz.contiguous()
     c, t = centre_xyz.contiguous(), threshold.contiguous()
-    lib = _cabi.load()
-    Uc, Vc = U.detach().contiguous(), V.detach().contiguous()
-    ids = torch.empty(B, K, device=dev, dtype=I64)
-    scores = torch.empty(B, K, device=dev, dtype=F32)
-    if B == 0:
-        return ids, scores
-    err = torch.zeros(1, device=dev, dtype=I32)
-    nbytes = lib.yr_recommend_geo_ws_bytes(B, nI, K)
-    ws = torch.empty(max(nbytes, 1), device=dev, dtype=torch.uint8)
-    check(lib.yr_recommend_geo_topk(Uc.data_ptr(), nU, Vc.data_ptr(), nI, d, _RT_DTYPES[U.dtype], dptr(uid, I64), B,
-                                    dptr(keys, I64), dptr(cptr, I32), int(cell_keys.numel()), dptr(citems, I32),
-                                    dptr(P, F64), cell_deg, nlat, nlon, dptr(c, F64), dptr(t, F64), dptr(seen_ptr),
-                                    dptr(seen_idx), K, dptr(ids), dptr(scores), dptr(ws), nbytes, dptr(err),
-                                    stream_ptr(dev), dptr(bias)), "yr_recommend_geo_topk")
-    e = int(err.item())
+
+    def launch(lib, Uc, Vc, ids, scores, ws, nbytes, err):
+        check(lib.yr_recommend_geo_topk(Uc.data_ptr(), nU, Vc.data_ptr(), nI, d, _RT_DTYPES[U.dtype], dptr(uid, I64), B,
+                                        dptr(keys, I64), dptr(cptr, I32), int(cell_keys.numel()), dptr(citems, I32),
+                                        dptr(P, F64), cell_deg, nlat, nlon, dptr(c, F64), dptr(t, F64), dptr(seen_ptr),
+                                        dptr(seen_idx), K, dptr(ids), dptr(scores), dptr(ws), nbytes, dptr(err),
+                                        stream_ptr(dev), dptr(bias)), "yr_recommend_geo_topk")
+
+    ids, scores, e = _rt_run(U, V, B, K, dev, lambda lib: lib.yr_recommend_geo_ws_bytes(B, nI, K), launch)
     if e & 1:
-        raise IndexError(f"recommend_geo_topk: user id out of range [0, {nU})")
+        raise IndexError(f"{what}: user id out of range [0, {nU})")
     if e & 2:
-        raise ValueError("recommend_geo_topk: a centre is not finite or a threshold is NaN or +inf")
+        raise ValueError(f"{what}: a centre is not finite or a threshold is NaN or +inf")
     return ids, scores

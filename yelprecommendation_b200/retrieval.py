@@ -70,6 +70,16 @@ def _as_f64(x) -> np.ndarray:
     return np.asarray(x.detach().cpu().numpy() if torch.is_tensor(x) else x, dtype=np.float64)
 
 
+def _on_device(cache: dict, device, tensors: Tuple[torch.Tensor, ...]) -> Tuple[torch.Tensor, ...]:
+    """`tensors` on `device`, copied once per device into `cache` (keyed by the device, "cuda" as the current one)."""
+    device = torch.device(device)
+    if device.type == "cuda" and device.index is None:
+        device = torch.device("cuda", torch.cuda.current_device())
+    if device not in cache:
+        cache[device] = tuple(x.to(device) for x in tensors)
+    return cache[device]
+
+
 class ItemLocations:
     """Item positions on the sphere and a grid index over them, for radius-restricted retrieval.
 
@@ -110,12 +120,7 @@ class ItemLocations:
 
     def on(self, device) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
         """(cell_keys, cell_ptr, cell_items, P) on `device`, copied once per device."""
-        device = torch.device(device)
-        if device.type == "cuda" and device.index is None:
-            device = torch.device("cuda", torch.cuda.current_device())
-        if device not in self._on:
-            self._on[device] = tuple(x.to(device) for x in (self.cell_keys, self.cell_ptr, self.cell_items, self.P))
-        return self._on[device]
+        return _on_device(self._on, device, (self.cell_keys, self.cell_ptr, self.cell_items, self.P))
 
 
 def geo_query(near, radius_km, B: int) -> Tuple[np.ndarray, np.ndarray]:
@@ -199,12 +204,7 @@ class ItemLists:
 
     def on(self, device) -> Tuple[torch.Tensor, torch.Tensor]:
         """(ptr, idx) on `device`, copied once per device."""
-        device = torch.device(device)
-        if device.type == "cuda" and device.index is None:
-            device = torch.device("cuda", torch.cuda.current_device())
-        if device not in self._on:
-            self._on[device] = (self.ptr.to(device), self.idx.to(device))
-        return self._on[device]
+        return _on_device(self._on, device, (self.ptr, self.idx))
 
 
 class SeenItems(ItemLists):
