@@ -636,6 +636,25 @@ int yr_recommend_geo_topk(const void* U, int64_t nU, const void* V, int64_t nI, 
                           const int32_t* seen_idx, int K, int64_t* out_ids, float* out_scores, void* ws, size_t ws_bytes,
                           int32_t* err, yr_stream stream, const float* item_bias);
 
+/* Diversity re-ranking (Maximal Marginal Relevance) of B pools of N candidates, e.g. the output of yr_recommend_topk
+ * with K = N. Position j of row b holds item p_j = pool_ids[b * N + j] (-1: an empty slot) with relevance
+ * r_j = pool_scores[b * N + j]. V [nI x d] of `dtype` is the item table similarity is measured in. With fp32 arithmetic,
+ * every operation separately rounded (no fma contraction outside the sums):
+ *   ss_j = sum_k V[p_j,k]^2 (any summation order), n_j = 1 / sqrt(ss_j) (sqrt and reciprocal each correctly rounded;
+ *   n_j = 0 when ss_j == 0), sim(i, j) = dot(V[p_i], V[p_j]) * (n_i * n_j) (the dot in any summation order).
+ * a = lam and c = one_minus_lam, both computed by the caller (c = fl(1 - a)). For t = 0 .. K-1: pen_j = 0 while nothing
+ * has been picked, after that the maximum of sim(j, s) over the picked positions s (a NaN similarity makes it NaN);
+ * m_j = (a * r_j) - (c * pen_j), with -0 ranking as +0 and NaN as -inf. Step t picks the unpicked non-empty position
+ * with the largest m_j, ties to the lower position, and writes out_ids[b * K + t] = p_j and out_scores[b * K + t] = r_j
+ * (pick order; the scores stay the pool's). When no non-empty position is left the rest of the row is -1 / -INFINITY.
+ * With lam = 1 and finite similarities, m_j = r_j: a pool in (score desc, id asc) order, as yr_recommend_topk writes
+ * it, comes back as its first K entries. A pool id outside [-1, nI) sets *err |= 1 (err may be
+ * NULL) and makes the row all padding. 1 <= K <= N <= 1024, 0 <= lam, one_minus_lam <= 1, d % 8 == 0, d <= 1024,
+ * nI < 2^31 - 1, B < 2^31 - 1. No workspace. */
+int yr_recommend_mmr(const void* V, int64_t nI, int d, int dtype, const int64_t* pool_ids, const float* pool_scores,
+                     int64_t B, int N, int K, float lam, float one_minus_lam, int64_t* out_ids, float* out_scores,
+                     int32_t* err, yr_stream stream);
+
 #ifdef __cplusplus
 }
 #endif

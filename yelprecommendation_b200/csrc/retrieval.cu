@@ -868,6 +868,172 @@ recommend_geo_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ 
       [&](int u, int j) { return j < cnt[u] ? keys[(size_t)u * CAP + j] : 0; });   // zero beyond the count: padding
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// Diversity re-ranking (Maximal Marginal Relevance) of a pool of N candidates per row, one block per row. Position j of
+// row b holds item p_j (-1: empty) with relevance r_j; n_j = 1 / sqrt(sum_k V[p_j,k]^2) (0 for a zero row), sim(i, j) =
+// fl(V[p_i] . V[p_j] * fl(n_i * n_j)). Step t picks the unpicked non-empty position with the largest
+// m_j = fl(fl(a * r_j) - fl(c * pen_j)) (-0 as +0, NaN as -inf; ties to the lower position), pen_j = 0 before the first
+// pick and the largest sim(j, s) over the picked s after it (a NaN similarity sticks: the candidate ranks last).
+//
+// The pool's rows are staged in shared memory as T when the block's layout fits kMmrStageMax, otherwise read from V (L2)
+// at every step. A group of G lanes (G = the largest power of two <= d / 8, at most 32) computes one candidate's dot
+// product, 8 elements a lane at a time. Each step updates pen for every live candidate against the last pick and takes
+// one block-wide maximum over 64-bit keys (order-preserving m, complemented position): one barrier a step, the warp
+// maxima double-buffered by parity.
+// ---------------------------------------------------------------------------------------------------------------------
+constexpr int kMmrMaxN = 1024;
+// Rows are staged only while two blocks fit an SM (228 KB, 1 KB of it reserved per block): on one B200, staging up to the
+// 227 KB a block may have ran 1.3-2.2x slower than reading the rows from L2 (one block of 8 warps an SM), while at this
+// limit staging is within 2 % of the L2 path or beats it by up to 7 % (scripts/recommend_diverse_bench.py).
+constexpr size_t kMmrStageMax = 113 * 1024;
+
+struct MmrSmem {   // recommend_mmr_kernel; the staged rows [N][d] of T at 0 (rows bytes, 0 when not staged)
+  size_t best, bad, pid, rs, nrm, pen, alive, bytes;
+  __host__ __device__ MmrSmem(int N, size_t rows)
+      : best(rows), bad(best + 2 * (kRtThreads / 32) * 8), pid(bad + 16), rs(pid + (size_t)N * 4),
+        nrm(rs + (size_t)N * 4), pen(nrm + (size_t)N * 4), alive(pen + (size_t)N * 4), bytes(alive + (size_t)N) {}
+};
+
+// v[0..7] = p[0..7] as floats, plain loads (p 16-byte aligned, in shared memory)
+__device__ __forceinline__ void mmr_lds8(const float* p, float (&v)[8]) {
+  const float4 a = reinterpret_cast<const float4*>(p)[0], b = reinterpret_cast<const float4*>(p)[1];
+  v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
+}
+__device__ __forceinline__ void mmr_lds8(const __nv_bfloat16* p, float (&v)[8]) {
+  const uint4 a = *reinterpret_cast<const uint4*>(p);
+  const uint32_t w[4] = {a.x, a.y, a.z, a.w};
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    v[2 * i] = __uint_as_float(w[i] << 16);
+    v[2 * i + 1] = __uint_as_float(w[i] & 0xffff0000u);
+  }
+}
+
+// x . y over d, split across a group of G lanes (gl = lane in the group): every lane of the group returns the sum.
+// All 32 lanes of the warp must call it; a lane with active == false contributes 0.
+template <typename T, bool kStaged>
+__device__ __forceinline__ float mmr_dot(const T* x, const T* y, int d, int gl, int G, bool active) {
+  float s = 0.f;
+  if (active) {
+    for (int k = gl * 8; k < d; k += G * 8) {
+      float u[8], v[8];
+      if constexpr (kStaged) { mmr_lds8(x + k, u); mmr_lds8(y + k, v); }
+      else { rt_load8(x + k, u); rt_load8(y + k, v); }
+#pragma unroll
+      for (int i = 0; i < 8; ++i) s = fmaf(u[i], v[i], s);
+    }
+  }
+  for (int o = G >> 1; o > 0; o >>= 1) s += __shfl_xor_sync(kFull, s, o);
+  return s;
+}
+
+// The key of position j with marginal relevance fl(fl(a * r) - fl(c * pen)): -0 ranks as +0, NaN as -inf. Never 0.
+__device__ __forceinline__ uint64_t mmr_key(float a, float c, float r, float pen, int j) {
+  float m = __fsub_rn(__fmul_rn(a, r), __fmul_rn(c, pen));
+  if (m == 0.f) m = 0.f;
+  if (m != m) m = -INFINITY;
+  return rt_key(m, (uint32_t)j);
+}
+
+template <typename T, bool kStaged>
+__global__ void __launch_bounds__(kRtThreads)
+recommend_mmr_kernel(const T* __restrict__ V, int64_t nI, int d, const int64_t* __restrict__ pool_ids,
+                     const float* __restrict__ pool_scores, int N, int K, float a, float c,
+                     int64_t* __restrict__ out_ids, float* __restrict__ out_scores, int32_t* err) {
+  extern __shared__ __align__(16) uint64_t rt_smem[];
+  const MmrSmem lay(N, kStaged ? (size_t)N * d * sizeof(T) : 0);
+  T* rows = rt_at<T>(rt_smem, 0);                              // [N][d] when staged
+  uint64_t* best = rt_at<uint64_t>(rt_smem, lay.best);         // [2][warps]: warp maxima, by step parity
+  int& bad = *rt_at<int>(rt_smem, lay.bad);                    // a pool id out of range
+  int* pid = rt_at<int>(rt_smem, lay.pid);                     // [N] item ids
+  float* rs = rt_at<float>(rt_smem, lay.rs);                   // [N] relevance
+  float* nrm = rt_at<float>(rt_smem, lay.nrm);                 // [N] inverse norms
+  float* pen = rt_at<float>(rt_smem, lay.pen);                 // [N] -inf until the first update
+  unsigned char* alive = rt_at<unsigned char>(rt_smem, lay.alive);   // [N] non-empty and unpicked
+
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int64_t b = blockIdx.x;
+  if (tid == 0) bad = 0;
+  __syncthreads();
+  for (int j = tid; j < N; j += kRtThreads) {
+    const int64_t id = pool_ids[b * N + j];
+    if (id < -1 || id >= nI) bad = 1;
+    pid[j] = (int)id;
+    rs[j] = pool_scores[b * N + j];
+    alive[j] = id >= 0;
+    pen[j] = -INFINITY;
+  }
+  __syncthreads();
+  if (bad) {   // uniform: the whole row is padding
+    if (tid == 0 && err) atomicOr(err, 1);
+    for (int t = tid; t < K; t += kRtThreads) { out_ids[b * K + t] = -1; out_scores[b * K + t] = -INFINITY; }
+    return;
+  }
+  if constexpr (kStaged) {
+    const int q = d * (int)sizeof(T) / 16;                     // 16-byte words a row
+    for (int i = tid; i < N * q; i += kRtThreads) {
+      const int j = i / q, w = i - j * q;
+      uint4 x = make_uint4(0u, 0u, 0u, 0u);
+      if (pid[j] >= 0) x = __ldg(reinterpret_cast<const uint4*>(V + (int64_t)pid[j] * d) + w);
+      reinterpret_cast<uint4*>(rows)[i] = x;
+    }
+    __syncthreads();
+  }
+  auto row = [&](int j) -> const T* { return kStaged ? rows + (size_t)j * d : V + (int64_t)pid[j] * d; };
+
+  int lg = 0;                                                  // G = 2^lg lanes a candidate (a division by G spills)
+  while (lg < 5 && (2 << lg) <= d / 8) ++lg;
+  const int G = 1 << lg, NG = kRtThreads >> lg, gi = tid >> lg, gl = tid & (G - 1);
+  // candidate j belongs to group j % NG: only that group reads or writes its pen, nrm (after this) and alive entries
+  for (int j0 = 0; j0 < N; j0 += NG) {
+    const int j = j0 + gi;
+    const bool live = j < N && alive[j];
+    const float ss = mmr_dot<T, kStaged>(live ? row(j) : nullptr, live ? row(j) : nullptr, d, gl, G, live);
+    if (live && gl == 0) nrm[j] = ss == 0.f ? 0.f : __frcp_rn(__fsqrt_rn(ss));
+  }
+  uint64_t mine = 0;                                           // the best key of this thread's candidates
+  for (int j0 = 0; j0 < N; j0 += NG) {
+    const int j = j0 + gi;
+    if (gl == 0 && j < N && alive[j]) mine = max(mine, mmr_key(a, c, rs[j], 0.f, j));
+  }
+  __syncthreads();                                             // every nrm written
+
+  for (int t = 0; t < K; ++t) {
+    uint64_t x = mine;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) x = max(x, __shfl_xor_sync(kFull, x, o));
+    uint64_t* bt = best + (t & 1) * (kRtThreads / 32);
+    if (lane == 0) bt[warp] = x;
+    __syncthreads();
+    x = 0;
+#pragma unroll
+    for (int w = 0; w < kRtThreads / 32; ++w) x = max(x, bt[w]);
+    if (x == 0) {                                              // nothing left: pad the rest of the row
+      for (int u = t + tid; u < K; u += kRtThreads) { out_ids[b * K + u] = -1; out_scores[b * K + u] = -INFINITY; }
+      return;
+    }
+    const int s = (int)~(uint32_t)x;
+    if (tid == 0) { out_ids[b * K + t] = pid[s]; out_scores[b * K + t] = rs[s]; }
+    if (t + 1 == K) return;
+    const T* vs = row(s);
+    const float ns = nrm[s];
+    mine = 0;
+    for (int j0 = 0; j0 < N; j0 += NG) {
+      const int j = j0 + gi;
+      const bool live = j < N && j != s && alive[j];
+      if (j == s && gl == 0) alive[s] = 0;
+      const float dot = mmr_dot<T, kStaged>(live ? row(j) : nullptr, vs, d, gl, G, live);
+      if (live && gl == 0) {
+        const float sim = __fmul_rn(dot, __fmul_rn(nrm[j], ns));
+        float p = pen[j];
+        if (sim > p || sim != sim) p = sim;                    // max, NaN-propagating (a NaN pen never leaves)
+        pen[j] = p;
+        mine = max(mine, mmr_key(a, c, rs[j], p, j));
+      }
+    }
+  }
+}
+
 }  // namespace yr
 
 using namespace yr;
@@ -1138,4 +1304,37 @@ extern "C" int yr_recommend_geo_topk(const void* U, int64_t nU, const void* V, i
   });
   if (rc || S == 1) return rc;
   return merge_launch(partial, S, B, K, out_ids, out_scores, s);
+}
+
+namespace {
+
+// recommend_mmr_kernel for table type T, the pool's rows staged in shared memory when they fit.
+template <typename T>
+int mmr_launch(const void* V, int64_t nI, int d, const int64_t* pool_ids, const float* pool_scores, int64_t B, int N,
+               int K, float a, float c, int64_t* out_ids, float* out_scores, int32_t* err, cudaStream_t s) {
+  const size_t staged = MmrSmem(N, (size_t)N * d * sizeof(T)).bytes;
+  const T* Vt = reinterpret_cast<const T*>(V);
+  if (staged <= kMmrStageMax)
+    return rt_launch<recommend_mmr_kernel<T, true>>((unsigned)B, staged, kMmrStageMax, s, Vt, nI, d, pool_ids,
+                                                     pool_scores, N, K, a, c, out_ids, out_scores, err);
+  return rt_launch<recommend_mmr_kernel<T, false>>((unsigned)B, MmrSmem(N, 0).bytes, MmrSmem(kMmrMaxN, 0).bytes, s, Vt,
+                                                    nI, d, pool_ids, pool_scores, N, K, a, c, out_ids, out_scores, err);
+}
+
+}  // namespace
+
+extern "C" int yr_recommend_mmr(const void* V, int64_t nI, int d, int dtype, const int64_t* pool_ids,
+                                const float* pool_scores, int64_t B, int N, int K, float lam, float one_minus_lam,
+                                int64_t* out_ids, float* out_scores, int32_t* err, yr_stream stream) {
+  if (!V || !out_ids || !out_scores || (B > 0 && (!pool_ids || !pool_scores))) return YR_ERR_BAD_ARG;
+  if (B < 0 || B >= 0x7fffffffLL || N < 1 || N > kMmrMaxN || K < 1 || K > N) return YR_ERR_BAD_ARG;
+  if (!(lam >= 0.f && lam <= 1.f) || !(one_minus_lam >= 0.f && one_minus_lam <= 1.f)) return YR_ERR_BAD_ARG;
+  if (nI <= 0 || nI >= 0x7fffffffLL || d <= 0 || d > kRtMaxD || (d & 7) != 0) return YR_ERR_BAD_DIM;
+  if (dtype != YR_DTYPE_F32 && dtype != YR_DTYPE_BF16) return YR_ERR_BAD_ARG;
+  if (B == 0) return YR_OK;
+  cudaStream_t s = (cudaStream_t)stream;
+  if (dtype == YR_DTYPE_F32)
+    return mmr_launch<float>(V, nI, d, pool_ids, pool_scores, B, N, K, lam, one_minus_lam, out_ids, out_scores, err, s);
+  return mmr_launch<__nv_bfloat16>(V, nI, d, pool_ids, pool_scores, B, N, K, lam, one_minus_lam, out_ids, out_scores,
+                                   err, s);
 }

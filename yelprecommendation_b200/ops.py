@@ -825,3 +825,69 @@ def recommend_geo_topk(U: torch.Tensor, V: torch.Tensor, user_ids: torch.Tensor,
     if e & 2:
         raise ValueError(f"{what}: a centre is not finite or a threshold is NaN or +inf")
     return ids, scores
+
+
+RECOMMEND_MMR_MAX_POOL = 1024
+
+
+def mmr_weights(lam) -> Tuple[float, float]:
+    """(a, c) of a diversity re-ranking with trade-off lam in [0, 1]: a = fp32(lam), c = fp32(1 - a) computed in fp32.
+    The one place both weights are made, for the kernel and the reference alike."""
+    if isinstance(lam, bool) or not isinstance(lam, (int, float, np.floating, np.integer)) or not 0.0 <= float(lam) <= 1.0:
+        raise ValueError(f"recommend_mmr: lam must be a number in [0, 1], got {lam}")
+    a = np.float32(lam)
+    return float(a), float(np.float32(1.0) - a)
+
+
+def mmr_sizes(what: str, K, N: int) -> int:
+    """K checked against a pool of N (1 <= K <= N <= RECOMMEND_MMR_MAX_POOL)."""
+    if not 1 <= N <= RECOMMEND_MMR_MAX_POOL:
+        raise ValueError(f"{what}: the pool must hold 1 to {RECOMMEND_MMR_MAX_POOL} entries a row, got {N}")
+    if isinstance(K, bool) or int(K) != K or not 1 <= int(K) <= N:
+        raise ValueError(f"{what}: k must be an integer in [1, {N}] (the pool size), got {K}")
+    return int(K)
+
+
+def recommend_mmr(V: torch.Tensor, pool_ids: torch.Tensor, pool_scores: torch.Tensor, K: int,
+                  lam: float) -> Tuple[torch.Tensor, torch.Tensor]:
+    """yr_recommend_mmr: diversity re-ranking (Maximal Marginal Relevance) of each row's pool (ids int64 [B x N], -1 =
+    empty; scores float32 [B x N], e.g. recommend_topk's output with K = N). Step t picks the unpicked entry with the
+    largest lam * score - (1 - lam) * (its largest cosine similarity in V to the entries already picked), ties to the
+    earlier entry. (ids int64 [B x K], scores float32 [B x K]) in pick order, the scores the pool's; rows that run out of
+    entries are padded with -1 / -inf. V: the item table [nI x d] (fp32 or bf16) the similarity is measured in. A pool id
+    outside [-1, nI) raises IndexError (after the launch, from the error word)."""
+    what = "recommend_mmr"
+    if not (torch.is_tensor(V) and torch.is_tensor(pool_ids) and torch.is_tensor(pool_scores)):
+        raise TypeError(f"{what}: V, pool_ids and pool_scores must be tensors")
+    if not (V.is_cuda and pool_ids.is_cuda and pool_scores.is_cuda):
+        raise YelprecError(f"{what}: V, pool_ids and pool_scores must be CUDA tensors (the reference path is "
+                           "retrieval.mmr_reference)")
+    dev = V.device
+    if pool_ids.device != dev or pool_scores.device != dev:
+        raise ValueError(f"{what}: tensors on different devices ({V.device}, {pool_ids.device}, {pool_scores.device})")
+    if V.dtype not in _RT_DTYPES or V.dim() != 2:
+        raise TypeError(f"{what}: V must be a float32 or bfloat16 [nI x d] table, got {V.dtype} {tuple(V.shape)}")
+    nI, d = int(V.shape[0]), int(V.shape[1])
+    if d % 8 != 0 or d > RECOMMEND_MAX_D:
+        raise ValueError(f"{what}: embedding width {d} must be a multiple of 8 and at most {RECOMMEND_MAX_D}")
+    if nI == 0 or nI >= 2 ** 31 - 1:
+        raise ValueError(f"{what}: {nI} items is not a valid catalog")
+    if pool_ids.dtype != I64 or pool_scores.dtype != F32 or pool_ids.dim() != 2 or \
+            pool_scores.shape != pool_ids.shape:
+        raise TypeError(f"{what}: pool_ids int64 [B x N] and pool_scores float32 [B x N] expected, got "
+                        f"{pool_ids.dtype} {tuple(pool_ids.shape)} and {pool_scores.dtype} {tuple(pool_scores.shape)}")
+    B, N = int(pool_ids.shape[0]), int(pool_ids.shape[1])
+    K = mmr_sizes(what, K, N)
+    a, c = mmr_weights(lam)
+    ids = torch.empty(B, K, device=dev, dtype=I64)
+    scores = torch.empty(B, K, device=dev, dtype=F32)
+    if B == 0:
+        return ids, scores
+    lib = _cabi.load()
+    Vc, pid, psc = V.detach().contiguous(), pool_ids.contiguous(), pool_scores.contiguous()
+    err = torch.zeros(1, device=dev, dtype=I32)
+    check(lib.yr_recommend_mmr(Vc.data_ptr(), nI, d, _RT_DTYPES[V.dtype], dptr(pid, I64), dptr(psc, F32), B, N, K, a, c,
+                               dptr(ids), dptr(scores), dptr(err), stream_ptr(dev)), "yr_recommend_mmr")
+    if int(err.item()) != 0:
+        raise IndexError(f"{what}: pool id out of range [-1, {nI})")
+    return ids, scores

@@ -34,6 +34,17 @@ product and sum rounded on its own, with p = ItemLocations.P[i], c the centre's 
 EARTH_RADIUS_KM) (-inf from half the Earth's circumference on), all computed on the host by geo_query. The kernel reads
 only the items of the grid cells around each centre; ids and scores equal what the unrestricted kernel returns with every
 item outside the radius excluded.
+
+    ids, scores = rec.recommend_diverse(user_ids, k=20, lam=0.5)   # same contract, a diverse list (CDAE too)
+
+recommend_diverse re-ranks a pool of the `pool` best items (recommend(user_ids, pool, ...), default min(1024, 4 k), with
+every restriction recommend takes) by Maximal Marginal Relevance: step t picks the pool entry with the largest
+a * score - c * (its largest cosine similarity to the items already picked), a = fp32(lam), c = fp32(1 - a), ties to the
+earlier entry (the higher score, then the lower id). Similarity is measured in the item table (item_emb; a CDAE's output
+layer rows W_o). The list comes back in pick order with the model's scores; lam = 1 returns recommend(user_ids, k) bit
+for bit. On CUDA tables the re-ranking is one kernel (yr_recommend_mmr: a block a row, no B x N x N similarity); on CPU
+tables, and as its oracle, `mmr_reference`, the plain PyTorch restatement (dense similarity, a k-step loop). The exact
+definition is in include/yelprec_b200.h.
 """
 from __future__ import annotations
 
@@ -342,6 +353,84 @@ def recommend_reference(user_emb: torch.Tensor, item_emb: torch.Tensor, user_ids
     return ids, out
 
 
+def _pool_size(k, pool) -> int:
+    """The pool a diverse list of k is re-ranked from: min(1024, 4 k) by default, else pool in [k, 1024]."""
+    k = _check_k(k)
+    N = min(ops.RECOMMEND_MMR_MAX_POOL, 4 * k) if pool is None else pool
+    if isinstance(N, bool) or int(N) != N or not k <= int(N) <= ops.RECOMMEND_MMR_MAX_POOL:
+        raise ValueError(f"recommend_diverse: pool must be an integer in [k, {ops.RECOMMEND_MMR_MAX_POOL}] = "
+                         f"[{k}, {ops.RECOMMEND_MMR_MAX_POOL}], got {pool}")
+    return int(N)
+
+
+def _order_key(m: torch.Tensor) -> torch.Tensor:
+    """int64 keys of fp32 values that order as the values do (rt_key's mapping of the float's bits)."""
+    u = m.contiguous().view(torch.int32).to(I64) & 0xffffffff
+    return torch.where(u >= 2 ** 31, (~u) & 0xffffffff, u | 2 ** 31)
+
+
+def mmr_reference(item_emb: torch.Tensor, pool_ids, pool_scores, k: int, lam: float) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Plain PyTorch on item_emb's device: Maximal Marginal Relevance re-ranking of each row's pool (ids int64 [B x N],
+    -1 = empty; scores float32 [B x N]) into k picks, the definition of yr_recommend_mmr (include/yelprec_b200.h) as
+    separate fp32 elementwise ops: the pool rows gathered [B x N x d], n = 1 / sqrt(sum of squares) (0 for a zero row), the
+    dense similarity (X X^T) * (n n^T) [B x N x N], then k steps of m = (a * r) - (c * pen) with a, c = ops.mmr_weights(lam),
+    pen = 0 before the first pick and the running maximum of the picked columns after it. (ids int64 [B x k], scores
+    float32 [B x k]) in pick order, padded with -1 / -inf."""
+    what = "mmr_reference"
+    dev = item_emb.device
+    ids = torch.as_tensor(pool_ids).to(device=dev, dtype=I64)
+    r = torch.as_tensor(pool_scores).to(device=dev, dtype=F32)
+    if ids.dim() != 2 or r.shape != ids.shape:
+        raise ValueError(f"{what}: pool_ids and pool_scores must both be [B x N], got {tuple(ids.shape)} and "
+                         f"{tuple(r.shape)}")
+    B, N = ids.shape
+    k = ops.mmr_sizes(what, k, N)
+    a, c = ops.mmr_weights(lam)
+    nI = item_emb.shape[0]
+    if ids.numel() and (int(ids.min()) < -1 or int(ids.max()) >= nI):
+        raise IndexError(f"{what}: pool id out of range [-1, {nI})")
+    valid = ids >= 0
+    X = item_emb.detach().to(F32)[ids.clamp(min=0)]
+    X = torch.where(valid[..., None], X, torch.zeros((), dtype=F32, device=dev))
+    ss = (X * X).sum(-1)
+    nrm = torch.where(ss == 0, torch.zeros_like(ss), torch.reciprocal(torch.sqrt(ss)))
+    sim = torch.bmm(X, X.transpose(1, 2)) * (nrm[:, :, None] * nrm[:, None, :])
+    ar = torch.tensor(a, dtype=F32, device=dev) * r
+    ct = torch.tensor(c, dtype=F32, device=dev)
+    pen = torch.zeros(B, N, dtype=F32, device=dev)
+    avail = valid.clone()
+    out_ids = torch.full((B, k), -1, dtype=I64, device=dev)
+    out_sc = torch.full((B, k), float("-inf"), dtype=F32, device=dev)
+    rows, pos = torch.arange(B, device=dev), torch.arange(N, device=dev)
+    for t in range(k):
+        m = ar - ct * pen
+        m = torch.where(m == 0, torch.zeros_like(m), m)
+        m = torch.where(torch.isnan(m), torch.full_like(m, float("-inf")), m)
+        key = torch.where(avail, _order_key(m) * 2048 + (2047 - pos), torch.full_like(ids, -1))
+        best = key.max(1).values if N else torch.full((B,), -1, dtype=I64, device=dev)
+        has = best >= 0
+        s = torch.where(has, 2047 - best % 2048, torch.zeros_like(best))
+        out_ids[has, t] = ids[rows, s][has]
+        out_sc[has, t] = r[rows, s][has]
+        avail[rows[has], s[has]] = False
+        col = sim[rows, :, s]
+        pen = col if t == 0 else torch.maximum(pen, col)
+    return out_ids, out_sc
+
+
+def recommend_diverse_reference(user_emb: torch.Tensor, item_emb: torch.Tensor, user_ids, k: int, lam: float = 0.5,
+                                pool: Optional[int] = None, seen: Optional[SeenItems] = None,
+                                subsets: Optional[ItemSubsets] = None, subset=None,
+                                locations: Optional[ItemLocations] = None, near=None,
+                                radius_km=None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Recommender.recommend_diverse restated: recommend_reference(..., pool) followed by mmr_reference over item_emb."""
+    N = _pool_size(k, pool)
+    ops.mmr_weights(lam)
+    ids, sc = recommend_reference(user_emb, item_emb, user_ids, N, seen, subsets, subset, locations=locations,
+                                  near=near, radius_km=radius_km)
+    return mmr_reference(item_emb, ids, sc, k, lam)
+
+
 class Recommender:
     """Top-K retrieval over fixed user / item tables ([num_users x d], [num_items x d], fp32 or bf16, same device),
     optionally restricted per request to one of the item subsets or to the items within a radius (locations)."""
@@ -384,6 +473,20 @@ class Recommender:
         ptr, idx = seen.on(dev) if seen is not None else (None, None)
         return _recommend_kernel(self.user_emb, self.item_emb, uid, k, ptr, idx, self.subsets, subset,
                                  locations=self.locations, near=near, radius_km=radius_km)
+
+    def recommend_diverse(self, user_ids, k: int, lam: float = 0.5, pool: Optional[int] = None,
+                          exclude_seen: bool = True, subset=None, near=None,
+                          radius_km=None) -> Tuple[torch.Tensor, torch.Tensor]:
+        """recommend's contract for a diverse list: the `pool` best items (default min(1024, 4 k)) of
+        recommend(user_ids, pool, exclude_seen, subset, near, radius_km), re-ranked by Maximal Marginal Relevance with
+        trade-off lam in [0, 1] (1: pure relevance, 0: pure novelty), similarity measured in item_emb. (item ids int64
+        [B x k], scores float32 [B x k]) in pick order; see the module docstring."""
+        N = _pool_size(k, pool)
+        ops.mmr_weights(lam)
+        ids, sc = self.recommend(user_ids, N, exclude_seen, subset, near, radius_km)
+        if self.item_emb.device.type != "cuda":
+            return mmr_reference(self.item_emb, ids, sc, k, lam)
+        return ops.recommend_mmr(self.item_emb, ids, sc, k, lam)
 
 
 def _recommend_kernel(U, V, uid, k, seen_ptr, seen_idx, subsets: Optional[ItemSubsets], subset, item_bias=None,
@@ -447,6 +550,20 @@ def cdae_recommend_reference(model, user_ids, k: int, seen: SeenItems, exclude_s
                                radius_km=radius_km)
 
 
+def cdae_recommend_diverse_reference(model, user_ids, k: int, seen: SeenItems, lam: float = 0.5,
+                                     pool: Optional[int] = None, exclude_seen: bool = True,
+                                     subsets: Optional[ItemSubsets] = None, subset=None,
+                                     locations: Optional[ItemLocations] = None, near=None,
+                                     radius_km=None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """CDAERecommender.recommend_diverse restated: cdae_recommend_reference(..., pool) followed by mmr_reference over the
+    output layer's rows W_o."""
+    N = _pool_size(k, pool)
+    ops.mmr_weights(lam)
+    ids, sc = cdae_recommend_reference(model, user_ids, N, seen, exclude_seen, subsets, subset, locations, near,
+                                       radius_km)
+    return mmr_reference(model.output_layer.weight.data, ids, sc, k, lam)
+
+
 def _batch_lists(seen: SeenItems, uid: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
     """(ptr int32 [B + 1], idx int32): seen[uid[b]] for every batch row b, a CSR indexed by the batch row (uid's device)."""
     dev = uid.device
@@ -465,7 +582,8 @@ class CDAERecommender:
 
     recommend(user_ids, k, exclude_seen=True, subset=None, near=None, radius_km=None) has Recommender.recommend's
     contract: (item ids int64 [B x k], scores float32 [B x k]), best first, ties to the lower id, short rows padded with
-    -1 / -inf, the same subset and radius semantics.
+    -1 / -inf, the same subset and radius semantics. recommend_diverse has Recommender.recommend_diverse's, with
+    similarity measured in the output layer's rows W_o.
     The scores are logits, the values CDAETrainer.evaluate ranks by; sigmoid(score) is the model's predicted probability.
     """
 
@@ -503,3 +621,13 @@ class CDAERecommender:
         return _recommend_kernel(z, m.output_layer.weight.data, rows, k, bptr, bidx, self.subsets, subset,
                                  item_bias=m.output_layer.bias.data, locations=self.locations, near=near,
                                  radius_km=radius_km)
+
+    def recommend_diverse(self, user_ids, k: int, lam: float = 0.5, pool: Optional[int] = None,
+                          exclude_seen: bool = True, subset=None, near=None,
+                          radius_km=None) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Recommender.recommend_diverse for the CDAE: the pool from recommend, re-ranked with similarity measured in the
+        output layer's rows W_o (the item vectors the logits are dot products with)."""
+        N = _pool_size(k, pool)
+        ops.mmr_weights(lam)
+        ids, sc = self.recommend(user_ids, N, exclude_seen, subset, near, radius_km)
+        return ops.recommend_mmr(self.model.output_layer.weight.data, ids, sc, k, lam)

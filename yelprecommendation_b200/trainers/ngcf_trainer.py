@@ -271,7 +271,8 @@ class NGCFTrainer(BaseTrainer):
         return result
 
     def recommender(self, seen=None, subsets=None, locations=None):
-        """retrieval.Recommender over the propagated, layer-concatenated user / item embeddings that evaluate() ranks with."""
+        """retrieval.Recommender over the propagated, layer-concatenated user / item embeddings that evaluate() ranks with;
+        recommend_diverse measures similarity in the concatenated item rows."""
         from ..retrieval import Recommender
         cat = ops.ngcf_concat(self.propagate()[0])
         return Recommender(cat[: self.num_users], cat[self.num_users:], seen, subsets, locations)
