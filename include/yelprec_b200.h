@@ -655,6 +655,35 @@ int yr_recommend_mmr(const void* V, int64_t nI, int d, int dtype, const int64_t*
                      int64_t B, int N, int K, float lam, float one_minus_lam, int64_t* out_ids, float* out_scores,
                      int32_t* err, yr_stream stream);
 
+/* Group retrieval: one ranked list for each of G groups of users. Group g has the m_g members
+ * members[group_ptr[g] .. group_ptr[g + 1]) (rows of U), 1 <= m_g <= YR_GROUP_MAX_MEMBERS; the caller lists them in
+ * ascending order without duplicates (retrieval.UserGroups does). For item i, s_j(i) is exactly the score
+ * yr_recommend_topk_ex gives member j (one fp32 fma chain, k ascending, then + item_bias[i] if item_bias is not NULL),
+ * and the group's score is
+ *   agg = YR_GROUP_MIN (least misery): a(i) = min_j s_j(i), NaN if any s_j(i) is NaN;
+ *   agg = YR_GROUP_MEAN: S = (((s_1 + s_2) + s_3) + ...) in member order, each add rounded on its own, then
+ *                        a(i) = S / m_g, one correctly rounded division.
+ * An item in the seen list of any member (seen_ptr / seen_idx indexed by the member's row of U; both NULL = none) is
+ * never returned; nor is an item scoring -inf or NaN. Ranking, ties and padding as yr_recommend_topk: out_ids /
+ * out_scores [G x K] by (a desc, id asc), short rows padded with id -1 / score -inf, rows in request order. A group of
+ * one member u gets exactly yr_recommend_topk_ex's row for u. subset_ids (NULL = every group ranks the whole catalog)
+ * restricts group g to subset subset_ids[g] of the subset CSR (subset_ptr [num_subsets + 1], subset_idx), -1 = the
+ * whole catalog, as yr_recommend_subset_topk (max_subset_len as there; with subset_ids NULL it is not read). No buffer
+ * of G x nI scores is made. num_members: the length of members. A member outside [0, nU) sets *err |= 1, a subset id
+ * outside [-1, num_subsets) *err |= 2, a group size outside [1, YR_GROUP_MAX_MEMBERS] (or a group_ptr range outside
+ * members) *err |= 4; each such row is all padding. G < 2^31 - 1; the other limits as yr_recommend_subset_topk.
+ * ws: yr_recommend_group_ws_bytes(G, num_subsets, max_subset_len, K) bytes (per-split lists and, with subset_ids, the
+ * row grouping; same device); without subset_ids pass num_subsets = 0 and max_subset_len = nI. */
+#define YR_GROUP_MAX_MEMBERS 32
+enum yr_group_agg { YR_GROUP_MIN = 0, YR_GROUP_MEAN = 1 };
+size_t yr_recommend_group_ws_bytes(int64_t G, int num_subsets, int64_t max_subset_len, int K);
+int yr_recommend_group_topk(const void* U, int64_t nU, const void* V, int64_t nI, int d, int dtype,
+                            const int32_t* group_ptr, int64_t G, const int64_t* members, int64_t num_members, int agg,
+                            const int32_t* subset_ptr, const int32_t* subset_idx, int num_subsets,
+                            int64_t max_subset_len, const int64_t* subset_ids, const int32_t* seen_ptr,
+                            const int32_t* seen_idx, int K, int64_t* out_ids, float* out_scores, void* ws,
+                            size_t ws_bytes, int32_t* err, yr_stream stream, const float* item_bias);
+
 #ifdef __cplusplus
 }
 #endif

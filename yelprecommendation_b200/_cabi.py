@@ -36,10 +36,13 @@ SYMBOLS = (
     "yr_recommend_ws_bytes", "yr_recommend_topk", "yr_recommend_subset_ws_bytes", "yr_recommend_subset_topk",
     "yr_recommend_topk_ex", "yr_recommend_subset_topk_ex", "yr_cdae_encode",
     "yr_recommend_geo_ws_bytes", "yr_recommend_geo_topk", "yr_recommend_mmr",
+    "yr_recommend_group_ws_bytes", "yr_recommend_group_topk",
 )
 
 YR_OPT_SGD, YR_OPT_ADAM, YR_OPT_ADAMW = 0, 1, 2
 YR_DTYPE_F32, YR_DTYPE_BF16 = 0, 1
+YR_GROUP_MIN, YR_GROUP_MEAN = 0, 1
+YR_GROUP_MAX_MEMBERS = 32
 # yr_dense_mode: where the NGCF d x d transforms run (per call / per trainer state)
 YR_DENSE_FP32, YR_DENSE_TC_FWD, YR_DENSE_TC = 0, 1, 2
 OPT_KINDS = {"sgd": YR_OPT_SGD, "adam": YR_OPT_ADAM, "adamw": YR_OPT_ADAMW}
@@ -214,6 +217,9 @@ def load() -> C.CDLL:
         "yr_recommend_geo_topk": (C.c_int, [p, i64, p, i64, i32, i32, p, i64, p, p, i64, p, p, C.c_double, i64, i64, p,
                                             p, p, p, i32, p, p, p, sz, p, p, p]),
         "yr_recommend_mmr": (C.c_int, [p, i64, i32, i32, p, p, i64, i32, i32, f32, f32, p, p, p, p]),
+        "yr_recommend_group_ws_bytes": (sz, [i64, i32, i64, i32]),
+        "yr_recommend_group_topk": (C.c_int, [p, i64, p, i64, i32, i32, p, i64, p, i64, i32, p, p, i32, i64, p, p, p,
+                                              i32, p, p, p, sz, p, p, p]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)

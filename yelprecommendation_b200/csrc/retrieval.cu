@@ -1034,6 +1034,197 @@ recommend_mmr_kernel(const T* __restrict__ V, int64_t nI, int d, const int64_t* 
   }
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// Group retrieval. Row g is a group of m_g users, members[group_ptr[g] .. group_ptr[g + 1]) (1 <= m_g <= 32); item i
+// scores the aggregate of the members' scores s_j(i) (each exactly recommend's: the fma chain, then the bias):
+// min_j s_j(i) (NaN if any is NaN) or (((s_1 + s_2) + s_3) + ...) / m_g, every add and the division rounded on their
+// own. Items in any member's seen list are excluded. Rows may be restricted to a subset as in recommend_subset_kernel
+// (plan buckets keyed by subset id); without subset ids every row streams the whole catalog and no plan is made.
+// ---------------------------------------------------------------------------------------------------------------------
+constexpr int kGrMaxMembers = 32;
+
+struct GrSmem {   // recommend_group_kernel; keys [TG][kRtEntries / TG] at 0
+  size_t thr, Us, bits, cnt, rowb, mbeg, mnum, cur, cend, sid, bytes;
+  __host__ __device__ GrSmem(int TG, int d)
+      : thr((size_t)kRtEntries * 8), Us(thr + (size_t)TG * 8), bits(Us + (size_t)TG * d * 4),
+        cnt(bits + (size_t)TG * (kRtTile / 32) * 4), rowb(cnt + (size_t)TG * 4), mbeg(rowb + (size_t)TG * 4),
+        mnum(mbeg + (size_t)TG * 4), cur(mnum + (size_t)TG * 4), cend(cur + (size_t)TG * kGrMaxMembers * 4),
+        sid(cend + (size_t)TG * kGrMaxMembers * 4), bytes(sid + (size_t)kRtTile * 4) {}
+};
+
+// One warp: the entries of the ascending list seen_idx[c, en) up to the tile's last id, each found among the tile's n
+// ascending ids sid and ORed into bits (by tile position); returns the cursor past them.
+__device__ __forceinline__ int gr_mark_seen(uint32_t* bits, const int* sid, int n, const int32_t* __restrict__ seen_idx,
+                                            int c, int en, int lane) {
+  const int last = sid[n - 1];
+  while (c < en) {
+    const int p = c + lane;
+    const int it = (p < en) ? seen_idx[p] : INT32_MAX;
+    const bool in = it <= last;
+    if (in) {
+      int l = 0, h = n;
+      while (l < h) {
+        const int mid = (l + h) >> 1;
+        if (sid[mid] < it) l = mid + 1; else h = mid;
+      }
+      if (l < n && sid[l] == it) atomicOr(bits + (l >> 5), 1u << (l & 31));
+    }
+    const int m = __popc(__ballot_sync(kFull, in));
+    c += m;
+    if (m < 32) break;
+  }
+  return c;
+}
+
+// Grid (blocks, S). Block x takes up to TG groups (of one plan bucket, or groups x * TG .. without a plan) and split y
+// of their list, sliced as in recommend_subset_kernel. Each tile of 256 ids takes one pass per member position j: the
+// j-th member of every group is staged into Us, scored by the fma chain of rt_score and folded into agg; the pass also
+// marks member j's seen entries of the tile in its group's bitmask (one ascending cursor per group and member). After the
+// last pass agg is offered like any score.
+template <typename T, int TG, bool kBias>
+__global__ void __launch_bounds__(kRtThreads, 2)   // 2 blocks an SM: up to 128 registers, no spills
+recommend_group_kernel(const T* __restrict__ U, int64_t nU, const T* __restrict__ V, int64_t nI, int d,
+                       const int32_t* __restrict__ group_ptr, int64_t Gn, const int64_t* __restrict__ members,
+                       int64_t num_members, int mean, const int32_t* __restrict__ sub_ptr,
+                       const int32_t* __restrict__ sub_idx, int NS, const int32_t* __restrict__ rows_at,
+                       const int32_t* __restrict__ blocks_at, const int32_t* __restrict__ order,
+                       const int32_t* __restrict__ seen_ptr, const int32_t* __restrict__ seen_idx, int K, int S,
+                       uint64_t* __restrict__ partial, int64_t* __restrict__ out_ids, float* __restrict__ out_scores,
+                       int32_t* err, const float* __restrict__ item_bias) {
+  constexpr int CAP = kRtEntries / TG;
+  constexpr int kWords = kRtTile / 32;
+  extern __shared__ __align__(16) uint64_t rt_smem[];
+  const GrSmem lay(TG, d);
+  uint64_t* keys = rt_smem;                                    // [TG][CAP]
+  uint64_t* thr = rt_at<uint64_t>(rt_smem, lay.thr);           // [TG]; ~0 = inactive row (no candidate beats it)
+  float* Us = rt_at<float>(rt_smem, lay.Us);                   // [TG][d]: member j of each group during pass j
+  uint32_t* bits = rt_at<uint32_t>(rt_smem, lay.bits);         // [TG][kWords]: the group's seen items of the tile
+  int* cnt = rt_at<int>(rt_smem, lay.cnt);                     // [TG]
+  int* rowb = rt_at<int>(rt_smem, lay.rowb);                   // [TG]: the group's row, -1 = none
+  int* mbeg = rt_at<int>(rt_smem, lay.mbeg);                   // [TG]: its first entry of members
+  int* mnum = rt_at<int>(rt_smem, lay.mnum);                   // [TG]: its member count, 0 = inactive
+  int* cur = rt_at<int>(rt_smem, lay.cur);                     // [TG][32]: next unconsumed entry of each seen list
+  int* cend = rt_at<int>(rt_smem, lay.cend);                   // [TG][32]
+  int* sid = rt_at<int>(rt_smem, lay.sid);                     // [kRtTile]: item ids of the tile, ascending
+
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int blk = blockIdx.x, split = blockIdx.y;
+  int bk = NS, r0 = blk * TG, nr = (int)min((int64_t)TG, Gn - r0);   // no plan: every row streams the whole catalog
+  if (order && !rs_block_rows<TG>(blocks_at, rows_at, NS + 2, blk, bk, r0, nr)) return;
+  const int32_t* list = bk < NS ? sub_idx + sub_ptr[bk] : nullptr;   // null: the identity (whole catalog)
+  const int64_t len = bk < NS ? sub_ptr[bk + 1] - sub_ptr[bk] : bk == NS ? nI : 0;
+  int64_t per = max((len + S - 1) / S, (int64_t)kRtMinSplit);
+  per = (per + kRtTile - 1) / kRtTile * kRtTile;
+  const int64_t pb = min(len, (int64_t)split * per);
+  const int64_t pe = min(len, pb + per);
+
+  if (tid < TG) {
+    int b = -1, m0 = 0, m = 0;
+    if (tid < nr) {
+      b = order ? order[r0 + tid] : r0 + tid;
+      m0 = group_ptr[b];
+      m = group_ptr[b + 1] - m0;
+      if (m < 1 || m > kGrMaxMembers || m0 < 0 || m0 + m > num_members) {
+        if (err) atomicOr(err, 4);
+        m = 0;
+      }
+    }
+    rowb[tid] = b; mbeg[tid] = m0; mnum[tid] = m;
+    thr[tid] = m ? 0ull : ~0ull;
+    cnt[tid] = 0;
+  }
+  __syncthreads();
+  // every member in range, and its seen cursor at the split's first id (lists ascending)
+  for (int i = tid; i < TG * kGrMaxMembers; i += kRtThreads) {
+    const int u = i / kGrMaxMembers, j = i - u * kGrMaxMembers;
+    int c = 0, en = 0;
+    if (j < mnum[u]) {
+      const int64_t uid = members[mbeg[u] + j];
+      if (uid < 0 || uid >= nU) {
+        if (err) atomicOr(err, 1);
+        thr[u] = ~0ull;
+      } else if (seen_ptr && pb < pe) {
+        c = seen_ptr[uid]; en = seen_ptr[uid + 1];
+        const int64_t first = list ? list[pb] : pb;
+        int l = c, h = en;
+        while (l < h) {
+          const int mid = (l + h) >> 1;
+          if (seen_idx[mid] < first) l = mid + 1; else h = mid;
+        }
+        c = l;
+      }
+    }
+    cur[i] = c; cend[i] = en;
+  }
+  __syncthreads();
+  if (tid < TG && thr[tid] != 0ull) mnum[tid] = 0;             // a member out of range: the row is all padding
+  __syncthreads();
+  int passes = 0;
+#pragma unroll
+  for (int u = 0; u < TG; ++u) passes = max(passes, mnum[u]);
+
+  if (pb < pe && passes > 0) {
+    for (int64_t p0 = pb; p0 < pe; p0 += kRtTile) {
+      const int n = (int)min((int64_t)kRtTile, pe - p0);
+      for (int i = tid; i < TG * kWords; i += kRtThreads) bits[i] = 0;
+      if (tid < n) sid[tid] = list ? list[p0 + tid] : (int)(p0 + tid);
+      const bool have = tid < n;
+      float agg[TG];
+      for (int j = 0; j < passes; ++j) {
+        __syncthreads();   // tile ids and bitmask ready (j = 0), the last pass's users consumed (j > 0)
+        rt_stage_users<T, TG>(Us, U, d, [&](int u, int64_t& uid) {
+          if (j >= mnum[u]) return false;
+          uid = members[mbeg[u] + j];
+          return true;
+        });
+        // ---- member j's seen items of this tile -> the group's bitmask (one warp per group) ----
+        if (seen_ptr) {
+          for (int u = warp; u < TG; u += kRtThreads / 32) {
+            if (j >= mnum[u]) continue;
+            const int c = gr_mark_seen(bits + u * kWords, sid, n, seen_idx, cur[u * kGrMaxMembers + j],
+                                       cend[u * kGrMaxMembers + j], lane);
+            if (lane == 0) cur[u * kGrMaxMembers + j] = c;
+          }
+        }
+        __syncthreads();   // member j staged
+        // ---- member j's score of my item in every group: one fma chain each, k ascending, then the fold ----
+        const int item = have ? sid[tid] : 0;
+        float acc[TG];
+        rt_score<T, TG>(have ? V + (int64_t)item * d : nullptr, Us, d, acc);
+        float bias = 0.f;
+        if constexpr (kBias) bias = have ? __ldg(item_bias + item) : 0.f;
+#pragma unroll
+        for (int u = 0; u < TG; ++u) {
+          const float s = kBias ? acc[u] + bias : acc[u];
+          if (j == 0) agg[u] = s;
+          else if (j < mnum[u]) {
+            if (mean) agg[u] = __fadd_rn(agg[u], s);
+            else if (s < agg[u] || s != s) agg[u] = s;   // min; a NaN, once in, stays
+          }
+        }
+      }
+      if (have) {
+        const int item = sid[tid];
+#pragma unroll
+        for (int u = 0; u < TG; ++u) {
+          if (seen_ptr && ((bits[u * kWords + warp] >> lane) & 1u)) continue;
+          rt_offer<TG>(keys, cnt, thr, u, mean ? __fdiv_rn(agg[u], (float)mnum[u]) : agg[u], (uint32_t)item);
+        }
+      }
+      __syncthreads();
+      bool full = p0 + kRtTile >= pe;              // the last tile: truncate to the K best
+#pragma unroll
+      for (int u = 0; u < TG; ++u) full |= cnt[u] > CAP - kRtTile;   // the next tile could overflow a buffer
+      if (full) rt_compact<TG>(keys, cnt, thr, K);
+    }
+  }
+
+  // every buffer that took an offer was truncated after the split's last tile: its first cnt keys are its K best
+  rt_write_rows<TG, int>(
+      K, split, Gn, partial, out_ids, out_scores, [&](int u, int& b) { b = rowb[u]; return b >= 0; },
+      [&](int u, int j) { return j < cnt[u] ? keys[(size_t)u * CAP + j] : 0; });   // zero beyond the count: padding
+}
+
 }  // namespace yr
 
 using namespace yr;
@@ -1337,4 +1528,55 @@ extern "C" int yr_recommend_mmr(const void* V, int64_t nI, int d, int dtype, con
     return mmr_launch<float>(V, nI, d, pool_ids, pool_scores, B, N, K, lam, one_minus_lam, out_ids, out_scores, err, s);
   return mmr_launch<__nv_bfloat16>(V, nI, d, pool_ids, pool_scores, B, N, K, lam, one_minus_lam, out_ids, out_scores,
                                    err, s);
+}
+
+extern "C" size_t yr_recommend_group_ws_bytes(int64_t G, int num_subsets, int64_t max_subset_len, int K) {
+  if (G <= 0 || num_subsets < 0 || K <= 0 || K > kRtMaxK) return 0;
+  return rs_partial_bytes(rs_splits(G, max_subset_len, K, rt_users_per_block(K)), G, K) + rs_plan_bytes(G, num_subsets);
+}
+
+extern "C" int yr_recommend_group_topk(const void* U, int64_t nU, const void* V, int64_t nI, int d, int dtype,
+                                       const int32_t* group_ptr, int64_t G, const int64_t* members,
+                                       int64_t num_members, int agg, const int32_t* subset_ptr,
+                                       const int32_t* subset_idx, int num_subsets, int64_t max_subset_len,
+                                       const int64_t* subset_ids, const int32_t* seen_ptr, const int32_t* seen_idx,
+                                       int K, int64_t* out_ids, float* out_scores, void* ws, size_t ws_bytes,
+                                       int32_t* err, yr_stream stream, const float* item_bias) {
+  if ((G > 0 && !group_ptr) || (subset_ids && (!subset_ptr || !subset_idx))) return YR_ERR_BAD_ARG;
+  if (agg != YR_GROUP_MIN && agg != YR_GROUP_MEAN) return YR_ERR_BAD_ARG;
+  if (G >= 0x7fffffffLL || num_members < 0 || num_members >= 0x7fffffffLL || num_subsets < 0 ||
+      num_subsets >= 0x7ffffff0 || max_subset_len < 0)
+    return YR_ERR_BAD_ARG;
+  if (int rc = rt_check(U, nU, V, nI, d, dtype, members, G, seen_ptr, seen_idx, K, out_ids, out_scores)) return rc;
+  if (G == 0) return YR_OK;
+  const int TG = rt_users(K, d);
+  const int NS = subset_ids ? num_subsets : 0;
+  const int S = rs_splits(G, subset_ids ? max_subset_len : nI, K, TG);
+  const size_t pbytes = rs_partial_bytes(S, G, K);
+  if ((pbytes || subset_ids) && (!ws || ws_bytes < pbytes + (subset_ids ? rs_plan_bytes(G, NS) : 0)))
+    return YR_ERR_WORKSPACE;
+  cudaStream_t s = (cudaStream_t)stream;
+  uint64_t* partial = S > 1 ? reinterpret_cast<uint64_t*>(ws) : nullptr;
+  const int32_t *rows_at = nullptr, *blocks_at = nullptr, *order = nullptr;
+  int64_t blocks = (G + TG - 1) / TG;
+  if (subset_ids) {   // plan buckets by subset id
+    const RsPlan plan(reinterpret_cast<char*>(ws) + pbytes, NS);
+    recommend_subset_plan_kernel<<<1, kRsPlanThreads, 0, s>>>(subset_ids, (int)G, NS, TG, plan.cursor, plan.rows_at,
+                                                              plan.blocks_at, plan.order, err);
+    YR_CHECK_LAUNCH();
+    rows_at = plan.rows_at; blocks_at = plan.blocks_at; order = plan.order;
+    blocks += std::min<int64_t>((int64_t)NS + 2, G);
+  }
+  const dim3 grid((unsigned)blocks, (unsigned)S);
+  const RtBytes<GrSmem> smem(TG, d);
+  const int rc = rt_dispatch(dtype, TG, item_bias != nullptr, [&](auto inst) {
+    using I = decltype(inst);
+    using T = typename I::T;
+    return rt_launch<recommend_group_kernel<T, I::TU, I::kBias>>(
+        grid, smem.bytes, smem.max, s, reinterpret_cast<const T*>(U), nU, reinterpret_cast<const T*>(V), nI, d,
+        group_ptr, G, members, num_members, agg == YR_GROUP_MEAN ? 1 : 0, subset_ptr, subset_idx, NS, rows_at,
+        blocks_at, order, seen_ptr, seen_idx, K, S, partial, out_ids, out_scores, err, item_bias);
+  });
+  if (rc || S == 1) return rc;
+  return merge_launch(partial, S, G, K, out_ids, out_scores, s);
 }

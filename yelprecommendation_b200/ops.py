@@ -891,3 +891,79 @@ def recommend_mmr(V: torch.Tensor, pool_ids: torch.Tensor, pool_scores: torch.Te
     if int(err.item()) != 0:
         raise IndexError(f"{what}: pool id out of range [-1, {nI})")
     return ids, scores
+
+
+RECOMMEND_GROUP_MAX_MEMBERS = _cabi.YR_GROUP_MAX_MEMBERS
+_GROUP_AGGS = {"min": _cabi.YR_GROUP_MIN, "mean": _cabi.YR_GROUP_MEAN}
+
+
+def group_agg(agg) -> int:
+    """The C ABI code of a group aggregation: "min" (least misery) or "mean"."""
+    if not isinstance(agg, str) or agg not in _GROUP_AGGS:
+        raise ValueError(f"recommend_group: agg must be 'min' or 'mean', got {agg!r}")
+    return _GROUP_AGGS[agg]
+
+
+def recommend_group_topk(U: torch.Tensor, V: torch.Tensor, group_ptr: torch.Tensor, members: torch.Tensor, K: int,
+                         agg: str, seen_ptr: Optional[torch.Tensor] = None, seen_idx: Optional[torch.Tensor] = None,
+                         subset_ptr: Optional[torch.Tensor] = None, subset_idx: Optional[torch.Tensor] = None,
+                         subset_ids: Optional[torch.Tensor] = None, max_len: Optional[int] = None,
+                         item_bias: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """yr_recommend_group_topk: (ids int64 [G x K], scores float32 [G x K]) of the K best items per group of users, group
+    g = members[group_ptr[g] .. group_ptr[g + 1]) (rows of U, 1 to RECOMMEND_GROUP_MAX_MEMBERS, ascending), by the
+    aggregate of the members' scores U[u] . V[i] (+ item_bias[i]): agg = "min" (least misery) or "mean" (summed in member
+    order, then divided by the member count). Items in any member's seen list (CSR int32 indexed by the row of U) are
+    never returned. subset_ids (int64 [G], -1 = whole catalog; None = every group ranks the whole catalog) restricts
+    group g to subset subset_ids[g] of the subset CSR, as recommend_subset_topk; max_len as there (None: num_items).
+    A member out of range raises IndexError, a subset id out of range IndexError and a group size outside
+    [1, RECOMMEND_GROUP_MAX_MEMBERS] ValueError, all after the launch, from the error word (one scalar read per call)."""
+    what = "recommend_group_topk"
+    if not (torch.is_tensor(group_ptr) and torch.is_tensor(members)):
+        raise TypeError(f"{what}: group_ptr and members must be tensors")
+    dev, d, nU, nI, K, M = _rt_tables(what, U, V, members, K)
+    code = group_agg(agg)
+    if group_ptr.dtype != I32 or group_ptr.dim() != 1 or group_ptr.numel() < 1:
+        raise ValueError(f"{what}: group_ptr must be int32 [G + 1]")
+    if members.dtype != I64 or group_ptr.device != dev:
+        raise ValueError(f"{what}: members must be int64 and group_ptr on the device of the embeddings")
+    G = int(group_ptr.numel()) - 1
+    if (subset_ids is None) != (subset_ptr is None) or (subset_ptr is None) != (subset_idx is None):
+        raise ValueError(f"{what}: subset_ptr, subset_idx and subset_ids go together")
+    NS, sptr, sidx, sid = 0, None, None, None
+    if subset_ids is not None:
+        if not (torch.is_tensor(subset_ptr) and torch.is_tensor(subset_idx) and torch.is_tensor(subset_ids)):
+            raise TypeError(f"{what}: subset_ptr, subset_idx and subset_ids must be tensors")
+        if subset_ids.dtype not in (I64, I32) or subset_ids.dim() != 1 or subset_ids.numel() != G:
+            raise ValueError(f"{what}: subset_ids must be a 1-D int64 or int32 tensor of {G} ids, got "
+                             f"{subset_ids.dtype} {tuple(subset_ids.shape)}")
+        if subset_ptr.dtype != I32 or subset_idx.dtype != I32 or subset_ptr.dim() != 1 or subset_ptr.numel() < 1:
+            raise ValueError(f"{what}: subsets must be an int32 CSR (subset_ptr [G + 1], subset_idx)")
+        if subset_ptr.device != dev or subset_idx.device != dev or subset_ids.device != dev:
+            raise ValueError(f"{what}: subsets and subset ids must live on the device of the embeddings")
+        NS = int(subset_ptr.numel()) - 1
+        sid, sptr = subset_ids.to(I64).contiguous(), subset_ptr.contiguous()
+        sidx = subset_idx.contiguous() if subset_idx.numel() else torch.zeros(1, dtype=I32, device=dev)
+    max_len = nI if max_len is None or subset_ids is None else max_len
+    if isinstance(max_len, bool) or int(max_len) != max_len or int(max_len) < 0:
+        raise ValueError(f"{what}: max_len must be a non-negative integer, got {max_len}")
+    seen_ptr, seen_idx, bias = _rt_seen_and_bias(what, seen_ptr, seen_idx, nU, item_bias, nI, dev)
+    gptr, mem = group_ptr.contiguous(), members.contiguous()
+    if M == 0:
+        mem = torch.zeros(1, dtype=I64, device=dev)
+
+    def launch(lib, Uc, Vc, ids, scores, ws, nbytes, err):
+        check(lib.yr_recommend_group_topk(Uc.data_ptr(), nU, Vc.data_ptr(), nI, d, _RT_DTYPES[U.dtype], dptr(gptr, I32),
+                                          G, dptr(mem, I64), M, code, dptr(sptr), dptr(sidx), NS, int(max_len),
+                                          dptr(sid), dptr(seen_ptr), dptr(seen_idx), K, dptr(ids), dptr(scores),
+                                          dptr(ws), nbytes, dptr(err), stream_ptr(dev), dptr(bias)),
+              "yr_recommend_group_topk")
+
+    ids, scores, e = _rt_run(U, V, G, K, dev, lambda lib: lib.yr_recommend_group_ws_bytes(G, NS, int(max_len), K),
+                             launch)
+    if e & 1:
+        raise IndexError(f"{what}: member id out of range [0, {nU})")
+    if e & 2:
+        raise IndexError(f"{what}: subset id out of range [-1, {NS})")
+    if e & 4:
+        raise ValueError(f"{what}: a group must have 1 to {RECOMMEND_GROUP_MAX_MEMBERS} members")
+    return ids, scores

@@ -45,6 +45,15 @@ layer rows W_o). The list comes back in pick order with the model's scores; lam 
 for bit. On CUDA tables the re-ranking is one kernel (yr_recommend_mmr: a block a row, no B x N x N similarity); on CPU
 tables, and as its oracle, `mmr_reference`, the plain PyTorch restatement (dense similarity, a k-step loop). The exact
 definition is in include/yelprec_b200.h.
+
+    ids, scores = rec.recommend_group([[3, 17, 42], [8, 9]], k=20, agg="min")   # one list per group (CDAE too)
+
+recommend_group ranks items for a group of 1 to 32 users (UserGroups, members sorted and deduplicated) by an aggregate
+of the members' recommend scores: agg="min" (least misery: the lowest member score, NaN if any is NaN) or agg="mean"
+(the scores summed in member order, each add rounded on its own, then divided by the member count). An item any member
+has seen is never returned; subset works as in recommend; a group of one gets recommend's row bit for bit. On CUDA
+tables it is one kernel (yr_recommend_group_topk: the members' scores are folded in registers, nothing of size
+groups x num_items is made); on CPU tables, and as its oracle, `recommend_group_reference`.
 """
 from __future__ import annotations
 
@@ -185,6 +194,7 @@ def _geo_args(subset, near, radius_km, locations: Optional[ItemLocations], nI: i
 class ItemLists:
     """Item lists as CSR: ptr int32 [num_rows + 1], idx int32 ascending and unique inside a row; max_len = the longest."""
     _row = "row"
+    _item = "item"
 
     def __init__(self, ptr, idx, num_rows: int, num_items: int):
         self.ptr = torch.as_tensor(ptr, dtype=I32)
@@ -203,11 +213,11 @@ class ItemLists:
         i = np.asarray(items.cpu() if torch.is_tensor(items) else items, dtype=np.int64).reshape(-1)
         name = f"{cls.__name__}.from_pairs"
         if r.shape != i.shape:
-            raise ValueError(f"{name}: {r.size} {cls._row}s but {i.size} items")
+            raise ValueError(f"{name}: {r.size} {cls._row}s but {i.size} {cls._item}s")
         if r.size and (r.min() < 0 or r.max() >= num_rows):
             raise IndexError(f"{name}: {cls._row} id out of range [0, {num_rows})")
         if i.size and (i.min() < 0 or i.max() >= num_items):
-            raise IndexError(f"{name}: item id out of range [0, {num_items})")
+            raise IndexError(f"{name}: {cls._item} id out of range [0, {num_items})")
         key = np.unique(r * num_items + i)
         ptr = np.zeros(num_rows + 1, dtype=np.int64)
         ptr[1:] = np.cumsum(np.bincount(key // num_items, minlength=num_rows))
@@ -261,6 +271,56 @@ class ItemSubsets(ItemLists):
     def from_pairs(cls, subset, item, num_subsets: int, num_items: int) -> "ItemSubsets":
         """From (subset, item) membership pairs; duplicates are dropped."""
         return cls._from_pairs(subset, item, num_subsets, num_items)
+
+
+class UserGroups(ItemLists):
+    """Groups of users as CSR: ptr int32 [num_groups + 1], members int64 ascending and unique inside a group (idx: the
+    same as int32). Every group has 1 to RECOMMEND_GROUP_MAX_MEMBERS (32) members; a builder raises ValueError for an
+    empty or larger group and IndexError for a user id outside [0, num_users)."""
+    _row = "group"
+    _item = "user"
+
+    def __init__(self, ptr, members, num_groups: int, num_users: int):
+        super().__init__(ptr, members, num_groups, num_users)
+        if self._rows and (self.lengths.min() < 1 or self.lengths.max() > ops.RECOMMEND_GROUP_MAX_MEMBERS):
+            raise ValueError(f"UserGroups: a group must have 1 to {ops.RECOMMEND_GROUP_MAX_MEMBERS} members, got "
+                             f"{int(self.lengths.min())} to {int(self.lengths.max())}")
+        self.members = self.idx.to(I64)
+        self._on = {self.ptr.device: (self.ptr, self.members)}
+
+    @property
+    def num_groups(self) -> int:
+        return self._rows
+
+    @property
+    def num_users(self) -> int:
+        return self.num_items
+
+    @classmethod
+    def from_pairs(cls, group, user, num_groups: int, num_users: int) -> "UserGroups":
+        """From (group, user) membership pairs; duplicates are dropped, members sorted."""
+        return cls._from_pairs(group, user, num_groups, num_users)
+
+    @classmethod
+    def from_lists(cls, groups, num_users: int) -> "UserGroups":
+        """From one sequence of user ids per group (e.g. [[3, 17, 42], [8, 9]]); duplicates are dropped, members sorted."""
+        lists = [np.asarray(g.cpu() if torch.is_tensor(g) else g, dtype=np.int64).reshape(-1) for g in groups]
+        group = np.repeat(np.arange(len(lists), dtype=np.int64), [x.size for x in lists])
+        user = np.concatenate(lists) if lists else np.zeros(0, np.int64)
+        return cls._from_pairs(group, user, len(lists), num_users)
+
+    def on(self, device) -> Tuple[torch.Tensor, torch.Tensor]:
+        """(ptr int32, members int64) on `device`, copied once per device."""
+        return _on_device(self._on, device, (self.ptr, self.members))
+
+
+def _as_groups(groups, num_users: int) -> UserGroups:
+    """`groups` (a UserGroups, or one sequence of user ids per group) as UserGroups over num_users users."""
+    if isinstance(groups, UserGroups):
+        if groups.num_users != num_users:
+            raise ValueError(f"recommend_group: the groups cover {groups.num_users} users, the user table {num_users}")
+        return groups
+    return UserGroups.from_lists(groups, num_users)
 
 
 def _check_k(k) -> int:
@@ -323,9 +383,25 @@ def recommend_reference(user_emb: torch.Tensor, item_emb: torch.Tensor, user_ids
     scores = user_emb[uid].to(F32) @ item_emb.to(F32).T
     if item_bias is not None:
         scores = scores + item_bias.to(device=dev, dtype=F32)[None, :]
+    inside = None
+    if geo:
+        c, t = geo_query(near, radius_km, B)
+        P = locations.P.to(dev)
+        inside = _geo_inside(P, torch.from_numpy(c).to(dev), torch.from_numpy(t).to(dev))
+    return _masked_topk(scores, k, _list_entries(seen, uid, dev) if seen is not None else None, subsets, subset, inside)
+
+
+def _masked_topk(scores: torch.Tensor, k: int, seen_entries, subsets: Optional[ItemSubsets], subset,
+                 inside: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """The tail of every reference: NaN scores, the seen entries (batch row, item), items outside the row's subset
+    (subsets[subset[b]]; -1 = whole catalog) and, given `inside` (bool [B x nI]), items outside it set to -inf; a stable
+    descending sort (torch.topk does not fix the order of ties), the first k kept and slots holding -inf turned into
+    padding (id -1). scores: float32 [B x nI]."""
+    dev = scores.device
+    B, nI = scores.shape
     scores = torch.where(torch.isnan(scores), torch.full_like(scores, float("-inf")), scores)
-    if seen is not None:
-        row, item = _list_entries(seen, uid, dev)
+    if seen_entries is not None:
+        row, item = seen_entries
         scores[row, item] = float("-inf")
     if subset is not None:
         sid = _subset_rows(subset, B, subsets).to(dev)
@@ -338,10 +414,7 @@ def recommend_reference(user_emb: torch.Tensor, item_emb: torch.Tensor, user_ids
         row, item = _list_entries(subsets, sid[limited], dev)
         outside[limited[row], item] = False
         scores[outside] = float("-inf")
-    if geo:
-        c, t = geo_query(near, radius_km, B)
-        P = locations.P.to(dev)
-        inside = _geo_inside(P, torch.from_numpy(c).to(dev), torch.from_numpy(t).to(dev))
+    if inside is not None:
         scores[~inside] = float("-inf")
     kk = min(k, nI)
     sc, order = torch.sort(scores, dim=1, descending=True, stable=True)
@@ -351,6 +424,51 @@ def recommend_reference(user_emb: torch.Tensor, item_emb: torch.Tensor, user_ids
     out = torch.full((B, k), float("-inf"), dtype=F32, device=dev)
     ids[:, :kk], out[:, :kk] = order, sc
     return ids, out
+
+
+def _group_agg(agg) -> str:
+    ops.group_agg(agg)
+    return agg
+
+
+def recommend_group_reference(user_emb: torch.Tensor, item_emb: torch.Tensor, groups, k: int, agg: str = "mean",
+                              seen: Optional[SeenItems] = None, subsets: Optional[ItemSubsets] = None, subset=None,
+                              item_bias: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Plain PyTorch on the tables' device: the dense [G x num_items] aggregate built member position by member position
+    j (rows of the groups with more than j members), each position's scores U[u_j] @ V^T (+ item_bias) folded by
+    separate elementwise ops: agg = "min": torch.minimum (NaN-propagating); "mean": an add per position, then one division
+    by the member count. Items in any member's seen list and items outside the row's subset then go through
+    recommend_reference's masking, stable sort and padding (_masked_topk)."""
+    k = _check_k(k)
+    agg = _group_agg(agg)
+    dev = user_emb.device
+    nU = user_emb.shape[0]
+    groups = _as_groups(groups, nU)
+    ptr, mem = groups.on(dev)
+    ptr = ptr.to(I64)
+    G, nI = groups.num_groups, item_emb.shape[0]
+    m = ptr[1:] - ptr[:-1]
+    V = item_emb.to(F32)
+    bias = item_bias.to(device=dev, dtype=F32)[None, :] if item_bias is not None else None
+    A = torch.zeros(G, nI, dtype=F32, device=dev)
+    for j in range(int(m.max()) if G else 0):
+        rows = (m > j).nonzero().reshape(-1)
+        s = user_emb[mem[ptr[rows] + j]].to(F32) @ V.T
+        if bias is not None:
+            s = s + bias
+        if j == 0:
+            A[rows] = s
+        elif agg == "min":
+            A[rows] = torch.minimum(A[rows], s)
+        else:
+            A[rows] = A[rows] + s
+    if agg == "mean":
+        A = A / m.to(F32)[:, None]
+    seen_entries = None
+    if seen is not None:
+        row, item = _list_entries(seen, mem, dev)                # entries of every member, by member position
+        seen_entries = (torch.repeat_interleave(torch.arange(G, device=dev), m)[row], item)
+    return _masked_topk(A, k, seen_entries, subsets, subset)
 
 
 def _pool_size(k, pool) -> int:
@@ -488,6 +606,57 @@ class Recommender:
             return mmr_reference(self.item_emb, ids, sc, k, lam)
         return ops.recommend_mmr(self.item_emb, ids, sc, k, lam)
 
+    def recommend_group(self, groups, k: int, agg: str = "mean", exclude_seen: bool = True, subset=None, near=None,
+                        radius_km=None) -> Tuple[torch.Tensor, torch.Tensor]:
+        """(item ids int64 [G x k], scores float32 [G x k]) on the tables' device: one list per group of users (a
+        UserGroups, or one sequence of user ids per group, 1 to 32 users each), ranked by the aggregate of the members'
+        recommend scores: agg = "min" (least misery: the lowest member score) or "mean". With exclude_seen, an item any
+        member has seen is never returned. subset as in recommend, one id for every group or G ids. Ranking, ties and
+        padding as recommend; a group of one user u gets recommend([u], k) bit for bit. The exact definition is in
+        include/yelprec_b200.h (yr_recommend_group_topk). near / radius_km are not supported for groups."""
+        if near is not None or radius_km is not None:
+            raise ValueError("recommend_group: near is not supported")
+        if exclude_seen and self.seen is None:
+            raise ValueError("recommend: exclude_seen=True needs the seen items (Recommender(..., seen=SeenItems...))")
+        if subset is not None and self.subsets is None:
+            raise ValueError("recommend: subset needs the item subsets (Recommender(..., subsets=ItemSubsets...))")
+        seen = self.seen if exclude_seen else None
+        dev = self.user_emb.device
+        groups = _as_groups(groups, self.user_emb.shape[0])
+        if dev.type != "cuda":
+            return recommend_group_reference(self.user_emb, self.item_emb, groups, k, agg, seen, self.subsets, subset)
+        k, agg = _check_k(k), _group_agg(agg)
+        gptr, mem = groups.on(dev)
+        ptr, idx = seen.on(dev) if seen is not None else (None, None)
+        return _recommend_group_kernel(self.user_emb, self.item_emb, gptr, mem, k, agg, ptr, idx, self.subsets, subset)
+
+
+def _subset_launch(subset, B: int, subsets: Optional[ItemSubsets], nI: int, dev):
+    """(subset_ptr, subset_idx, subset ids int64 [B], max_len) of a subset-restricted launch on `dev`. Host-side subset
+    ids let max_len (and so the number of item splits) follow the requested subsets; on a CUDA tensor it is num_items
+    (no device read)."""
+    sid = _subset_rows(subset, B, subsets)
+    if sid.is_cuda:
+        max_len = nI
+    else:
+        h = sid.numpy()
+        max_len = int(subsets.lengths[h[h >= 0]].max(initial=0))
+        if (h == -1).any():
+            max_len = nI
+    sptr, sidx = subsets.on(dev)
+    return sptr, sidx, sid.to(dev), max_len
+
+
+def _recommend_group_kernel(U, V, gptr, mem, k, agg, seen_ptr, seen_idx, subsets: Optional[ItemSubsets], subset,
+                            item_bias=None):
+    """ops.recommend_group_topk over the groups (gptr, mem: rows of U) on U's device, with `subset` restricted as in
+    _recommend_kernel; seen lists indexed by the rows of U."""
+    if subset is None:
+        return ops.recommend_group_topk(U, V, gptr, mem, k, agg, seen_ptr, seen_idx, item_bias=item_bias)
+    sptr, sidx, sid, max_len = _subset_launch(subset, gptr.numel() - 1, subsets, V.shape[0], U.device)
+    return ops.recommend_group_topk(U, V, gptr, mem, k, agg, seen_ptr, seen_idx, sptr, sidx, sid, max_len,
+                                    item_bias=item_bias)
+
 
 def _recommend_kernel(U, V, uid, k, seen_ptr, seen_idx, subsets: Optional[ItemSubsets], subset, item_bias=None,
                       locations: Optional[ItemLocations] = None, near=None, radius_km=None):
@@ -502,18 +671,8 @@ def _recommend_kernel(U, V, uid, k, seen_ptr, seen_idx, subsets: Optional[ItemSu
                                       seen_idx, item_bias=item_bias)
     if subset is None:
         return ops.recommend_topk(U, V, uid, k, seen_ptr, seen_idx, item_bias=item_bias)
-    sid = _subset_rows(subset, uid.numel(), subsets)
-    nI = V.shape[0]
-    if sid.is_cuda:
-        max_len = nI
-    else:
-        h = sid.numpy()
-        max_len = int(subsets.lengths[h[h >= 0]].max(initial=0))
-        if (h == -1).any():
-            max_len = nI
-    sptr, sidx = subsets.on(U.device)
-    return ops.recommend_subset_topk(U, V, uid, k, sptr, sidx, sid.to(U.device), max_len, seen_ptr, seen_idx,
-                                     item_bias=item_bias)
+    sptr, sidx, sid, max_len = _subset_launch(subset, uid.numel(), subsets, V.shape[0], U.device)
+    return ops.recommend_subset_topk(U, V, uid, k, sptr, sidx, sid, max_len, seen_ptr, seen_idx, item_bias=item_bias)
 
 
 def _cdae_check(model, seen: Optional[SeenItems], subsets: Optional[ItemSubsets], what: str) -> None:
@@ -538,16 +697,48 @@ def cdae_recommend_reference(model, user_ids, k: int, seen: SeenItems, exclude_s
     if uid.numel() and (int(uid.min()) < 0 or int(uid.max()) >= model.num_users):
         raise IndexError(f"recommend: user id out of range [0, {model.num_users})")
     B = uid.numel()
-    x = torch.zeros(B, model.num_items, device=dev, dtype=F32)
-    row, item = _list_entries(seen, uid, dev)
-    x[row, item] = 1.0
-    Wh, bh = model.hidden_layer.weight.data, model.hidden_layer.bias.data
-    pre = x @ Wh.T + bh + model.user_nodes.weight.data[uid]
-    z = pre if model.hidden_act == 1 else torch.sigmoid(pre)
+    z = _cdae_hidden_reference(model, uid, seen)
     rows = SeenItems(*_batch_lists(seen, uid), B, model.num_items) if exclude_seen else None
     return recommend_reference(z, model.output_layer.weight.data, torch.arange(B, device=dev), k, rows, subsets, subset,
                                item_bias=model.output_layer.bias.data, locations=locations, near=near,
                                radius_km=radius_km)
+
+
+def _cdae_hidden_reference(model, uid: torch.Tensor, seen: SeenItems) -> torch.Tensor:
+    """z [B x hidden] of the users uid (on the model's device), densely: the multi-hot x of their seen items,
+    z = act(x @ W_h^T + b_h + V_u[u])."""
+    dev = uid.device
+    x = torch.zeros(uid.numel(), model.num_items, device=dev, dtype=F32)
+    row, item = _list_entries(seen, uid, dev)
+    x[row, item] = 1.0
+    Wh, bh = model.hidden_layer.weight.data, model.hidden_layer.bias.data
+    pre = x @ Wh.T + bh + model.user_nodes.weight.data[uid]
+    return pre if model.hidden_act == 1 else torch.sigmoid(pre)
+
+
+def _cdae_group_rows(groups: UserGroups, dev):
+    """(unique members int64 ascending, the groups re-indexed onto them): the CDAE encodes each member once, z row r for
+    user uniq[r]; members stay ascending inside a group, so the mean sums them in the same order as over user ids."""
+    gptr, mem = groups.on(dev)
+    uniq = torch.unique(mem)
+    return uniq, gptr, torch.searchsorted(uniq, mem)
+
+
+def cdae_recommend_group_reference(model, groups, k: int, seen: SeenItems, agg: str = "mean",
+                                   exclude_seen: bool = True, subsets: Optional[ItemSubsets] = None,
+                                   subset=None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Plain PyTorch restatement of CDAERecommender.recommend_group on the model's device: the unique members' z
+    (dense, as cdae_recommend_reference), then recommend_group_reference over the logits z . W_o[i] + b_o[i] with the
+    members' seen lists by z row."""
+    _cdae_check(model, seen, subsets, "cdae_recommend_group_reference")
+    dev = model.hidden_layer.weight.device
+    groups = _as_groups(groups, model.num_users)
+    uniq, gptr, zrow = _cdae_group_rows(groups, dev)
+    z = _cdae_hidden_reference(model, uniq, seen)
+    zgroups = UserGroups(gptr.cpu(), zrow.cpu(), groups.num_groups, uniq.numel())
+    rows = SeenItems(*_batch_lists(seen, uniq), uniq.numel(), model.num_items) if exclude_seen else None
+    return recommend_group_reference(z, model.output_layer.weight.data, zgroups, k, agg, rows, subsets, subset,
+                                     item_bias=model.output_layer.bias.data)
 
 
 def cdae_recommend_diverse_reference(model, user_ids, k: int, seen: SeenItems, lam: float = 0.5,
@@ -631,3 +822,27 @@ class CDAERecommender:
         ops.mmr_weights(lam)
         ids, sc = self.recommend(user_ids, N, exclude_seen, subset, near, radius_km)
         return ops.recommend_mmr(self.model.output_layer.weight.data, ids, sc, k, lam)
+
+    def recommend_group(self, groups, k: int, agg: str = "mean", exclude_seen: bool = True, subset=None, near=None,
+                        radius_km=None) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Recommender.recommend_group for the CDAE: each distinct member is encoded once (yr_cdae_encode, in ascending
+        user id order), and the group kernel ranks the aggregated logits z . W_o[i] + b_o[i] with every member's seen
+        list (by z row) excluded."""
+        if near is not None or radius_km is not None:
+            raise ValueError("recommend_group: near is not supported")
+        if subset is not None and self.subsets is None:
+            raise ValueError("recommend: subset needs the item subsets (CDAERecommender(..., subsets=ItemSubsets...))")
+        m = self.model
+        dev = m.hidden_layer.weight.device
+        k, agg = _check_k(k), _group_agg(agg)
+        groups = _as_groups(groups, m.num_users)
+        if subset is not None:
+            _subset_rows(subset, groups.num_groups, self.subsets)
+        if groups.num_groups == 0:
+            return torch.empty(0, k, device=dev, dtype=I64), torch.empty(0, k, device=dev, dtype=F32)
+        uniq, gptr, zrow = _cdae_group_rows(groups, dev)
+        ptr, idx = self.seen.on(dev)
+        z = m.hidden_from_lists(uniq, ptr, idx)
+        bptr, bidx = _batch_lists(self.seen, uniq) if exclude_seen else (None, None)
+        return _recommend_group_kernel(z, m.output_layer.weight.data, gptr, zrow, k, agg, bptr, bidx, self.subsets,
+                                       subset, item_bias=m.output_layer.bias.data)

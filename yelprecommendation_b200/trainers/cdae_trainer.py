@@ -222,7 +222,8 @@ class CDAETrainer(BaseTrainer):
     def recommender(self, seen=None, subsets=None, locations=None):
         """retrieval.CDAERecommender over the model's live parameters (recommend(user_ids, k, exclude_seen=True,
         subset=None, near=None, radius_km=None); scores are output logits; recommend_diverse re-ranks with similarity in
-        the output layer's rows W_o). `seen` is required: it is the users' input as well as what is excluded."""
+        the output layer's rows W_o; recommend_group encodes each member once and aggregates the members' logits). `seen`
+        is required: it is the users' input as well as what is excluded."""
         from ..retrieval import CDAERecommender
         return CDAERecommender(self.model, seen, subsets, locations)
 

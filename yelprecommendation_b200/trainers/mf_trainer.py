@@ -179,8 +179,9 @@ class MFTrainer(BaseTrainer):
 
     def recommender(self, seen=None, subsets=None, locations=None):
         """retrieval.Recommender over the current user / item tables (recommend(user_ids, k, exclude_seen=True, subset=None,
-        near=None, radius_km=None), and recommend_diverse(user_ids, k, lam=0.5, pool=None, ...) for a diverse list re-ranked
-        from a pool of recommend's best)."""
+        near=None, radius_km=None), recommend_diverse(user_ids, k, lam=0.5, pool=None, ...) for a diverse list re-ranked
+        from a pool of recommend's best, and recommend_group(groups, k, agg="mean", ...) for one list per group of users
+        ranked by the members' least-misery or mean score)."""
         from ..retrieval import Recommender
         return Recommender(self.model.user_embedding.weight.data, self.model.item_embedding.weight.data, seen, subsets,
                            locations)

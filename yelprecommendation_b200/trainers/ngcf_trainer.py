@@ -272,7 +272,8 @@ class NGCFTrainer(BaseTrainer):
 
     def recommender(self, seen=None, subsets=None, locations=None):
         """retrieval.Recommender over the propagated, layer-concatenated user / item embeddings that evaluate() ranks with;
-        recommend_diverse measures similarity in the concatenated item rows."""
+        recommend_diverse measures similarity in the concatenated item rows, and recommend_group aggregates the members'
+        scores over the same rows."""
         from ..retrieval import Recommender
         cat = ops.ngcf_concat(self.propagate()[0])
         return Recommender(cat[: self.num_users], cat[self.num_users:], seen, subsets, locations)
