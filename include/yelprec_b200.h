@@ -444,9 +444,12 @@ int yr_cdae_output(const yr_cdae_tensors* P, int64_t nI, int h, const float* z, 
 
 /* One CDAETrainer.train step (trainers/cdae_trainer.py:39-52) or, with opt == NULL, the loss-only pass of
  * validate (:62-70): forward, NSBCELoss over the positions where target + negative_mask != 0 (loss.py:12-16, BCE
- * mean, logs clamped at -100 like torch), backward restricted to those positions, dense optimizer step over all
- * five tensors. grads must be all-zero on entry and are all-zero on exit. loss (device double[2]): [0] += batch
- * loss, [1] scratch. step_loss may be NULL. `target` is input_mask for train, input_mask + valid_mask for validate. */
+ * mean, logs clamped at -100 like torch), backward restricted to those positions with torch's autograd chain
+ * d loss / d logit = (p - t) / max((1 - p) p, 1e-12) / m * (1 - p) p (m loss positions; p - t except where p
+ * saturates), dense optimizer step over all five tensors. grads must be all-zero on entry and are all-zero on exit.
+ * loss (device double[2]): [0] += batch loss, [1] scratch. step_loss may be NULL. `target` is input_mask for train,
+ * input_mask + valid_mask for validate. P->Wo and grads->Wo must be aligned to 4 * min(h / 32, 4) bytes (their rows are
+ * read and accumulated as float2 / float4), YR_ERR_BAD_ARG otherwise; the other tensors need 4 bytes. */
 int yr_cdae_step(const yr_cdae_tensors* P, const yr_cdae_tensors* grads, const yr_cdae_tensors* m,
                  const yr_cdae_tensors* v, const yr_opt* opt, int64_t nU, int64_t nI, int h,
                  const int64_t* uid, const float* x, const float* keep, const float* target,
@@ -463,7 +466,9 @@ int yr_cdae_step_ex(const yr_cdae_tensors* P, const yr_cdae_tensors* grads, cons
  * per user; the lists are a few hundred bytes): in_ptr [B + 1] / in_idx = the active inputs of every row (ascending item ids),
  * in_val = their values after dropout (NULL = 1: evaluation), tgt_ptr / tgt_idx / tgt_val = the loss positions of every row
  * (ascending item ids: the union of the target items, value 1, and the sampled negatives, value 0). Same arithmetic and
- * order as yr_cdae_step_ex on the equivalent dense tensors. opt == NULL: loss only. */
+ * order as yr_cdae_step_ex on the equivalent dense tensors when in_val is NULL or has no zero. A listed input of value 0
+ * (dropped by dropout) stays in the hidden layer's sums, where the dense path compacts it out, so the terms are split
+ * differently over the partial sums and the results may differ in the last bits. opt == NULL: loss only. */
 int yr_cdae_step_idx(const yr_cdae_tensors* P, const yr_cdae_tensors* grads, const yr_cdae_tensors* m,
                      const yr_cdae_tensors* v, const yr_opt* opt, int64_t nU, int64_t nI, int h, int hidden_act,
                      const int64_t* uid, const int32_t* in_ptr, const int32_t* in_idx, const float* in_val,

@@ -270,7 +270,11 @@ cdae_row_kernel(yr_cdae_tensors P, yr_cdae_tensors Gr, int64_t nU, int64_t nI, c
       const float lp = fmaxf(logf(p), -100.f), lq = fmaxf(log1pf(-p), -100.f);
       lsum += (double)(-(t[q] * lp + (1.f - t[q]) * lq));
       if (GRAD) {
-        const float dl = (p - t[q]) * inv_m;                     // d loss / d logit (mean over all loss positions)
+        // d loss / d logit (mean over all loss positions) as torch's autograd takes it: binary_cross_entropy's backward
+        // (p - t) / max((1 - p) p, 1e-12), then sigmoid's (1 - p) p, i.e. (p - t) min(1, (1 - p) p / 1e-12). That is
+        // p - t, bit for bit, except where (1 - p) p < 1e-12 (logit above ~16.6, where p rounds to 1, or below ~-27.6):
+        // a negative the model is sure about gets 0, not 1. The product form keeps a division out of the loop.
+        const float dl = (p - t[q]) * inv_m * fminf(1.f, (1.f - p) * p * 1e12f);
         Row<VPL> gw;
 #pragma unroll
         for (int i = 0; i < VPL; ++i) { dz.x[i] = fmaf(dl, wo[q].x[i], dz.x[i]); gw.x[i] = dl * zz.x[i]; }
@@ -470,13 +474,20 @@ static int cdae_step_tail(const yr_cdae_tensors* P, const yr_cdae_tensors* grads
                           const int64_t* uid, int64_t B, double* loss, float* step_loss, const CdaeWs& w, int32_t* err,
                           yr_stream stream);
 
+// the row kernel reads Wo's rows and accumulates their gradients as float (h = 32), float2 (64) or float4 (128 and up)
+static bool cdae_wo_aligned(const float* Wo, int h) {
+  const int vpl = dim_vpl(h);
+  return ((uintptr_t)Wo % (sizeof(float) * (size_t)(vpl < 4 ? vpl : 4))) == 0;
+}
+
 static int cdae_step_args_ok(const yr_cdae_tensors* P, const yr_cdae_tensors* grads, const yr_cdae_tensors* m,
                              const yr_cdae_tensors* v, const yr_opt* opt, int h, int hidden_act) {
   if (cdae_tensors_ok(P)) return YR_ERR_BAD_ARG;
   if (hidden_act != YR_ACT_SIGMOID && hidden_act != YR_ACT_IDENTITY) return YR_ERR_BAD_ARG;
   if (!dim_vpl(h)) return YR_ERR_BAD_DIM;
+  if (!cdae_wo_aligned(P->Wo, h)) return YR_ERR_BAD_ARG;
   if (opt) {
-    if (cdae_tensors_ok(grads)) return YR_ERR_BAD_ARG;
+    if (cdae_tensors_ok(grads) || !cdae_wo_aligned(grads->Wo, h)) return YR_ERR_BAD_ARG;
     if (opt->kind < YR_OPT_SGD || opt->kind > YR_OPT_ADAMW) return YR_ERR_BAD_OPT;
     if (opt->kind != YR_OPT_SGD && (cdae_tensors_ok(m) || cdae_tensors_ok(v))) return YR_ERR_BAD_ARG;
   }
@@ -515,16 +526,10 @@ extern "C" int yr_cdae_step_ex(const yr_cdae_tensors* P, const yr_cdae_tensors* 
                                const int64_t* uid, const float* x, const float* keep, const float* target,
                                const float* negative_mask, int64_t B, double* loss, float* step_loss, void* ws,
                                size_t ws_bytes, int32_t* err, yr_stream stream) {
-  if (cdae_tensors_ok(P) || !uid || !x || !target || !loss || !ws || B <= 0 || nI <= 0) return YR_ERR_BAD_ARG;
-  if (hidden_act != YR_ACT_SIGMOID && hidden_act != YR_ACT_IDENTITY) return YR_ERR_BAD_ARG;
-  if (!dim_vpl(h)) return YR_ERR_BAD_DIM;
+  if (!uid || !x || !target || !loss || !ws || B <= 0 || nI <= 0) return YR_ERR_BAD_ARG;
+  int rc = cdae_step_args_ok(P, grads, m, v, opt, h, hidden_act);
+  if (rc) return rc;
   if (ws_bytes < yr_cdae_ws_bytes(B, nI)) return YR_ERR_WORKSPACE;
-  const bool train = opt != nullptr;
-  if (train) {
-    if (cdae_tensors_ok(grads)) return YR_ERR_BAD_ARG;
-    if (opt->kind < YR_OPT_SGD || opt->kind > YR_OPT_ADAMW) return YR_ERR_BAD_OPT;
-    if (opt->kind != YR_OPT_SGD && (cdae_tensors_ok(m) || cdae_tensors_ok(v))) return YR_ERR_BAD_ARG;
-  }
   cudaStream_t s = (cudaStream_t)stream;
   CdaeWs w;
   cdae_ws_layout(B, nI, ws, &w);

@@ -14,8 +14,10 @@ class BPRLoss(nn.Module):
 
 class NSBCELoss(nn.Module):
     """Drop-in for the reference's loss.py:7-16: BCE (mean) over the positions where target + negative_mask != 0,
-    on dense tensors (yr_nsbce_loss). Inference-style (no autograd): the fused CDAE trainer computes the same loss and
-    its gradient at the compacted positions without ever building the dense prediction."""
+    on dense tensors (yr_nsbce_loss). Inference-style (no autograd): the fused CDAE trainer computes the same loss at the
+    compacted positions without ever building the dense prediction, and its gradient the way torch's autograd takes it
+    through sigmoid and binary_cross_entropy, (p - t) / max((1 - p) p, 1e-12) * (1 - p) p, so a saturated p gives
+    torch's gradient rather than p - t."""
 
     def __init__(self, weight=None, size_average=None, reduce=None, reduction: str = "mean") -> None:
         super().__init__()
